@@ -2,7 +2,7 @@
 """Benchmark of the PoVar hot path on B200: stratified two-step solve of a synthetic
 venice-1778-shaped BAL problem (BASELINE.json, configs[3]).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--dump-outputs DIR]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one full stratified solve (step 1 pOSE PoVar + step 2 RIPOBA) of the workload.
@@ -131,7 +131,7 @@ def reference_arm(args, sp, path, workdir):
     threads = os.cpu_count() or 1
     it1, it2 = args.ref_iters
     # warm-up runs would cost minutes on the CPU; one untimed tiny run checks the binary, then K samples
-    steps = max(1, args.steps)
+    steps = args.steps
     runs = [run_reference_sample(path, threads, it1, it2, args.robust, workdir) for _ in range(steps)]
     trials = sum(r["trials"] for r in runs)
     t = sum(r["optimize_s"] for r in runs)
@@ -151,6 +151,34 @@ def reference_arm(args, sp, path, workdir):
     }
 
 
+DUMP_BYTES = 60_000_000      # payload of --dump-outputs: with the .npy headers, below 64 MB
+
+
+def dump_outputs(out_dir, its, summ, P, X):
+    """Write what a caller of the timed solve receives, one float64 .npy per output, so that two builds can be
+    compared output for output on the same seeded problem: every field of the per-trial records (trial_<field>) and
+    of the summary (summary_<field>) except the timings and the message, the final cameras [C, 3, 4] and landmarks
+    [L, 4].  Landmarks beyond what fits in DUMP_BYTES are a fixed seeded sample of rows, listed in landmark_rows."""
+    from povar_b200 import capi
+
+    def fields(struct):
+        return [f for f, _ in struct._fields_ if not f.endswith("_time") and f != "message"]
+
+    out = {f"trial_{f}": np.array([getattr(e, f) for e in its], dtype=np.float64) for f in fields(capi.Iteration)}
+    out.update({f"summary_{f}": np.float64(getattr(summ, f)) for f in fields(capi.SolveSummary)})
+    out["cameras"] = np.asarray(P, dtype=np.float64)
+    room = DUMP_BYTES - sum(np.asarray(a).nbytes for a in out.values())
+    X = np.asarray(X, dtype=np.float64)
+    if X.nbytes > room:
+        rows = np.sort(np.random.default_rng(0).choice(X.shape[0], room // (X[0].nbytes + 8), replace=False))
+        out["landmark_rows"] = rows.astype(np.float64)
+        X = X[rows]
+    out["landmarks"] = X
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 # ---------------------------------------------------------------------------------------------
 def main():
     ap = argparse.ArgumentParser()
@@ -167,7 +195,14 @@ def main():
     ap.add_argument("--trace-out", default=None,
                     help="write the logged trace of the last timed solve (cost, accept/reject, term counts) as json: "
                          "what runs at different GPU counts are compared by (tools/compare_traces.py)")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="after the timed steps, write what the last timed solve returned (per-trial records, summary, "
+                         "final cameras and landmarks) as DIR/<name>.npy in float64, below 64 MB in all (--impl ours)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the GPU solve returned: it needs --impl ours")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -291,6 +326,13 @@ def main():
     t_res = reduce_max(ev0.elapsed_time(ev1) * 1e-3)
     launches = solver.launch_count() - launches0
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs:
+        # read now: the roofline runs below overwrite the handle's state
+        P_out, X_out = solver.get_state(capi.STATE_JOINT)
+        if world > 1:       # cameras are replicated, landmarks come back per shard in rank order
+            shards = [None] * world
+            dist.all_gather_object(shards, X_out)
+            X_out = np.concatenate(shards)
     final_cost = its[-1].cost
     step1_trials = sum(1 for e in its if e.step == 1)
     # what the solve produced, so that runs at different GPU counts can be compared from their bench lines: the
@@ -447,6 +489,8 @@ def main():
         if world > 1:
             dist.destroy_process_group()
         return
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, its, summ, P_out, X_out)
 
     # ---- CPU baseline on a bounded sample (rank 0, N == 1 only)
     cpu = None

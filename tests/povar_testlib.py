@@ -1,9 +1,11 @@
 """Shared helpers of the test-suite: golden fixtures, problem construction for both sides."""
 from __future__ import annotations
 
+import atexit
 import hashlib
 import json
 import os
+import shutil
 import tempfile
 
 import numpy as np
@@ -15,6 +17,17 @@ GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 _traces = None
 _files = {}
+_regen_dir = None
+
+
+def _private_tmp() -> str:
+    """Directory of this test process for regenerated problem files: a fixed name in the shared temp directory
+    can belong to another user (or to a concurrent run) and then cannot be rewritten."""
+    global _regen_dir
+    if _regen_dir is None:
+        _regen_dir = tempfile.mkdtemp(prefix="povar_golden_")
+        atexit.register(shutil.rmtree, _regen_dir, True)
+    return _regen_dir
 
 
 def traces():
@@ -47,7 +60,7 @@ def golden_file(shape: str) -> str:
     if meta["committed"]:
         path = os.path.join(GOLD, f"{shape}.txt")
     else:
-        path = os.path.join(tempfile.gettempdir(), f"povar_golden_{shape}.txt")
+        path = os.path.join(_private_tmp(), f"{shape}.txt")
         synthetic.write_bal(synthetic.generate_named(shape), path)
     h = hashlib.sha256()
     with open(path, "rb") as f:
@@ -56,6 +69,33 @@ def golden_file(shape: str) -> str:
     assert h.hexdigest() == meta["sha256"], f"{shape}: regenerated file differs from the golden one"
     _files[shape] = path
     return path
+
+
+def write_bal9(path, sp, rng):
+    """A BAL file (9 parameters per camera) of a synthetic problem, the input of --create-dataset; returns the cameras."""
+    with open(path, "w") as f:
+        f.write(f"{sp.num_cams} {sp.num_lms} {sp.num_obs}\n")
+        for c, l, (x, y) in zip(sp.obs_cam, sp.obs_lm, sp.obs_xy):
+            f.write(f"{c} {l}     {x:.10e} {y:.10e}\n")
+        cams = rng.normal(size=(sp.num_cams, 9))
+        cams[:, 6] = 1000.0 + rng.normal(size=sp.num_cams)
+        cams[:, 7:] *= 1e-7
+        for v in cams.reshape(-1):
+            f.write(f"{v:.16e}\n")
+        for v in sp.points.reshape(-1):
+            f.write(f"{v:.16e}\n")
+    return cams
+
+
+def create_dataset_lines(text, num_obs, num_cams):
+    """Lines of a --create-dataset output without a trailing empty one, the random camera-matrix entries (the first 8
+    of each camera's 15 lines) as None: what two programs writing the same input must agree on."""
+    lines = text.split("\n")
+    if lines and lines[-1] == "":
+        lines.pop()
+    first_cam = 1 + num_obs
+    return [None if 0 <= i - first_cam < 15 * num_cams and (i - first_cam) % 15 < 8 else s
+            for i, s in enumerate(lines)]
 
 
 def flags_to_options(flags):

@@ -16,6 +16,11 @@ that the GPU box, which has no /root/reference, can check against them.
                                    the reference is not bit-reproducible across thread counts (SURVEY
                                    F10), and its own 1-vs-8-thread deviation is the yardstick for how
                                    far a re-implementation can be expected to agree late in step 2.
+  tests/golden/create_dataset_small.json   what `--create-dataset` writes for the seeded BAL file of
+                                   tests/test_host_abi.py, the random camera-matrix entries masked
+  tests/golden/dump_config.json    what `--dump-config --input x` prints (every default)
+                                   These two come from the reference program where it is built, otherwise from this
+                                   project's bal; their "source" says which.
 """
 from __future__ import annotations
 
@@ -36,6 +41,7 @@ GOLD = os.path.join(ROOT, "tests", "golden")
 BAL_REF = os.path.join(ROOT, "oracle", "_ref", "bal_ref")
 COD_PROBE = os.path.join(ROOT, "oracle", "_ref", "cod_probe")
 INDEX_PROBE = os.path.join(ROOT, "oracle", "_ref", "index_probe")
+BAL_OURS = os.path.join(ROOT, "povar_b200", "bin", "bal")
 
 # (name, shape, extra reference flags).  --alpha / --power-sc-iterations are always explicit (SURVEY F3).
 CONFIGS = [
@@ -177,9 +183,36 @@ def make_ba_log_keys():
     print("ba_log_keys.json written")
 
 
+def make_bal_cli_fixtures():
+    """tests/golden/create_dataset_small.json and dump_config.json (tests/test_host_abi.py compares this project's
+    bal with them, and with the reference program where it is built)."""
+    sys.path.insert(0, os.path.join(ROOT, "tests"))
+    import povar_testlib as common
+    if os.path.exists(BAL_REF):
+        prog, source = BAL_REF, "the reference program (oracle/_ref/bal_ref)"
+    else:
+        prog, source = BAL_OURS, "this project's bal; the reference program was not built where this file was made"
+    sp = synthetic.generate_named("small")
+    with tempfile.TemporaryDirectory() as tmp:
+        src = os.path.join(tmp, "problem-16-400-pre.txt")
+        common.write_bal9(src, sp, np.random.default_rng(7))
+        subprocess.run([prog, "--input", src, "--create-dataset"], cwd=tmp, capture_output=True, check=True)
+        with open(os.path.join(tmp, "data_custom", os.path.basename(src))) as f:
+            lines = common.create_dataset_lines(f.read(), sp.num_obs, sp.num_cams)
+        dump = subprocess.run([prog, "--dump-config", "--input", "x"], cwd=tmp, capture_output=True, text=True).stdout
+    with open(os.path.join(GOLD, "create_dataset_small.json"), "w") as f:
+        json.dump({"_comment": "--create-dataset output for common.write_bal9(synthetic 'small', default_rng(7)), one "
+                               "entry per line, null where the program draws a random camera-matrix entry; made by "
+                               "tools/make_golden.py", "source": source, "lines": lines}, f, indent=0)
+    with open(os.path.join(GOLD, "dump_config.json"), "w") as f:
+        json.dump({"_comment": "--dump-config --input x print-out; made by tools/make_golden.py", "source": source,
+                   "dump": dump}, f, indent=1)
+    print("create_dataset_small.json and dump_config.json written from", prog)
+
+
 def main():
     """python tools/make_golden.py            everything (kernel_COD vectors, index fixture, all traces)
-    python tools/make_golden.py NAME ...   only these configurations / "index" / "cod" / "keys", merged into the
+    python tools/make_golden.py NAME ...   only these configurations / "index" / "cod" / "keys" / "cli", merged into the
                                            existing traces.json"""
     os.makedirs(GOLD, exist_ok=True)
     want = set(sys.argv[1:])
@@ -194,6 +227,8 @@ def main():
         make_index_fixture()
     if not want or "keys" in want:
         make_ba_log_keys()
+    if not want or "cli" in want:
+        make_bal_cli_fixtures()
     configs = [c for c in CONFIGS if not want or c[0] in want]
     paths = {}
     with tempfile.TemporaryDirectory() as tmp:
