@@ -356,6 +356,26 @@ int povar_debug_walk_trace(uint64_t* out, int32_t n);
  * reference does with Eigen::SimplicialLLT (sc/linearization_sc.hpp:236-245); exposed for the tests. */
 int povar_debug_cholesky(int32_t n, const double* A, const double* b, double* x, int32_t* info);
 
+/* CHOLESKY keeps the reduced camera system dense while that takes at most 96 GB and switches to tile-sparse storage
+ * beyond: only the 64x64 tiles of the factor that can be non-zero, cameras in reverse Cuthill-McKee order of their
+ * co-visibility graph (DESIGN.md 4).  If the tile-sparse factor does not fit the device's free memory either, the
+ * solve fails with POVAR_ERR_UNSUPPORTED.  mode 0: that automatic choice, 1: tile-sparse always (tests).
+ * povar_debug_read names "chol_perm" [C] (position of every camera in the factor order) and "chol_tiles" [1]
+ * (stored tiles) have 0 elements unless the handle's last CHOLESKY solve ran on tile-sparse storage. */
+int povar_debug_set_cholesky_storage(povar_handle* h, int32_t mode);
+
+/* povar_debug_cholesky on tile-sparse storage: the pattern is that of the non-zero block x block blocks of A's lower
+ * triangle, ordered and factorised symbolically as a handle's S is (one block per camera), and the same kernels run.
+ * *stored_tiles: 64x64 tiles of the factor kept. */
+int povar_debug_sparse_cholesky(int32_t n, int32_t block, const double* A, const double* b, double* x,
+                                int32_t* info, int64_t* stored_tiles);
+
+/* the host ordering and symbolic factorisation of the tile-sparse CHOLESKY for a landmark-major index (the
+ * co-visibility bitmap built on the host): perm [num_cams] = position of every camera, *stored_tiles.  `threads` > 0
+ * fixes the number of host threads (the result does not depend on it), 0 = automatic. */
+int povar_debug_cholesky_symbolic(int32_t num_cams, int32_t num_lms, const int64_t* lm_ptr, const int32_t* obs_cam,
+                                  int32_t threads, int32_t* perm, int64_t* stored_tiles);
+
 /* Caps the number of camera records the landmark half of a power-series term stages in shared memory (0 = as many
  * as fit).  The result must not depend on it: cameras outside the staged window are read from global memory.  Tests
  * use it to exercise that path on problems whose whole camera table would fit. */

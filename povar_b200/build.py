@@ -35,6 +35,7 @@ LIB_SOURCES = [
     "host/bal_io.cpp",
     "host/ba_log_writer.cpp",
     "host/lm_driver.cpp",
+    "host/chol_symbolic.cpp",
 ]
 HEADERS = ["device_math.cuh", "sell_walk.cuh", "povar_internal.h", "engine.h", "../../include/povar_b200.h"]
 

@@ -157,6 +157,11 @@ SIGNATURES = {
     "povar_peer_exchange_active": (C.c_int, [_H]),
     "povar_debug_set_window": (C.c_int, [_H, C.c_int32]),
     "povar_debug_cholesky": (C.c_int, [C.c_int32, _DP, _DP, _DP, C.POINTER(C.c_int32)]),
+    "povar_debug_set_cholesky_storage": (C.c_int, [_H, C.c_int32]),
+    "povar_debug_sparse_cholesky": (C.c_int, [C.c_int32, C.c_int32, _DP, _DP, _DP, C.POINTER(C.c_int32),
+                                              C.POINTER(C.c_int64)]),
+    "povar_debug_cholesky_symbolic": (C.c_int, [C.c_int32, C.c_int32, C.POINTER(C.c_int64), C.POINTER(C.c_int32),
+                                                C.c_int32, C.POINTER(C.c_int32), C.POINTER(C.c_int64)]),
     "povar_write_ba_log": (C.c_int, [C.c_char_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p]),
     "povar_debug_sell_layout": (C.c_int, [C.c_int32, C.c_int32, C.POINTER(C.c_int64), C.POINTER(C.c_int32), C.c_int32,
                                           C.c_int32, C.POINTER(C.c_int32), C.POINTER(C.c_int32),
@@ -447,6 +452,10 @@ class Solver:
     def debug_set_window(self, cams: int) -> None:
         self._check(self.lib.povar_debug_set_window(self.h, cams))
 
+    def debug_set_cholesky_storage(self, mode: int) -> None:
+        """CHOLESKY storage of S: 0 dense while it fits under 96 GB, tile-sparse beyond; 1 tile-sparse always."""
+        self._check(self.lib.povar_debug_set_cholesky_storage(self.h, mode))
+
     def launch_count(self) -> int:
         return int(self.lib.povar_launch_count(self.h))
 
@@ -547,6 +556,37 @@ def cholesky_solve(A: np.ndarray, b: np.ndarray):
     if rc != OK:
         raise PovarError(rc, "povar_debug_cholesky failed")
     return x, info.value
+
+
+def sparse_cholesky_solve(A: np.ndarray, b: np.ndarray, block: int = 12):
+    """x = A^-1 b by the library's tile-sparse Cholesky (povar_debug_sparse_cholesky): the pattern is that of the
+    non-zero block x block blocks of A's lower triangle.  Returns (x, info, stored_tiles)."""
+    lib = load()
+    A = np.ascontiguousarray(A, dtype=np.float64)
+    b = np.ascontiguousarray(b, dtype=np.float64)
+    x = np.empty_like(b)
+    info = C.c_int32(0)
+    tiles = C.c_int64(0)
+    rc = lib.povar_debug_sparse_cholesky(A.shape[0], block, _dp(A), _dp(b), _dp(x), C.byref(info), C.byref(tiles))
+    if rc != OK:
+        raise PovarError(rc, "povar_debug_sparse_cholesky failed")
+    return x, info.value, tiles.value
+
+
+def cholesky_symbolic(hp: "HostProblem", threads: int = 0):
+    """Camera order and stored 64x64 tiles of the tile-sparse CHOLESKY factor of `hp` (povar_debug_cholesky_symbolic):
+    (perm, stored_tiles), perm[c] = position of camera c."""
+    lib = load()
+    lp = np.ascontiguousarray(hp.lm_ptr, dtype=np.int64)
+    oc = np.ascontiguousarray(hp.obs_cam, dtype=np.int32)
+    perm = np.empty(hp.num_cams, dtype=np.int32)
+    tiles = C.c_int64(0)
+    rc = lib.povar_debug_cholesky_symbolic(hp.num_cams, hp.num_lms, lp.ctypes.data_as(C.POINTER(C.c_int64)),
+                                           oc.ctypes.data_as(C.POINTER(C.c_int32)), threads,
+                                           perm.ctypes.data_as(C.POINTER(C.c_int32)), C.byref(tiles))
+    if rc != OK:
+        raise PovarError(rc, "povar_debug_cholesky_symbolic failed")
+    return perm, tiles.value
 
 
 def host_id() -> bytes:

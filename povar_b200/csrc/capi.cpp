@@ -12,6 +12,8 @@ int nccl_unique_id(uint8_t id[128], std::string* err);
 int nccl_finalize();
 int host_unique_id(uint8_t id[128]);
 int debug_cholesky(int n, const double* A, const double* b, double* x, int* info_out);
+int debug_sparse_cholesky(int n, int block, const double* A, const double* b, double* x, int* info_out,
+                          long long* stored_tiles);
 }
 
 struct povar_handle {
@@ -286,6 +288,41 @@ int povar_debug_walk_trace(uint64_t* out, int32_t n) {
 
 int povar_debug_cholesky(int32_t n, const double* A, const double* b, double* x, int32_t* info) {
   return povar::debug_cholesky(n, A, b, x, info);
+}
+
+int povar_debug_sparse_cholesky(int32_t n, int32_t block, const double* A, const double* b, double* x, int32_t* info,
+                                int64_t* stored_tiles) {
+  long long tiles = 0;
+  const int rc = povar::debug_sparse_cholesky(n, block, A, b, x, info, &tiles);
+  if (stored_tiles) *stored_tiles = tiles;
+  return rc;
+}
+
+int povar_debug_cholesky_symbolic(int32_t num_cams, int32_t num_lms, const int64_t* lm_ptr, const int32_t* obs_cam,
+                                  int32_t threads, int32_t* perm, int64_t* stored_tiles) {
+  if (num_cams <= 0 || num_lms < 0 || !lm_ptr || lm_ptr[0] != 0 || (lm_ptr[num_lms] > 0 && !obs_cam)) {
+    return POVAR_ERR_INVALID;
+  }
+  for (int32_t l = 0; l < num_lms; ++l) {
+    if (lm_ptr[l + 1] < lm_ptr[l]) return POVAR_ERR_INVALID;
+  }
+  for (int64_t i = 0; i < lm_ptr[num_lms]; ++i) {
+    if (obs_cam[i] < 0 || obs_cam[i] >= num_cams) return POVAR_ERR_INVALID;
+  }
+  std::vector<unsigned int> bits;
+  povar::covisibility_host(num_cams, num_lms, lm_ptr, obs_cam, &bits);
+  povar::CholPattern p;
+  povar::chol_symbolic(num_cams, 12, bits, threads, &p);
+  if (perm) std::copy(p.perm.begin(), p.perm.end(), perm);
+  if (stored_tiles) *stored_tiles = p.tiles();
+  return POVAR_OK;
+}
+
+int povar_debug_set_cholesky_storage(povar_handle* h, int32_t mode) {
+  PV_ENGINE(h);
+  if (mode != 0 && mode != 1) return POVAR_ERR_INVALID;
+  e.debug_set_cholesky_storage(mode);
+  return POVAR_OK;
 }
 
 int povar_debug_set_window(povar_handle* h, int32_t cams) {

@@ -1504,32 +1504,111 @@ int Engine::solve_pcg(bool joint, double lambda) {
 }
 
 // CHOLESKY, step 1 (solver/linearizor_sc.cpp:121-128, sc/linearization_sc.hpp:236-245): the reference
-// factorises the sparse reduced camera system with Eigen::SimplicialLLT; here S is assembled densely without
-// atomics and factorised by the hand-written blocked LL^T of kernels_chol.cu (FP64 tensor-core tile updates).
-// The solution of S x = -b is unique, so ordering / blocking do not change the result beyond rounding.
+// factorises the sparse reduced camera system with Eigen::SimplicialLLT; here S is assembled without atomics and
+// factorised by the hand-written blocked LL^T of kernels_chol.cu (FP64 tensor-core tile updates).  S is dense while
+// that fits under kCholDenseCap, tile-sparse beyond (only the tiles of the factor that can be non-zero, in reverse
+// Cuthill-McKee camera order).  The solution of S x = -b is unique, so ordering / blocking do not change the result
+// beyond rounding.
+constexpr long long kCholDenseCap = 96LL << 30;
+
+// the tile pattern of the factor: co-visibility bitmap on the device, ordering and symbolic factorisation on the
+// host, the pattern and the tiles in device memory.  Fails with POVAR_ERR_UNSUPPORTED when the factor would not fit.
+int Engine::setup_cholesky_tiles() {
+  const size_t words = (static_cast<size_t>(C_) + 31) / 32;
+  std::vector<unsigned int> bits(static_cast<size_t>(C_) * words);
+  {   // the bitmap (C^2 / 8 bytes) lives only until the host has it
+    void* dbits = nullptr;
+    PV_CUDA(cudaMallocAsync(&dbits, sizeof(unsigned int) * bits.size(), stream_));
+    cudaError_t e = build_covisibility(L_, C_, d_.ix.lm_ptr, d_.ix.obs_cam, static_cast<unsigned int*>(dbits), lc());
+    if (e == cudaSuccess) {
+      e = cudaMemcpyAsync(bits.data(), dbits, sizeof(unsigned int) * bits.size(), cudaMemcpyDeviceToHost, stream_);
+    }
+    cudaFreeAsync(dbits, stream_);
+    PV_CUDA(e);
+    PV_CUDA(cudaStreamSynchronize(stream_));
+  }
+  CholPattern& p = chol_pat_;
+  chol_symbolic(C_, 12, bits, 0, &p);
+  const size_t T = static_cast<size_t>(p.T), tiles = static_cast<size_t>(p.tiles());
+  const size_t need = sizeof(double) * (tiles * 4096 + (chol_linv_ ? 0 : T * 4096 + static_cast<size_t>(p.n_pad))) +
+                      sizeof(int) * (T * T + 2 * (T + 1) + 2 * tiles + static_cast<size_t>(C_));
+  size_t free_b = 0, total_b = 0;
+  PV_CUDA(cudaMemGetInfo(&free_b, &total_b));
+  if (need > free_b) {
+    return fail(POVAR_ERR_UNSUPPORTED, "CHOLESKY: tile-sparse factor needs " + std::to_string(need) + " bytes, " +
+                                           std::to_string(free_b) + " bytes free on the device");
+  }
+  int *slot = nullptr, *col_ptr = nullptr, *col_row = nullptr, *row_ptr = nullptr, *row_col = nullptr, *perm = nullptr;
+  PV_ALLOC(chol_dev_.tiles, tiles * 4096);
+  if (!chol_linv_) {   // the same sizes as on the dense path: a handle switched between the two shares them
+    PV_ALLOC(chol_linv_, T * 4096);
+    PV_ALLOC(chol_rhs_, p.n_pad);
+  }
+  PV_ALLOC(slot, T * T);
+  PV_ALLOC(col_ptr, T + 1);
+  PV_ALLOC(row_ptr, T + 1);
+  PV_ALLOC(col_row, tiles);
+  PV_ALLOC(row_col, tiles);
+  PV_ALLOC(perm, C_);
+  auto up = [&](int* dst, const std::vector<int>& src) {
+    return cudaMemcpyAsync(dst, src.data(), sizeof(int) * src.size(), cudaMemcpyHostToDevice, stream_);
+  };
+  PV_CUDA(up(slot, p.slot));
+  PV_CUDA(up(col_ptr, p.col_ptr));
+  PV_CUDA(up(col_row, p.col_row));
+  PV_CUDA(up(row_ptr, p.row_ptr));
+  PV_CUDA(up(row_col, p.row_col));
+  PV_CUDA(up(perm, p.perm));
+  PV_CUDA(cudaStreamSynchronize(stream_));   // the host vectors are pageable
+  chol_dev_.T = p.T;
+  chol_dev_.slot = slot;
+  chol_dev_.col_ptr = col_ptr;
+  chol_dev_.col_row = col_row;
+  chol_dev_.row_ptr = row_ptr;
+  chol_dev_.row_col = row_col;
+  chol_dev_.perm = perm;
+  chol_tiled_ready_ = true;
+  return POVAR_OK;
+}
+
 int Engine::solve_cholesky(double lambda) {
   const int n = 12 * C_;
   const int n_pad = chol_padded(n);
-  if (static_cast<long long>(n_pad) * n_pad * 8 > (96LL << 30)) {
-    return fail(POVAR_ERR_UNSUPPORTED, "CHOLESKY: dense reduced system would exceed 96 GB");
-  }
+  const bool tiled = chol_storage_ == 1 || static_cast<long long>(n_pad) * n_pad * 8 > kCholDenseCap;
+  chol_tiled_active_ = tiled;
   PV_CUDA(cudaEventRecord(ev_[0], stream_));
   int rc = prepare_reduced_system(false, lambda, 0.0);
   if (rc != POVAR_OK) return rc;
-  if (!d_.dense_S) {
-    PV_ALLOC(d_.dense_S, static_cast<size_t>(n_pad) * n_pad);
-    PV_ALLOC(chol_linv_, static_cast<size_t>(n_pad) * 64);
-    PV_ALLOC(chol_rhs_, static_cast<size_t>(n_pad));
+  if (tiled) {
+    if (!chol_tiled_ready_) {   // once per handle, inside this trial's prepare time
+      rc = setup_cholesky_tiles();
+      if (rc != POVAR_OK) return rc;
+    }
+    PV_CUDA(cudaMemsetAsync(chol_dev_.tiles, 0, sizeof(double) * 4096 * static_cast<size_t>(chol_pat_.tiles()), stream_));
+    launch_schur_tiles(d_, mp_, chol_dev_, n_pad, lc());
+  } else {
+    if (!d_.dense_S) PV_ALLOC(d_.dense_S, static_cast<size_t>(n_pad) * n_pad);
+    if (!chol_linv_) {
+      PV_ALLOC(chol_linv_, static_cast<size_t>(n_pad) * 64);
+      PV_ALLOC(chol_rhs_, static_cast<size_t>(n_pad));
+    }
+    PV_CUDA(cudaMemsetAsync(d_.dense_S, 0, sizeof(double) * static_cast<size_t>(n_pad) * n_pad, stream_));
+    launch_schur_lower(d_, mp_, d_.dense_S, n_pad, lc());
   }
-  PV_CUDA(cudaMemsetAsync(d_.dense_S, 0, sizeof(double) * static_cast<size_t>(n_pad) * n_pad, stream_));
-  launch_schur_lower(d_, mp_, d_.dense_S, n_pad, lc());
   PV_CUDA(cudaEventRecord(ev_[1], stream_));
   PV_CUDA(cudaMemsetAsync(chol_rhs_, 0, sizeof(double) * static_cast<size_t>(n_pad), stream_));
-  launch_axpby(d_, n, -1.0, d_.b, 0.0, nullptr, chol_rhs_, lc());
   int* info = d_.flags + 2;
-  launch_cholesky_factor(d_.dense_S, n_pad, chol_linv_, info, lc());
-  launch_cholesky_solve(d_.dense_S, n_pad, chol_linv_, chol_rhs_, info, lc());
-  PV_CUDA(cudaMemcpyAsync(d_.vec_acc, chol_rhs_, sizeof(double) * static_cast<size_t>(n), cudaMemcpyDeviceToDevice, stream_));
+  if (tiled) {
+    launch_perm_gather_neg(C_, chol_dev_.perm, d_.b, chol_rhs_, lc());
+    launch_cholesky_factor_tiles(chol_pat_, chol_dev_, chol_linv_, info, lc());
+    launch_cholesky_solve_tiles(chol_pat_, chol_dev_, chol_linv_, chol_rhs_, info, lc());
+    launch_perm_scatter(C_, chol_dev_.perm, chol_rhs_, d_.vec_acc, lc());
+  } else {
+    launch_axpby(d_, n, -1.0, d_.b, 0.0, nullptr, chol_rhs_, lc());
+    launch_cholesky_factor(d_.dense_S, n_pad, chol_linv_, info, lc());
+    launch_cholesky_solve(d_.dense_S, n_pad, chol_linv_, chol_rhs_, info, lc());
+    PV_CUDA(cudaMemcpyAsync(d_.vec_acc, chol_rhs_, sizeof(double) * static_cast<size_t>(n), cudaMemcpyDeviceToDevice, stream_));
+  }
   int hinfo = 0;
   PV_CUDA(cudaMemcpyAsync(&hinfo, info, sizeof(int), cudaMemcpyDeviceToHost, stream_));
   SeriesCtl h{};
@@ -1588,6 +1667,100 @@ int debug_cholesky(int n, const double* A, const double* b, double* x, int* info
   cudaFree(linv);
   cudaFree(r);
   cudaFree(info);
+  return rc;
+}
+
+// the tile-sparse factorisation and substitution on a caller-supplied symmetric matrix (tests): the pattern is that of
+// the non-zero block x block blocks of A's lower triangle, ordered and factorised symbolically as a handle's S is
+int debug_sparse_cholesky(int n, int block, const double* A, const double* b, double* x, int* info_out,
+                          long long* stored_tiles) {
+  if (n <= 0 || block <= 0 || !A || !b || !x) return POVAR_ERR_INVALID;
+  int ndev = 0;
+  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return POVAR_ERR_NO_DEVICE;
+  const int nb = (n + block - 1) / block;
+  const size_t words = (static_cast<size_t>(nb) + 31) / 32;
+  std::vector<unsigned int> bits(static_cast<size_t>(nb) * words, 0u);
+  for (int a = 0; a < nb; ++a) {
+    for (int c = 0; c <= a; ++c) {
+      bool nz = a == c;
+      for (int i = a * block; i < std::min(n, a * block + block) && !nz; ++i) {
+        for (int j = c * block; j < std::min(i + 1, c * block + block); ++j) nz = nz || A[static_cast<size_t>(i) * n + j] != 0.0;
+      }
+      if (!nz) continue;
+      bits[static_cast<size_t>(a) * words + (c >> 5)] |= 1u << (c & 31);
+      bits[static_cast<size_t>(c) * words + (a >> 5)] |= 1u << (a & 31);
+    }
+  }
+  CholPattern p;
+  chol_symbolic(nb, block, bits, 0, &p);
+  // original row of every row of the factor order, -1 on padding (identity)
+  std::vector<int> at(nb), orig(p.n_pad, -1);
+  for (int c = 0; c < nb; ++c) at[p.perm[c]] = c;
+  for (int R = 0; R < p.n_pad; ++R) {
+    const int pos = R / block;
+    if (pos < nb && block * at[pos] + R % block < n) orig[R] = block * at[pos] + R % block;
+  }
+  const size_t tiles = static_cast<size_t>(p.tiles()), T = static_cast<size_t>(p.T);
+  std::vector<double> H(tiles * 4096, 0.0), r(p.n_pad, 0.0);
+  for (int J = 0; J < p.T; ++J) {
+    for (int q = p.col_ptr[J]; q < p.col_ptr[J + 1]; ++q) {
+      const int I = p.col_row[q];
+      for (int rr = 0; rr < 64; ++rr) {
+        for (int cc = 0; cc < 64; ++cc) {
+          const int R = I * 64 + rr, Cc = J * 64 + cc;
+          if (R < Cc) continue;
+          const int oi = orig[R], oj = orig[Cc];
+          H[static_cast<size_t>(q) * 4096 + rr * 64 + cc] =
+              (oi < 0 || oj < 0) ? (R == Cc ? 1.0 : 0.0)
+                                 : A[static_cast<size_t>(std::max(oi, oj)) * n + std::min(oi, oj)];
+        }
+      }
+    }
+  }
+  for (int R = 0; R < p.n_pad; ++R) r[R] = orig[R] >= 0 ? b[orig[R]] : 0.0;
+  double *dt = nullptr, *linv = nullptr, *dr = nullptr;
+  int *slot = nullptr, *col_ptr = nullptr, *col_row = nullptr, *row_ptr = nullptr, *row_col = nullptr, *info = nullptr;
+  int rc = POVAR_OK;
+  auto ok = [&](cudaError_t e) {
+    if (e != cudaSuccess) rc = POVAR_ERR_CUDA;
+    return e == cudaSuccess;
+  };
+  auto up = [&](int** dst, const std::vector<int>& src) {
+    return ok(cudaMalloc(dst, sizeof(int) * std::max<size_t>(src.size(), 1))) &&
+           ok(cudaMemcpy(*dst, src.data(), sizeof(int) * src.size(), cudaMemcpyHostToDevice));
+  };
+  if (ok(cudaSetDevice(0)) && ok(cudaMalloc(&dt, sizeof(double) * H.size())) &&
+      ok(cudaMalloc(&linv, sizeof(double) * T * 4096)) && ok(cudaMalloc(&dr, sizeof(double) * r.size())) &&
+      ok(cudaMalloc(&info, sizeof(int))) &&
+      ok(cudaMemcpy(dt, H.data(), sizeof(double) * H.size(), cudaMemcpyHostToDevice)) &&
+      ok(cudaMemcpy(dr, r.data(), sizeof(double) * r.size(), cudaMemcpyHostToDevice)) && up(&slot, p.slot) &&
+      up(&col_ptr, p.col_ptr) && up(&col_row, p.col_row) && up(&row_ptr, p.row_ptr) && up(&row_col, p.row_col)) {
+    CholTilesDev s;
+    s.T = p.T;
+    s.tiles = dt;
+    s.slot = slot;
+    s.col_ptr = col_ptr;
+    s.col_row = col_row;
+    s.row_ptr = row_ptr;
+    s.row_col = row_col;
+    LaunchCfg lc{};
+    launch_cholesky_factor_tiles(p, s, linv, info, lc);
+    launch_cholesky_solve_tiles(p, s, linv, dr, info, lc);
+    int hinfo = 0;
+    ok(cudaMemcpy(&hinfo, info, sizeof(int), cudaMemcpyDeviceToHost));
+    ok(cudaMemcpy(r.data(), dr, sizeof(double) * r.size(), cudaMemcpyDeviceToHost));
+    ok(cudaGetLastError());
+    for (int R = 0; R < p.n_pad; ++R) {
+      if (orig[R] >= 0) x[orig[R]] = r[R];
+    }
+    if (info_out) *info_out = hinfo;
+    if (stored_tiles) *stored_tiles = p.tiles();
+  }
+  for (void* q : {static_cast<void*>(dt), static_cast<void*>(linv), static_cast<void*>(dr), static_cast<void*>(slot),
+                  static_cast<void*>(col_ptr), static_cast<void*>(col_row), static_cast<void*>(row_ptr),
+                  static_cast<void*>(row_col), static_cast<void*>(info)}) {
+    cudaFree(q);
+  }
   return rc;
 }
 
@@ -1815,6 +1988,17 @@ int64_t Engine::debug_read(const char* name, double* out, int64_t capacity) {
     return 1;
   }
   else if (n == "obs_slot") isrc = d_.ix.obs_slot, count = nnz_;
+  else if (n == "chol_perm" || n == "chol_tiles") {   // tile-sparse CHOLESKY: 0 elements on the dense path
+    count = !chol_tiled_active_ ? 0 : (n == "chol_tiles" ? 1 : C_);
+    if (!out || count == 0) return count;
+    if (capacity < count) {
+      fail(POVAR_ERR_INVALID, "debug_read: buffer too small");
+      return POVAR_ERR_INVALID;
+    }
+    if (n == "chol_tiles") out[0] = static_cast<double>(chol_pat_.tiles());
+    else for (int c = 0; c < C_; ++c) out[c] = chol_pat_.perm[c];
+    return count;
+  }
   else {
     fail(POVAR_ERR_INVALID, "debug_read: unknown array '" + n + "'");
     return POVAR_ERR_INVALID;

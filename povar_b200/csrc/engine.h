@@ -52,6 +52,7 @@ class Engine {
   int world_size() const { return world_; }
   bool peer_exchange_active() const { return peer_ok_; }
   void debug_set_window(int cams) { d_.debug_window_cams = cams; }
+  void debug_set_cholesky_storage(int mode) { chol_storage_ = mode; }
   int rank() const { return rank_; }
 
  private:
@@ -68,6 +69,7 @@ class Engine {
   int solve_power(bool joint, double lambda);
   int solve_pcg(bool joint, double lambda);
   int solve_cholesky(double lambda);
+  int setup_cholesky_tiles();
   int prepare_reduced_system(bool joint, double lambda, double lambda_lm);
   int schur_product(bool joint, const double* p, double* out, bool skip_when_done);
   int e0_product(bool joint, bool skip_when_done, bool fused_reduce);
@@ -104,6 +106,12 @@ class Engine {
   void count_series_terms(int terms);
   double* chol_linv_ = nullptr;   // CHOLESKY: inverses of the factor's diagonal tiles [n_pad / 64][64][64]
   double* chol_rhs_ = nullptr;    // CHOLESKY: padded right-hand side / solution [n_pad]
+  // CHOLESKY on tile-sparse storage (when the dense matrix would exceed kCholDenseCap, or forced)
+  int chol_storage_ = 0;          // povar_debug_set_cholesky_storage: 0 automatic, 1 tile-sparse
+  bool chol_tiled_ready_ = false; // the pattern below is built (at the first tile-sparse solve)
+  bool chol_tiled_active_ = false;  // the last CHOLESKY solve used the tiles
+  CholPattern chol_pat_;
+  CholTilesDev chol_dev_;
   // distributed
   int rank_ = 0, world_ = 1, device_ = 0;
   void* nccl_comm_ = nullptr;

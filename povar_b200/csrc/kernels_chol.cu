@@ -16,8 +16,16 @@
 //              that profiles as a contraction (DESIGN.md 4).
 //   solve      forward / backward substitution tile row by tile row with the stored inverses of the diagonal
 //              factors.
-// Dense storage, row-major, leading dimension n_pad = 12 C rounded up to 64 (identity on the padding).
+// Two storages of S and its factor, one set of kernels: the kernels take an addressing policy.
+//   dense        the whole matrix, row-major, leading dimension n_pad = 12 C rounded up to 64 (identity on the
+//                padding), cameras in their own order;
+//   tile-sparse  only the 64x64 tiles of the factor that can be non-zero (CholPattern, host/chol_symbolic.cpp),
+//                each stored contiguously (ld = 64) in slot order, cameras in the fill-reducing order perm; the
+//                panel and the update walk the stored tiles of a column, the backward substitution those of a row.
+// The dense instantiations compute what they computed before the policies existed, bit for bit.
 #include <cuda_runtime.h>
+
+#include <cassert>
 
 #include "device_math.cuh"
 #include "povar_internal.h"
@@ -61,13 +69,89 @@ __device__ __forceinline__ void pose_wk(const Cam3x4& cam, double u, double v, c
 
 constexpr int kRowWarps = 8;
 
+// ---- addressing policies --------------------------------------------------------------------------
+// element (R, C) and element (r, cc) of the 12x12 block (ci, cj), cj <= ci in camera order, of S; stores(..): whether
+// the assembly writes that element of the block at all
+struct DenseS {
+  double* S;
+  long long ld;
+  __device__ bool stores(int, int, int, int) const { return true; }
+  __device__ double* elem(long long R, long long C) const { return S + R * ld + C; }
+  __device__ double* block(int ci, int cj, int r, int cc) const {
+    return S + (static_cast<long long>(ci) * 12 + r) * ld + (static_cast<long long>(cj) * 12 + cc);
+  }
+};
+// rows of camera c at 12 perm[c] ..; a block that lands in the upper triangle of that order is stored transposed.
+// Only the lower triangle of a diagonal block is written: rows 12 p .. 12 p + 11 of a camera can straddle two tiles,
+// and the upper part of its block would then fall into tile (I, I + 1), which is not stored.
+struct TiledS {
+  double* tiles;
+  const int* slot;
+  const int* perm;
+  int T;
+  __device__ bool stores(int ci, int cj, int r, int cc) const { return ci != cj || cc <= r; }
+  __device__ double* elem(long long R, long long C) const {
+    const int s = slot[(R >> 6) * T + (C >> 6)];
+    assert(s >= 0);   // every tile the assembly writes is in the pattern of the factor
+    return tiles + static_cast<size_t>(s) * (kNB * kNB) + (R & 63) * kNB + (C & 63);
+  }
+  __device__ double* block(int ci, int cj, int r, int cc) const {
+    const long long pi = perm[ci], pj = perm[cj];
+    return pi >= pj ? elem(pi * 12 + r, pj * 12 + cc) : elem(pj * 12 + cc, pi * 12 + r);
+  }
+};
+
+// tiles of the factor: tile(I, J); below(k, i) the i-th stored tile row under the diagonal of column k; left(k, i)
+// the i-th stored tile column left of the diagonal of row k; pair(k, ..) the tiles (ti, tj), tj <= ti, the update
+// of column k writes from this thread block
+struct DenseTiles {
+  double* S;
+  long long ld;
+  __device__ double* tile(int I, int J) const {
+    return S + (static_cast<long long>(I) * kNB) * ld + static_cast<long long>(J) * kNB;
+  }
+  __device__ int below(int k, int i) const { return k + 1 + i; }
+  __device__ int left(int, int i) const { return i; }
+  __device__ bool pair(int k, int& ti, int& tj) const {
+    ti = k + 1 + static_cast<int>(blockIdx.x);
+    tj = k + 1 + static_cast<int>(blockIdx.y);
+    return tj <= ti;
+  }
+};
+struct SparseTiles {
+  double* tiles;
+  const int* slot;
+  const int* col_ptr;
+  const int* col_row;
+  const int* row_ptr;
+  const int* row_col;
+  int T;
+  static constexpr long long ld = kNB;
+  __device__ double* tile(int I, int J) const {
+    return tiles + static_cast<size_t>(slot[static_cast<long long>(I) * T + J]) * (kNB * kNB);
+  }
+  __device__ int below(int k, int i) const { return col_row[col_ptr[k] + 1 + i]; }
+  __device__ int left(int k, int i) const { return row_col[row_ptr[k] + i]; }
+  // blockIdx.x = i (i + 1) / 2 + j, j <= i, over the stored tiles below the diagonal of column k
+  __device__ bool pair(int k, int& ti, int& tj) const {
+    const long long p = blockIdx.x;
+    int i = static_cast<int>((sqrt(8.0 * static_cast<double>(p) + 1.0) - 1.0) * 0.5);
+    while (static_cast<long long>(i + 1) * (i + 2) / 2 <= p) ++i;
+    while (static_cast<long long>(i) * (i + 1) / 2 > p) --i;
+    const int j = static_cast<int>(p - static_cast<long long>(i) * (i + 1) / 2);
+    ti = below(k, i);
+    tj = below(k, j);
+    return true;
+  }
+};
+
 // block row i of S (lower triangle): S_ij -= (s_i s_j^T) o [(Wk_i^T Hll^-1 Wk_j) (x) (Xt Xt^T)] summed over the
 // landmarks l seen by both cameras, in the order of camera i's observation list (landmarks ascending)
+template <class Addr>
 __global__ void __launch_bounds__(32 * kRowWarps)
 k_schur_rows(DeviceIndex ix, const double* __restrict__ P, const double* __restrict__ X, double c1, double c2,
              Robust rb, const double* __restrict__ lm_scale, const double* __restrict__ hll_inv,
-             const double* __restrict__ pose_scale, const double* __restrict__ Bmat, double* __restrict__ S,
-             long long ld) {
+             const double* __restrict__ pose_scale, const double* __restrict__ Bmat, Addr S) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   for (int ci = blockIdx.x; ci < ix.C; ci += gridDim.x) {
     Cam3x4 cam_i;
@@ -111,6 +195,7 @@ k_schur_rows(DeviceIndex ix, const double* __restrict__ P, const double* __restr
         const double* sj = pose_scale + 12 * static_cast<size_t>(cj);
         for (int t = lane; t < 144; t += 32) {
           const int r = t / 12, cc = t % 12;
+          if (!S.stores(ci, cj, r, cc)) continue;
           double q = 0.0;
 #pragma unroll
           for (int a = 0; a < 3; ++a) {
@@ -118,7 +203,7 @@ k_schur_rows(DeviceIndex ix, const double* __restrict__ P, const double* __restr
             for (int b2 = 0; b2 < 3; ++b2) q = (a == (r >> 2) && b2 == (cc >> 2)) ? Q[a][b2] : q;
           }
           const double val = si[r] * sj[cc] * q * x[r & 3] * x[cc & 3];
-          double* dst = S + (static_cast<long long>(ci) * 12 + r) * ld + (static_cast<long long>(cj) * 12 + cc);
+          double* dst = S.block(ci, cj, r, cc);
           *dst -= val;
         }
       }
@@ -128,27 +213,29 @@ k_schur_rows(DeviceIndex ix, const double* __restrict__ P, const double* __restr
     if (ci % kRowWarps == warp) {
       for (int t = lane; t < 144; t += 32) {
         const int r = t / 12, cc = t % 12;
-        S[(static_cast<long long>(ci) * 12 + r) * ld + (static_cast<long long>(ci) * 12 + cc)] +=
-            Bmat[144 * static_cast<size_t>(ci) + t];
+        if (S.stores(ci, ci, r, cc)) *S.block(ci, ci, r, cc) += Bmat[144 * static_cast<size_t>(ci) + t];
       }
     }
   }
 }
 
 // identity on the padding rows
-__global__ void k_pad_identity(int n, int n_pad, double* __restrict__ S, long long ld) {
+template <class Addr>
+__global__ void k_pad_identity(int n, int n_pad, Addr S) {
   const int i = n + blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < n_pad) S[static_cast<long long>(i) * ld + i] = 1.0;
+  if (i < n_pad) *S.elem(i, i) = 1.0;
 }
 
 // ---- factorisation --------------------------------------------------------------------------------
 // diagonal tile k: A = L L^T in shared memory (lower part read), L written back with a zero upper part,
 // L^-1 written to linv[k].  info != 0: a pivot was not positive (the matrix is not positive definite).
+template <class Tiles>
 __global__ void __launch_bounds__(256)
-k_potrf_tile(double* __restrict__ S, long long ld, int k, double* __restrict__ linv, int* __restrict__ info) {
+k_potrf_tile(Tiles S, int k, double* __restrict__ linv, int* __restrict__ info) {
   __shared__ double A[kNB][kNB + 1];
   __shared__ int bad;
-  double* tile = S + (static_cast<long long>(k) * kNB) * ld + static_cast<long long>(k) * kNB;
+  double* tile = S.tile(k, k);
+  const long long ld = S.ld;
   if (*info != 0) return;   // an earlier tile was not positive definite
   if (threadIdx.x == 0) bad = 0;
   for (int t = threadIdx.x; t < kNB * kNB; t += blockDim.x) {
@@ -202,23 +289,26 @@ k_potrf_tile(double* __restrict__ S, long long ld, int k, double* __restrict__ l
 
 // One 64x64 tile product on the FP64 tensor cores, 256 threads: warp w owns rows 8 w .. 8 w + 7 of the tile and
 // all eight 8-column fragments.
-//   kUpdate:  C(ti, tj) -= A(ti, k) A(tj, k)^T   for k < tj <= ti   (trailing update; grid = (m, m), upper skipped)
+//   kUpdate:  C(ti, tj) -= A(ti, k) A(tj, k)^T   for k < tj <= ti   (trailing update; dense: grid = (m, m), upper
+//                                                                      skipped; tile-sparse: one block per pair)
 //   kPanel:   A(ti, k)  = A(ti, k) Linv_k^T      for ti > k          (the panel below the diagonal tile)
 enum TileMode { kUpdate = 0, kPanel = 1 };
 
-template <int MODE>
+template <int MODE, class Tiles>
 __global__ void __launch_bounds__(256)
-k_tile_gemm(double* __restrict__ S, long long ld, int k, const double* __restrict__ linv,
-            const int* __restrict__ info) {
+k_tile_gemm(Tiles S, int k, const double* __restrict__ linv, const int* __restrict__ info) {
   if (*info != 0) return;
   __shared__ double sA[kNB][kKC + kPad];
   __shared__ double sB[kNB][kKC + kPad];
-  const int ti = k + 1 + static_cast<int>(blockIdx.x);
-  const int tj = MODE == kUpdate ? k + 1 + static_cast<int>(blockIdx.y) : k;
-  if (MODE == kUpdate && tj > ti) return;
-  const double* Ap = S + (static_cast<long long>(ti) * kNB) * ld + static_cast<long long>(k) * kNB;
-  const double* Bp = MODE == kUpdate ? S + (static_cast<long long>(tj) * kNB) * ld + static_cast<long long>(k) * kNB
-                                     : linv + static_cast<size_t>(k) * kNB * kNB;
+  const long long ld = S.ld;
+  int ti = 0, tj = k;
+  if (MODE == kUpdate) {
+    if (!S.pair(k, ti, tj)) return;
+  } else {
+    ti = S.below(k, static_cast<int>(blockIdx.x));
+  }
+  const double* Ap = S.tile(ti, k);
+  const double* Bp = MODE == kUpdate ? S.tile(tj, k) : linv + static_cast<size_t>(k) * kNB * kNB;
   const long long ldb = MODE == kUpdate ? ld : kNB;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int fr = lane >> 2, fk = lane & 3;
@@ -241,8 +331,7 @@ k_tile_gemm(double* __restrict__ S, long long ld, int k, const double* __restric
     }
   }
   // C fragment: row fr, columns 2 fk, 2 fk + 1 of the 8x8 tile
-  double* Cp = MODE == kUpdate ? S + (static_cast<long long>(ti) * kNB) * ld + static_cast<long long>(tj) * kNB
-                               : S + (static_cast<long long>(ti) * kNB) * ld + static_cast<long long>(k) * kNB;
+  double* Cp = MODE == kUpdate ? S.tile(ti, tj) : S.tile(ti, k);
   if (MODE == kPanel) __syncthreads();   // every warp has read the tile it is about to overwrite
 #pragma unroll
   for (int n = 0; n < 8; ++n) {
@@ -278,38 +367,55 @@ k_solve_diag(int k, const double* __restrict__ linv, double* __restrict__ r, con
   r[static_cast<size_t>(k) * kNB + i] = s;
 }
 
-// forward: r_i -= L(i, k) x_k for the rows below tile row k (one thread per row)
+// forward: r_i -= L(i, k) x_k for the rows of the stored tiles below tile row k (one thread per row; `rows` =
+// 64 x those tiles)
+template <class Tiles>
 __global__ void __launch_bounds__(256)
-k_solve_fwd_update(int k, int n_pad, const double* __restrict__ S, long long ld, double* __restrict__ r,
-                   const int* __restrict__ info) {
+k_solve_fwd_update(Tiles S, int k, int rows, double* __restrict__ r, const int* __restrict__ info) {
   if (*info != 0) return;
   __shared__ double xk[kNB];
   if (threadIdx.x < kNB) xk[threadIdx.x] = r[static_cast<size_t>(k) * kNB + threadIdx.x];
   __syncthreads();
-  const int row = (k + 1) * kNB + blockIdx.x * blockDim.x + threadIdx.x;
-  if (row >= n_pad) return;
-  const double* a = S + static_cast<long long>(row) * ld + static_cast<long long>(k) * kNB;
+  const int idx = blockIdx.x * blockDim.x + threadIdx.x;
+  if (idx >= rows) return;
+  const int ti = S.below(k, idx / kNB), rr = idx % kNB;
+  const double* a = S.tile(ti, k) + static_cast<long long>(rr) * S.ld;
   double s = 0.0;
 #pragma unroll 8
   for (int m = 0; m < kNB; ++m) s += a[m] * xk[m];
-  r[row] -= s;
+  r[static_cast<size_t>(ti) * kNB + rr] -= s;
 }
 
-// backward: r_j -= L(k, j)^T x_k for the columns left of tile column k (one thread per column)
+// backward: r_j -= L(k, j)^T x_k for the columns of the stored tiles left of tile column k (one thread per column;
+// `cols` = 64 x those tiles)
+template <class Tiles>
 __global__ void __launch_bounds__(256)
-k_solve_bwd_update(int k, const double* __restrict__ S, long long ld, double* __restrict__ r,
-                   const int* __restrict__ info) {
+k_solve_bwd_update(Tiles S, int k, int cols, double* __restrict__ r, const int* __restrict__ info) {
   if (*info != 0) return;
   __shared__ double xk[kNB];
   if (threadIdx.x < kNB) xk[threadIdx.x] = r[static_cast<size_t>(k) * kNB + threadIdx.x];
   __syncthreads();
-  const int col = blockIdx.x * blockDim.x + threadIdx.x;
-  if (col >= k * kNB) return;
-  const double* a = S + (static_cast<long long>(k) * kNB) * ld + col;
+  const int idx = blockIdx.x * blockDim.x + threadIdx.x;
+  if (idx >= cols) return;
+  const int tj = S.left(k, idx / kNB), cc = idx % kNB;
+  const double* a = S.tile(k, tj) + cc;
+  const long long ld = S.ld;
   double s = 0.0;
 #pragma unroll 8
   for (int m = 0; m < kNB; ++m) s += a[static_cast<long long>(m) * ld] * xk[m];
-  r[col] -= s;
+  r[static_cast<size_t>(tj) * kNB + cc] -= s;
+}
+
+// the right-hand side into the factor order and the solution back
+__global__ void k_perm_gather_neg(int n, const int* __restrict__ perm, const double* __restrict__ b,
+                                  double* __restrict__ r) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n) r[12 * static_cast<size_t>(perm[i / 12]) + i % 12] = -b[i];
+}
+__global__ void k_perm_scatter(int n, const int* __restrict__ perm, const double* __restrict__ r,
+                               double* __restrict__ x) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n) x[i] = r[12 * static_cast<size_t>(perm[i / 12]) + i % 12];
 }
 
 }  // namespace
@@ -320,10 +426,24 @@ void launch_schur_lower(const DeviceState& d, const ModelParams& mp, double* S, 
   const Robust rb = {mp.robust_norm, mp.huber};
   int blocks = d.ix.C;
   if (blocks > sm_count() * 8) blocks = sm_count() * 8;
+  const DenseS a{S, n_pad};
   k_schur_rows<<<blocks, 32 * kRowWarps, 0, lc.stream>>>(d.ix, d.P, d.X, mp.c1, mp.c2, rb, d.lm_scale, d.hll_inv,
-                                                         d.pose_scale, d.Bmat, S, n_pad);
+                                                         d.pose_scale, d.Bmat, a);
   const int n = 12 * d.ix.C;
-  if (n_pad > n) k_pad_identity<<<1, kNB, 0, lc.stream>>>(n, n_pad, S, n_pad);
+  if (n_pad > n) k_pad_identity<<<1, kNB, 0, lc.stream>>>(n, n_pad, a);
+  count(lc, n_pad > n ? 2 : 1);
+}
+
+void launch_schur_tiles(const DeviceState& d, const ModelParams& mp, const CholTilesDev& s, int n_pad,
+                        const LaunchCfg& lc) {
+  const Robust rb = {mp.robust_norm, mp.huber};
+  int blocks = d.ix.C;
+  if (blocks > sm_count() * 8) blocks = sm_count() * 8;
+  const TiledS a{s.tiles, s.slot, s.perm, s.T};
+  k_schur_rows<<<blocks, 32 * kRowWarps, 0, lc.stream>>>(d.ix, d.P, d.X, mp.c1, mp.c2, rb, d.lm_scale, d.hll_inv,
+                                                         d.pose_scale, d.Bmat, a);
+  const int n = 12 * d.ix.C;
+  if (n_pad > n) k_pad_identity<<<1, kNB, 0, lc.stream>>>(n, n_pad, a);
   count(lc, n_pad > n ? 2 : 1);
 }
 
@@ -331,15 +451,16 @@ void launch_schur_lower(const DeviceState& d, const ModelParams& mp, double* S, 
 // tile with a non-positive pivot, 0 if the matrix is positive definite
 void launch_cholesky_factor(double* S, int n_pad, double* linv, int* info, const LaunchCfg& lc) {
   const int T = n_pad / kNB;
+  const DenseTiles a{S, n_pad};
   cudaMemsetAsync(info, 0, sizeof(int), lc.stream);
   int launches = 0;
   for (int k = 0; k < T; ++k) {
-    k_potrf_tile<<<1, 256, 0, lc.stream>>>(S, n_pad, k, linv, info);
+    k_potrf_tile<<<1, 256, 0, lc.stream>>>(a, k, linv, info);
     ++launches;
     const int m = T - 1 - k;
     if (m > 0) {
-      k_tile_gemm<kPanel><<<dim3(m, 1), 256, 0, lc.stream>>>(S, n_pad, k, linv, info);
-      k_tile_gemm<kUpdate><<<dim3(m, m), 256, 0, lc.stream>>>(S, n_pad, k, linv, info);
+      k_tile_gemm<kPanel><<<dim3(m, 1), 256, 0, lc.stream>>>(a, k, linv, info);
+      k_tile_gemm<kUpdate><<<dim3(m, m), 256, 0, lc.stream>>>(a, k, linv, info);
       launches += 2;
     }
   }
@@ -350,13 +471,14 @@ void launch_cholesky_factor(double* S, int n_pad, double* linv, int* info, const
 void launch_cholesky_solve(const double* S, int n_pad, const double* linv, double* r, const int* info,
                            const LaunchCfg& lc) {
   const int T = n_pad / kNB;
+  const DenseTiles a{const_cast<double*>(S), n_pad};
   int launches = 0;
   for (int k = 0; k < T; ++k) {
     k_solve_diag<false><<<1, kNB, 0, lc.stream>>>(k, linv, r, info);
     ++launches;
     const int rows = n_pad - (k + 1) * kNB;
     if (rows > 0) {
-      k_solve_fwd_update<<<(rows + 255) / 256, 256, 0, lc.stream>>>(k, n_pad, S, n_pad, r, info);
+      k_solve_fwd_update<<<(rows + 255) / 256, 256, 0, lc.stream>>>(a, k, rows, r, info);
       ++launches;
     }
   }
@@ -365,11 +487,75 @@ void launch_cholesky_solve(const double* S, int n_pad, const double* linv, doubl
     ++launches;
     const int cols = k * kNB;
     if (cols > 0) {
-      k_solve_bwd_update<<<(cols + 255) / 256, 256, 0, lc.stream>>>(k, S, n_pad, r, info);
+      k_solve_bwd_update<<<(cols + 255) / 256, 256, 0, lc.stream>>>(a, k, cols, r, info);
       ++launches;
     }
   }
   count(lc, launches);
+}
+
+namespace {
+SparseTiles sparse_tiles(const CholTilesDev& s) {
+  return SparseTiles{s.tiles, s.slot, s.col_ptr, s.col_row, s.row_ptr, s.row_col, s.T};
+}
+}  // namespace
+
+// the same factorisation over the stored tiles only: column k's panel and the pairs of its stored tiles; *info as
+// above, tiles numbered in the factor order
+void launch_cholesky_factor_tiles(const CholPattern& p, const CholTilesDev& s, double* linv, int* info,
+                                  const LaunchCfg& lc) {
+  const SparseTiles a = sparse_tiles(s);
+  cudaMemsetAsync(info, 0, sizeof(int), lc.stream);
+  int launches = 0;
+  for (int k = 0; k < p.T; ++k) {
+    k_potrf_tile<<<1, 256, 0, lc.stream>>>(a, k, linv, info);
+    ++launches;
+    const long long m = p.col_ptr[k + 1] - p.col_ptr[k] - 1;
+    if (m > 0) {
+      k_tile_gemm<kPanel><<<dim3(static_cast<unsigned>(m), 1), 256, 0, lc.stream>>>(a, k, linv, info);
+      k_tile_gemm<kUpdate><<<dim3(static_cast<unsigned>(m * (m + 1) / 2), 1), 256, 0, lc.stream>>>(a, k, linv, info);
+      launches += 2;
+    }
+  }
+  count(lc, launches);
+}
+
+// forward substitution down the column lists, backward up the row lists
+void launch_cholesky_solve_tiles(const CholPattern& p, const CholTilesDev& s, const double* linv, double* r,
+                                 const int* info, const LaunchCfg& lc) {
+  const SparseTiles a = sparse_tiles(s);
+  int launches = 0;
+  for (int k = 0; k < p.T; ++k) {
+    k_solve_diag<false><<<1, kNB, 0, lc.stream>>>(k, linv, r, info);
+    ++launches;
+    const int rows = (p.col_ptr[k + 1] - p.col_ptr[k] - 1) * kNB;
+    if (rows > 0) {
+      k_solve_fwd_update<<<(rows + 255) / 256, 256, 0, lc.stream>>>(a, k, rows, r, info);
+      ++launches;
+    }
+  }
+  for (int k = p.T - 1; k >= 0; --k) {
+    k_solve_diag<true><<<1, kNB, 0, lc.stream>>>(k, linv, r, info);
+    ++launches;
+    const int cols = (p.row_ptr[k + 1] - p.row_ptr[k] - 1) * kNB;
+    if (cols > 0) {
+      k_solve_bwd_update<<<(cols + 255) / 256, 256, 0, lc.stream>>>(a, k, cols, r, info);
+      ++launches;
+    }
+  }
+  count(lc, launches);
+}
+
+void launch_perm_gather_neg(int C, const int* perm, const double* b, double* r, const LaunchCfg& lc) {
+  const int n = 12 * C;
+  k_perm_gather_neg<<<(n + 255) / 256, 256, 0, lc.stream>>>(n, perm, b, r);
+  count(lc);
+}
+
+void launch_perm_scatter(int C, const int* perm, const double* r, double* x, const LaunchCfg& lc) {
+  const int n = 12 * C;
+  k_perm_scatter<<<(n + 255) / 256, 256, 0, lc.stream>>>(n, perm, r, x);
+  count(lc);
 }
 
 }  // namespace povar

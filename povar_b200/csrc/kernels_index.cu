@@ -381,4 +381,33 @@ cudaError_t build_device_sell(int L, int num_cams, int n, int window, int max_de
   return cudaGetLastError();
 }
 
+namespace {
+// one warp per landmark: bits (a, b) and (b, a) for every pair of its cameras, the diagonal included.  atomicOr is
+// idempotent, so the bitmap does not depend on the order.
+__global__ void __launch_bounds__(kBlock)
+k_covisibility(int L, int words, const int* __restrict__ lm_ptr, const int* __restrict__ obs_cam,
+               unsigned int* __restrict__ bits) {
+  const int lane = threadIdx.x & 31;
+  const int l = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  if (l >= L) return;
+  const int ob = lm_ptr[l], deg = lm_ptr[l + 1] - ob;
+  for (long long p = lane; p < static_cast<long long>(deg) * deg; p += 32) {
+    const int a = obs_cam[ob + static_cast<int>(p / deg)], b = obs_cam[ob + static_cast<int>(p % deg)];
+    atomicOr(bits + static_cast<size_t>(a) * words + (b >> 5), 1u << (b & 31));
+  }
+}
+}  // namespace
+
+cudaError_t build_covisibility(int L, int C, const int* lm_ptr, const int* obs_cam, unsigned int* bits,
+                               const LaunchCfg& lc) {
+  const int words = (C + 31) / 32;
+  cudaError_t e = cudaMemsetAsync(bits, 0, sizeof(unsigned int) * static_cast<size_t>(C) * words, lc.stream);
+  if (e != cudaSuccess || L <= 0) return e;
+  const long long threads = 32LL * L;
+  k_covisibility<<<static_cast<unsigned>((threads + kBlock - 1) / kBlock), kBlock, 0, lc.stream>>>(L, words, lm_ptr,
+                                                                                                  obs_cam, bits);
+  if (lc.launch_counter) *lc.launch_counter += 1;
+  return cudaGetLastError();
+}
+
 }  // namespace povar

@@ -336,6 +336,46 @@ void launch_cholesky_factor(double* S, int n_pad, double* linv, int* info, const
 void launch_cholesky_solve(const double* S, int n_pad, const double* linv, double* r, const int* info,
                            const LaunchCfg& lc);
 void launch_finite_check(const DeviceState& d, int n, const double* x, const LaunchCfg& lc);
+
+// CHOLESKY on tile-sparse storage: only the 64x64 tiles of the factor that can be non-zero, in a fill-reducing block
+// order.  Made once per handle on the host (host/chol_symbolic.cpp).
+struct CholPattern {
+  int nb = 0, block = 0, n_pad = 0, T = 0;   // nb blocks (cameras) of `block` rows; T = n_pad / 64 tile rows
+  std::vector<int> perm;               // [nb] position of block c in the factor order (reverse Cuthill-McKee)
+  std::vector<int> col_ptr, col_row;   // [T + 1], [tiles]: tile rows of column J, ascending, the diagonal first;
+                                       // the index into col_row is the tile's slot in storage
+  std::vector<int> row_ptr, row_col;   // [T + 1], [tiles]: tile columns of row I, ascending, the diagonal last
+  std::vector<int> slot;               // [T * T] slot of tile (I, J), I >= J, or -1
+  long long tiles() const { return static_cast<long long>(col_row.size()); }
+};
+// bits: nb rows of (nb + 31) / 32 words, bit (a, b) set when blocks a and b are coupled (symmetric); threads = 0:
+// automatic.  The result does not depend on `threads`.
+void chol_symbolic(int nb, int block, const std::vector<unsigned int>& bits, int threads, CholPattern* out);
+// the camera co-visibility bitmap of a landmark-major index, [C][(C + 31) / 32] words: on the host (tests) and in
+// HBM (kernels_index.cu, one pass over lm_ptr / obs_cam)
+void covisibility_host(int num_cams, int num_lms, const int64_t* lm_ptr, const int32_t* obs_cam,
+                       std::vector<unsigned int>* bits);
+cudaError_t build_covisibility(int L, int C, const int* lm_ptr, const int* obs_cam, unsigned int* bits,
+                               const LaunchCfg& lc);
+// the pattern in device memory
+struct CholTilesDev {
+  int T = 0;
+  double* tiles = nullptr;   // [tiles][64][64], row-major tiles in slot order
+  const int* slot = nullptr;      // [T * T]
+  const int* col_ptr = nullptr;   // [T + 1]
+  const int* col_row = nullptr;
+  const int* row_ptr = nullptr;   // [T + 1]
+  const int* row_col = nullptr;
+  const int* perm = nullptr;      // [C] (assembly of a handle's S)
+};
+// S in the tiled, permuted layout (lower tile triangle of the factor order; tiles must be zero on entry)
+void launch_schur_tiles(const DeviceState& d, const ModelParams& mp, const CholTilesDev& s, int n_pad, const LaunchCfg& lc);
+void launch_cholesky_factor_tiles(const CholPattern& p, const CholTilesDev& s, double* linv, int* info, const LaunchCfg& lc);
+void launch_cholesky_solve_tiles(const CholPattern& p, const CholTilesDev& s, const double* linv, double* r,
+                                 const int* info, const LaunchCfg& lc);
+// r[12 perm[c] + k] = -b[12 c + k] (r zero elsewhere beforehand) / x[12 c + k] = r[12 perm[c] + k]
+void launch_perm_gather_neg(int C, const int* perm, const double* b, double* r, const LaunchCfg& lc);
+void launch_perm_scatter(int C, const int* perm, const double* r, double* x, const LaunchCfg& lc);
 // PCG / RIPCG with the scalars and the termination tests on the device (kernels_schur.cu); every kernel returns
 // at once when ctl->done is set
 enum CgStage { CG_BEGIN = 0, CG_RHO = 1, CG_PQ = 2, CG_ZETA = 3 };
