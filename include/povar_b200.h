@@ -97,6 +97,22 @@ typedef struct povar_problem_desc {
   const double* cam_P;     /* [C*12] 3x4 camera matrices, row-major */
 } povar_problem_desc;
 
+/* An observation list that already lives in device memory, in any order (povar_create_device puts it into the
+ * canonical order above on the GPU).  The handle takes the landmarks [lm_begin, lm_end) of it: landmark l becomes
+ * local landmark l - lm_begin, exactly as in a shard handed to povar_create; the entries of other landmarks are
+ * checked (index ranges, duplicate pairs) but otherwise ignored, so every rank may pass the whole list. */
+typedef struct povar_device_problem_desc {
+  int32_t num_cams;          /* C */
+  int32_t num_lms;           /* landmarks of the whole problem: every obs_lm is < num_lms */
+  int64_t num_obs;           /* entries of the three lists, in any order */
+  int32_t lm_begin, lm_end;  /* landmarks of this handle: 0, num_lms on one GPU; povar_partition_landmarks bounds when sharded */
+  const int32_t* obs_cam;    /* device [num_obs] */
+  const int32_t* obs_lm;     /* device [num_obs] */
+  const double* obs_uv;      /* device [num_obs*2], the convention of povar_problem_desc.obs_uv (after the y flip) */
+  const double* cam_P;       /* device [C*12], row-major 3x4 */
+  void* stream;              /* cudaStream_t on which the caller produced the arrays; NULL = legacy default stream */
+} povar_device_problem_desc;
+
 /* bal/residual_info.hpp:59-102 */
 typedef struct povar_residual_info {
   int64_t num_obs_all;
@@ -123,7 +139,8 @@ typedef struct povar_handle povar_handle;
 int povar_abi_version(void);
 /* sizeof of the public structs as this library was compiled, for bindings that mirror them (ctypes, cgo ...):
  * 0 povar_options, 1 povar_problem_desc, 2 povar_comm_desc, 3 povar_residual_info, 4 povar_iteration,
- * 5 povar_solve_summary, 6 povar_bal_data, 7 povar_ba_log_info, 8 povar_phase_times; -1 for anything else */
+ * 5 povar_solve_summary, 6 povar_bal_data, 7 povar_ba_log_info, 8 povar_phase_times, 9 povar_device_problem_desc;
+ * -1 for anything else */
 int64_t povar_abi_sizeof(int32_t which);
 
 /* BAL text reader for the 15-parameter format written by --create-dataset:
@@ -181,6 +198,18 @@ int povar_comm_finalize(void);
  * comm == NULL means a single GPU (device 0). */
 int povar_create(const povar_problem_desc* desc, const povar_options* opt,
                  const povar_comm_desc* comm, povar_handle** out);
+/* povar_create from device-resident observations (povar_device_problem_desc), in any order.
+ *   - The arrays are read after the work already enqueued on desc->stream: the handle's stream waits on an event
+ *     recorded there; the caller's stream is not synchronised with the host.
+ *   - The arrays are never written, and are no longer needed when the call returns.
+ *   - The canonical order and the index are made on the device; the same observations give the same index arrays,
+ *     and so the same results, as povar_canonical_order + povar_create of the same landmark range.
+ *   - POVAR_ERR_INVALID (text via povar_last_error(NULL)): an index out of range, a duplicate (cam, lm) pair anywhere
+ *     in the list, lm_begin > lm_end or a bound outside [0, num_lms], a pointer that is not device memory of the
+ *     handle's device (comm->device, or 0).  POVAR_ERR_UNSUPPORTED: 2^31 or more entries.  POVAR_ERR_NO_DEVICE
+ *     without a GPU. */
+int povar_create_device(const povar_device_problem_desc* desc, const povar_options* opt,
+                        const povar_comm_desc* comm, povar_handle** out);
 /* povar_destroy frees the device state (back to the device's memory pool, which keeps it for the next handle) and
  * hands the handle's stream, events and 256 bytes of page-locked scratch to the next povar_create on the same device
  * instead of destroying them: a process keeps one such set per handle it ever had alive at the same time. */
@@ -221,6 +250,11 @@ int povar_normalize_joint(povar_handle* h);
 /* cameras [C*12]; landmarks of this shard [num_lms*3] (POVAR_STATE_POSE) or [num_lms*4] (JOINT) */
 int povar_get_state(povar_handle* h, int32_t which, double* cam_P, double* lms);
 int povar_set_state(povar_handle* h, int32_t which, const double* cam_P, const double* lms);
+/* The same in device memory of the handle's device, with the same layouts (set: POVAR_STATE_POSE writes w = 1).
+ * Stream-ordered, no host synchronisation: the copies run after the work enqueued on `stream` (cudaStream_t, NULL =
+ * legacy default stream) so far, and `stream` waits for them.  Either pointer may be NULL. */
+int povar_get_state_device(povar_handle* h, int32_t which, double* cam_P, double* lms, void* stream);
+int povar_set_state_device(povar_handle* h, int32_t which, const double* cam_P, const double* lms, void* stream);
 
 /* ---------- the two-step driver -------------------------------------------------------- */
 

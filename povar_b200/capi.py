@@ -3,6 +3,9 @@
 This is plumbing for the tests, the benchmark and Python callers; the product is the shared
 library.  There is no Python or CPU implementation behind these calls: if the library is
 missing, import fails; if there is no CUDA device, `povar_create` returns POVAR_ERR_NO_DEVICE.
+The logic of its own is argument checking and the conversions around the calls: HostProblem's
+canonical order and shards, DeviceProblem's checks of torch tensors and its shards (torch is
+imported only where a DeviceProblem or a device-state call needs it).
 """
 from __future__ import annotations
 
@@ -52,6 +55,15 @@ class ProblemDesc(C.Structure):
         ("num_cams", C.c_int32), ("num_lms", C.c_int32), ("num_obs", C.c_int64),
         ("lm_ptr", C.POINTER(C.c_int64)), ("obs_cam", C.POINTER(C.c_int32)),
         ("obs_uv", C.POINTER(C.c_double)), ("cam_P", C.POINTER(C.c_double)),
+    ]
+
+
+class DeviceProblemDesc(C.Structure):
+    _fields_ = [
+        ("num_cams", C.c_int32), ("num_lms", C.c_int32), ("num_obs", C.c_int64),
+        ("lm_begin", C.c_int32), ("lm_end", C.c_int32),
+        ("obs_cam", C.c_void_p), ("obs_lm", C.c_void_p), ("obs_uv", C.c_void_p), ("cam_P", C.c_void_p),
+        ("stream", C.c_void_p),
     ]
 
 
@@ -128,6 +140,8 @@ SIGNATURES = {
     "povar_get_timings": (C.c_int, [_H, C.POINTER(PhaseTimes)]),
     "povar_reset_timings": (C.c_int, [_H]),
     "povar_create": (C.c_int, [C.POINTER(ProblemDesc), C.POINTER(Options), C.POINTER(CommDesc), C.POINTER(_H)]),
+    "povar_create_device": (C.c_int, [C.POINTER(DeviceProblemDesc), C.POINTER(Options), C.POINTER(CommDesc),
+                                      C.POINTER(_H)]),
     "povar_destroy": (None, [_H]),
     "povar_last_error": (C.c_char_p, [_H]),
     "povar_init_varproj": (C.c_int, [_H, C.c_double]),
@@ -145,6 +159,8 @@ SIGNATURES = {
     "povar_normalize_joint": (C.c_int, [_H]),
     "povar_get_state": (C.c_int, [_H, C.c_int32, _DP, _DP]),
     "povar_set_state": (C.c_int, [_H, C.c_int32, _DP, _DP]),
+    "povar_get_state_device": (C.c_int, [_H, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "povar_set_state_device": (C.c_int, [_H, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]),
     "povar_bundle_adjust": (C.c_int, [_H, C.POINTER(Options), C.POINTER(Iteration), C.c_int32,
                                       C.POINTER(SolveSummary)]),
     "povar_comm_finalize": (C.c_int, []),
@@ -283,25 +299,100 @@ class HostProblem:
         return hp
 
 
+class DeviceProblem:
+    """A BAL problem whose observations live on the GPU as torch CUDA tensors, in any order: the library orders
+    them on the device (povar_create_device).  cam_P [C, 12] or [C, 3, 4] float64; obs_cam, obs_lm [N] int32;
+    obs_uv [N, 2] float64 after the y flip; all contiguous, on one CUDA device.  num_lms: landmarks of the whole
+    problem (default: max(obs_lm) + 1, which reads one number back); lm_range: the landmarks [begin, end) this
+    handle takes (default: all).  num_lms is that of the range, num_obs the length of the list."""
+
+    def __init__(self, cam_P, obs_cam, obs_lm, obs_uv, num_lms=None, lm_range=None):
+        import torch
+        ts = {"cam_P": cam_P, "obs_cam": obs_cam, "obs_lm": obs_lm, "obs_uv": obs_uv}
+        for name, t in ts.items():
+            if not isinstance(t, torch.Tensor):
+                raise ValueError(f"DeviceProblem: {name} must be a torch tensor")
+            if t.dtype != (torch.int32 if name in ("obs_cam", "obs_lm") else torch.float64):
+                raise ValueError(f"DeviceProblem: {name} has dtype {t.dtype}")
+            if not t.is_contiguous():
+                raise ValueError(f"DeviceProblem: {name} must be contiguous")
+        n = obs_cam.shape[0] if obs_cam.dim() == 1 else -1
+        if obs_cam.dim() != 1 or tuple(obs_lm.shape) != (n,) or tuple(obs_uv.shape) != (n, 2):
+            raise ValueError("DeviceProblem: obs_cam, obs_lm must be [N] and obs_uv [N, 2]")
+        if cam_P.dim() == 0 or cam_P.shape[0] == 0 or cam_P.numel() != cam_P.shape[0] * 12:
+            raise ValueError("DeviceProblem: cam_P must be [C, 12] or [C, 3, 4] with C > 0")
+        if num_lms is not None and int(num_lms) < 0:
+            raise ValueError(f"DeviceProblem: num_lms = {num_lms}")
+        if lm_range is not None:
+            lb, le = int(lm_range[0]), int(lm_range[1])
+            if not 0 <= lb <= le or (num_lms is not None and le > int(num_lms)):
+                raise ValueError(f"DeviceProblem: landmark range [{lb}, {le}) is not inside [0, num_lms = {num_lms}]")
+        for name, t in ts.items():
+            if t.device.type != "cuda":
+                raise ValueError(f"DeviceProblem: {name} must be a CUDA tensor (it is on {t.device})")
+            if t.device != cam_P.device:
+                raise ValueError(f"DeviceProblem: {name} is on {t.device}, cam_P on {cam_P.device}")
+        if num_lms is None:
+            num_lms = int(obs_lm.max().item()) + 1 if n > 0 else 0
+        num_lms = int(num_lms)
+        lb, le = (0, num_lms) if lm_range is None else (int(lm_range[0]), int(lm_range[1]))
+        if le > num_lms:
+            raise ValueError(f"DeviceProblem: landmark range [{lb}, {le}) is not inside [0, num_lms = {num_lms}]")
+        self.cam_P, self.obs_cam, self.obs_lm, self.obs_uv = cam_P, obs_cam, obs_lm, obs_uv
+        self.num_cams = int(cam_P.shape[0])
+        self.num_lms_total = num_lms
+        self.lm_begin, self.lm_end = lb, le
+        self.num_lms = le - lb
+        self.num_obs = int(n)
+        self.device = cam_P.device
+
+    def shard(self, rank: int, world: int) -> "DeviceProblem":
+        """The landmark range of `rank` out of `world` (povar_partition_landmarks on the per-landmark counts of the
+        whole list); every rank keeps the whole list."""
+        import torch
+        counts = torch.bincount(self.obs_lm.long(), minlength=self.num_lms_total)[:self.num_lms_total]
+        lm_ptr = np.zeros(self.num_lms_total + 1, dtype=np.int64)
+        lm_ptr[1:] = torch.cumsum(counts, 0).cpu().numpy()
+        bounds = np.empty(world + 1, dtype=np.int32)
+        rc = load().povar_partition_landmarks(self.num_lms_total, lm_ptr.ctypes.data_as(C.POINTER(C.c_int64)), world,
+                                              bounds.ctypes.data_as(C.POINTER(C.c_int32)))
+        if rc != OK:
+            raise PovarError(rc, "povar_partition_landmarks failed")
+        return DeviceProblem(self.cam_P, self.obs_cam, self.obs_lm, self.obs_uv, self.num_lms_total,
+                             (int(bounds[rank]), int(bounds[rank + 1])))
+
+
 class Solver:
     """Handle wrapper with the reference's Linearizor method names
     (/root/reference/src/rootba_povar/solver/linearizor.hpp:47-82)."""
 
-    def __init__(self, problem: HostProblem, options: Options | None = None, comm: CommDesc | None = None):
+    def __init__(self, problem: HostProblem | DeviceProblem, options: Options | None = None,
+                 comm: CommDesc | None = None):
         self.lib = load()
         self.problem = problem
         self.options = options if options is not None else default_options()
-        desc = ProblemDesc()
-        desc.num_cams = problem.num_cams
-        desc.num_lms = problem.num_lms
-        desc.num_obs = problem.num_obs
-        desc.lm_ptr = problem.lm_ptr.ctypes.data_as(C.POINTER(C.c_int64))
-        desc.obs_cam = problem.obs_cam.ctypes.data_as(C.POINTER(C.c_int32))
-        desc.obs_uv = problem.obs_uv.ctypes.data_as(_DP)
-        desc.cam_P = problem.cam_P.ctypes.data_as(_DP)
+        self.device_index = comm.device if comm else 0   # the handle's CUDA device
         h = _H()
-        rc = self.lib.povar_create(C.byref(desc), C.byref(self.options), C.byref(comm) if comm else None,
-                                   C.byref(h))
+        if isinstance(problem, DeviceProblem):
+            import torch
+            with torch.cuda.device(problem.device):
+                desc = DeviceProblemDesc(problem.num_cams, problem.num_lms_total, problem.num_obs, problem.lm_begin,
+                                         problem.lm_end, problem.obs_cam.data_ptr(), problem.obs_lm.data_ptr(),
+                                         problem.obs_uv.data_ptr(), problem.cam_P.data_ptr(),
+                                         torch.cuda.current_stream().cuda_stream)
+            rc = self.lib.povar_create_device(C.byref(desc), C.byref(self.options), C.byref(comm) if comm else None,
+                                              C.byref(h))
+        else:
+            desc = ProblemDesc()
+            desc.num_cams = problem.num_cams
+            desc.num_lms = problem.num_lms
+            desc.num_obs = problem.num_obs
+            desc.lm_ptr = problem.lm_ptr.ctypes.data_as(C.POINTER(C.c_int64))
+            desc.obs_cam = problem.obs_cam.ctypes.data_as(C.POINTER(C.c_int32))
+            desc.obs_uv = problem.obs_uv.ctypes.data_as(_DP)
+            desc.cam_P = problem.cam_P.ctypes.data_as(_DP)
+            rc = self.lib.povar_create(C.byref(desc), C.byref(self.options), C.byref(comm) if comm else None,
+                                       C.byref(h))
         if rc != OK:
             raise PovarError(rc, self.lib.povar_last_error(None).decode())
         self.h = h
@@ -399,6 +490,39 @@ class Solver:
         Xc = np.ascontiguousarray(X, dtype=np.float64) if X is not None else None
         self._check(self.lib.povar_set_state(self.h, which, _dp(Pc) if Pc is not None else None,
                                              _dp(Xc) if Xc is not None else None))
+
+    def get_state_device(self, which):
+        """-> (P [C, 3, 4], X [L, 3|4]) float64 tensors on the handle's device, written on the current torch stream
+        (no host synchronisation)."""
+        import torch
+        dev = torch.device("cuda", self.device_index)
+        P = torch.empty((self.problem.num_cams, 3, 4), dtype=torch.float64, device=dev)
+        X = torch.empty((self.problem.num_lms, 4 if which == STATE_JOINT else 3), dtype=torch.float64, device=dev)
+        with torch.cuda.device(dev):
+            stream = torch.cuda.current_stream().cuda_stream
+        self._check(self.lib.povar_get_state_device(self.h, which, P.data_ptr(), X.data_ptr(), stream))
+        return P, X
+
+    def set_state_device(self, which, P=None, X=None):
+        """State from float64 CUDA tensors (P [C, 3, 4] or [C, 12], X [L, 3|4]) on the current torch stream."""
+        import torch
+        w = 4 if which == STATE_JOINT else 3
+        want = {"P": self.problem.num_cams * 12, "X": self.problem.num_lms * w}
+        dev = None
+        for name, t in (("P", P), ("X", X)):
+            if t is None:
+                continue
+            if (not isinstance(t, torch.Tensor) or t.device.type != "cuda" or t.dtype != torch.float64
+                    or not t.is_contiguous() or t.numel() != want[name]):
+                raise ValueError(f"set_state_device: {name} must be a contiguous float64 CUDA tensor of "
+                                 f"{want[name]} elements")
+            dev = t.device
+        if dev is None:
+            return
+        with torch.cuda.device(dev):
+            stream = torch.cuda.current_stream().cuda_stream
+        self._check(self.lib.povar_set_state_device(self.h, which, P.data_ptr() if P is not None else None,
+                                                    X.data_ptr() if X is not None else None, stream))
 
     # --- driver and instrumentation
     def bundle_adjust(self, options: Options | None = None):

@@ -23,6 +23,21 @@ struct povar_handle {
 
 static thread_local std::string g_last_global_error;
 
+template <typename F>
+static int make_handle(povar_handle** out, F&& create) {
+  if (!out) return POVAR_ERR_INVALID;
+  *out = nullptr;
+  povar_handle* h = new povar_handle();
+  const int rc = create(&h->engine, &h->create_error);
+  if (rc != POVAR_OK) {
+    g_last_global_error = h->create_error;
+    delete h;
+    return rc;
+  }
+  *out = h;
+  return POVAR_OK;
+}
+
 extern "C" {
 
 int povar_abi_version(void) { return POVAR_ABI_VERSION; }
@@ -38,6 +53,7 @@ int64_t povar_abi_sizeof(int32_t which) {
     case 6: return sizeof(povar_bal_data);
     case 7: return sizeof(povar_ba_log_info);
     case 8: return sizeof(povar_phase_times);
+    case 9: return sizeof(povar_device_problem_desc);
     default: return -1;
   }
 }
@@ -85,17 +101,14 @@ int povar_comm_finalize(void) { return povar::nccl_finalize(); }
 
 int povar_create(const povar_problem_desc* desc, const povar_options* opt, const povar_comm_desc* comm,
                  povar_handle** out) {
-  if (!out) return POVAR_ERR_INVALID;
-  *out = nullptr;
-  povar_handle* h = new povar_handle();
-  const int rc = povar::Engine::create(desc, opt, comm, &h->engine, &h->create_error);
-  if (rc != POVAR_OK) {
-    g_last_global_error = h->create_error;
-    delete h;
-    return rc;
-  }
-  *out = h;
-  return POVAR_OK;
+  return make_handle(out, [&](povar::Engine** e, std::string* err) { return povar::Engine::create(desc, opt, comm, e, err); });
+}
+
+int povar_create_device(const povar_device_problem_desc* desc, const povar_options* opt, const povar_comm_desc* comm,
+                        povar_handle** out) {
+  return make_handle(out, [&](povar::Engine** e, std::string* err) {
+    return povar::Engine::create_device(desc, opt, comm, e, err);
+  });
 }
 
 void povar_destroy(povar_handle* h) {
@@ -188,6 +201,16 @@ int povar_get_state(povar_handle* h, int32_t which, double* cam_P, double* lms) 
 int povar_set_state(povar_handle* h, int32_t which, const double* cam_P, const double* lms) {
   PV_ENGINE(h);
   return e.set_state(which, cam_P, lms);
+}
+
+int povar_get_state_device(povar_handle* h, int32_t which, double* cam_P, double* lms, void* stream) {
+  PV_ENGINE(h);
+  return e.get_state_device(which, cam_P, lms, static_cast<cudaStream_t>(stream));
+}
+
+int povar_set_state_device(povar_handle* h, int32_t which, const double* cam_P, const double* lms, void* stream) {
+  PV_ENGINE(h);
+  return e.set_state_device(which, cam_P, lms, static_cast<cudaStream_t>(stream));
 }
 
 int64_t povar_debug_read(povar_handle* h, const char* name, double* out, int64_t capacity) {

@@ -311,21 +311,6 @@ int sell_window(int landmarks, int max_window) {
   return w;
 }
 
-// Largest degree of a landmark of the sliced-ELL set.  A slice is walked row by row by ONE warp, so a slice of 32
-// rows is a chain of 32 dependent steps (0.76 us each when the SM is not full); on a large shard every warp has
-// dozens of rows anyway, on a small one (a venice-1778 shard on 8 GPUs: one slice of ~5 rows per warp) the few
-// slices of 30 rows set the time of the whole launch (27 us where the median block needs 19).  There the
-// landmarks with more than about twice the rows a warp has anyway go to the warp-per-landmark kernels instead
-// (32 observations per step): 31 -> 22 us per launch with 12, measured on that shard.
-int sell_max_degree(long long nnz, int sms) {
-  const long long rows_per_warp = nnz / (32LL * 32 * sms);   // rows of one resident wave of warps
-  if (rows_per_warp >= 16) return 32;
-  long long t = (2 * rows_per_warp + 3) / 4 * 4;
-  if (t < 8) t = 8;
-  if (t > 32) t = 32;
-  return static_cast<int>(t);
-}
-
 void build_sell(const std::vector<int>& lm_ptr, const int* obs_cam, int num_cams, int max_window,
                 SellLayout* out, int max_deg) {
   const int L = static_cast<int>(lm_ptr.size()) - 1;
@@ -592,6 +577,32 @@ int Engine::create(const povar_problem_desc* desc, const povar_options* opt,
     if (err) *err = "povar_create: more than 2^31 observations in one shard";
     return POVAR_ERR_UNSUPPORTED;
   }
+  return create_with(opt, comm, out, err, [desc](Engine* e) { return e->upload(desc); });
+}
+
+int Engine::create_device(const povar_device_problem_desc* desc, const povar_options* opt,
+                          const povar_comm_desc* comm, Engine** out, std::string* err) {
+  *out = nullptr;
+  const char* bad = nullptr;
+  if (!desc || !opt || desc->num_cams <= 0 || desc->num_lms < 0 || desc->num_obs < 0 || !desc->cam_P ||
+      (desc->num_obs > 0 && (!desc->obs_cam || !desc->obs_lm || !desc->obs_uv))) {
+    bad = "povar_create_device: invalid problem description";
+  } else if (desc->lm_begin < 0 || desc->lm_begin > desc->lm_end || desc->lm_end > desc->num_lms) {
+    bad = "povar_create_device: landmark range [lm_begin, lm_end) is not inside [0, num_lms]";
+  }
+  if (bad) {
+    if (err) *err = bad;
+    return POVAR_ERR_INVALID;
+  }
+  if (desc->num_obs >= (1LL << 31)) {
+    if (err) *err = "povar_create_device: 2^31 or more observations";
+    return POVAR_ERR_UNSUPPORTED;
+  }
+  return create_with(opt, comm, out, err, [desc](Engine* e) { return e->upload_device(desc); });
+}
+
+int Engine::create_with(const povar_options* opt, const povar_comm_desc* comm, Engine** out, std::string* err,
+                        const std::function<int(Engine*)>& upload) {
   const auto t_create = std::chrono::steady_clock::now();
   int ndev = 0;
   if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
@@ -669,7 +680,7 @@ int Engine::create(const povar_problem_desc* desc, const povar_options* opt,
     std::fprintf(stderr, "povar_create: %-28s %8.3f ms\n", "device, stream, scratch",
                  std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_create).count());
   }
-  if (rc == POVAR_OK) rc = e->upload(desc);
+  if (rc == POVAR_OK) rc = upload(e);
   if (rc == POVAR_OK) rc = e->setup_peer_exchange();
   if (rc != POVAR_OK) {
     if (err) *err = e->err_;
@@ -707,6 +718,7 @@ Engine::~Engine() {
   bool clean = stream_ != nullptr && host_out_ != nullptr && cudaStreamSynchronize(stream_) == cudaSuccess;
   for (auto& ev : ev_) clean = clean && ev != nullptr;
   lap("free (synchronize)");
+  if (join_ev_) cudaEventDestroy(join_ev_);
   if (clean) {
     // stream, events and scratch wait for the next handle on this device (HostKit)
     HostKit kit;
@@ -725,26 +737,33 @@ Engine::~Engine() {
   lap("stream, events, scratch");
 }
 
+// phase times of povar_create on stderr (POVAR_TRACE_CREATE)
+namespace {
+struct CreateLap {
+  bool on = getenv("POVAR_TRACE_CREATE") != nullptr;
+  std::chrono::steady_clock::time_point prev = std::chrono::steady_clock::now();
+  void operator()(const char* what) {
+    if (!on) return;
+    const auto now = std::chrono::steady_clock::now();
+    std::fprintf(stderr, "povar_create: %-28s %8.3f ms\n", what, std::chrono::duration<double, std::milli>(now - prev).count());
+    prev = now;
+  }
+};
+}  // namespace
+
+// Front half of the host route: the landmark table (one pass over lm_ptr) and the uploads of lm_ptr and the camera
+// indices; everything per observation -- the check of the camera indices and the per-camera counts included -- is
+// made on the device (kernels_index.cu)
 int Engine::upload(const povar_problem_desc* desc) {
   const int C = desc->num_cams, L = desc->num_lms;
   const int nnz = static_cast<int>(desc->num_obs);
   C_ = C;
   L_ = L;
   nnz_ = nnz;
-  // ---- host: the landmark table (one pass over lm_ptr) and the small tables; everything per observation --
-  // the check of the camera indices and the per-camera counts included -- is made on the device
-  // (kernels_index.cu)
-  static const bool trace = getenv("POVAR_TRACE_CREATE") != nullptr;   // phase times of povar_create on stderr
-  auto t_prev = std::chrono::steady_clock::now();
-  auto lap = [&](const char* what) {
-    if (!trace) return;
-    const auto now = std::chrono::steady_clock::now();
-    std::fprintf(stderr, "povar_create: %-28s %8.3f ms\n", what, std::chrono::duration<double, std::milli>(now - t_prev).count());
-    t_prev = now;
-  };
-  std::vector<int> lm_ptr(L + 1), cam_ptr(C + 1, 0);
-  SellLayout sell;    // sliced-ELL order: the long landmarks from the pass below, the slices from the device
-  int sell_n = 0;     // landmarks with 1..sell_max_deg observations
+  CreateLap lap;
+  std::vector<int> lm_ptr(L + 1);
+  std::vector<int> long_lms;   // landmarks with more than sell_max_deg observations
+  int sell_n = 0;              // landmarks with 1..sell_max_deg observations
   const int sell_max_deg = sell_max_degree(nnz, sm_count());
   d_.ix.sell_max_deg = sell_max_deg;
   if (desc->lm_ptr[0] != 0 || desc->lm_ptr[L] != nnz) return fail(POVAR_ERR_INVALID, "lm_ptr does not span the observations");
@@ -754,21 +773,138 @@ int Engine::upload(const povar_problem_desc* desc) {
     const int64_t b = desc->lm_ptr[l], e = desc->lm_ptr[l + 1];
     if (e < b || b < 0 || e > nnz) return fail(POVAR_ERR_INVALID, "lm_ptr is not monotone");
     lm_ptr[l] = static_cast<int>(b);
-    if (e - b > sell_max_deg) sell.long_lms.push_back(l);
+    if (e - b > sell_max_deg) long_lms.push_back(l);
     else if (e > b) ++sell_n;
   }
   lm_ptr[L] = nnz;
   lap("landmark table");
   // the observation list starts travelling now: camera indices first (the device checks and counts them while
-  // the image coordinates follow), and the copies run while the host derives the work items below
-#define PV_UP(dst, src, n) PV_CUDA(cudaMemcpyAsync((dst), (src), (n), cudaMemcpyHostToDevice, stream_))
+  // the image coordinates follow, build_index), and the copies run while the host derives the work items
   DeviceIndex& ix = d_.ix;
   PV_ALLOC(ix.lm_ptr, L + 1);
   PV_ALLOC(ix.obs_cam, nnz);
   PV_ALLOC(ix.obs_lm, nnz);
   PV_ALLOC(ix.obs_uv, nnz);
-  PV_UP(ix.lm_ptr, lm_ptr.data(), sizeof(int) * (L + 1));
-  if (nnz > 0) PV_UP(ix.obs_cam, desc->obs_cam, sizeof(int) * static_cast<size_t>(nnz));
+  PV_CUDA(cudaMemcpyAsync(ix.lm_ptr, lm_ptr.data(), sizeof(int) * (L + 1), cudaMemcpyHostToDevice, stream_));
+  if (nnz > 0) {
+    PV_CUDA(cudaMemcpyAsync(ix.obs_cam, desc->obs_cam, sizeof(int) * static_cast<size_t>(nnz), cudaMemcpyHostToDevice,
+                            stream_));
+  }
+  ix.num_long = static_cast<int>(long_lms.size());
+  return build_index(sell_n, long_lms.data(), desc->obs_uv, desc->cam_P);
+}
+
+int Engine::check_device_ptr(const void* p, const char* what) {
+  cudaPointerAttributes a{};
+  const cudaError_t e = cudaPointerGetAttributes(&a, p);
+  cudaGetLastError();   // not sticky: a failed query must not fail the next call
+  if (e != cudaSuccess || (a.type != cudaMemoryTypeDevice && a.type != cudaMemoryTypeManaged) || a.device != device_) {
+    return fail(POVAR_ERR_INVALID, std::string(what) + " is not device memory of device " + std::to_string(device_));
+  }
+  return POVAR_OK;
+}
+
+int Engine::wait_for(cudaStream_t waiter, cudaStream_t producer) {
+  if (!join_ev_) PV_CUDA(cudaEventCreateWithFlags(&join_ev_, cudaEventDisableTiming));
+  const cudaError_t e = cudaEventRecord(join_ev_, producer);
+  if (e != cudaSuccess) {
+    cudaGetLastError();
+    return fail(POVAR_ERR_INVALID, std::string("stream of the caller: ") + cudaGetErrorString(e));
+  }
+  PV_CUDA(cudaStreamWaitEvent(waiter, join_ev_, 0));
+  return POVAR_OK;
+}
+
+// Front half of the device route: the canonical order of the caller's list on the device (kernels_index.cu), the
+// shard's entries gathered straight into the landmark-major arrays, the landmark table made there too; the host
+// reads the shard's observation count as soon as the keys are counted (the sort runs meanwhile) and the landmark
+// table once it is made.
+int Engine::upload_device(const povar_device_problem_desc* desc) {
+  const int C = desc->num_cams, L = desc->lm_end - desc->lm_begin;
+  const int n = static_cast<int>(desc->num_obs);
+  PV_CUDA(cudaSetDevice(device_));
+  for (const auto& pw : {std::make_pair(static_cast<const void*>(desc->cam_P), "cam_P"),
+                         std::make_pair(static_cast<const void*>(desc->obs_cam), "obs_cam"),
+                         std::make_pair(static_cast<const void*>(desc->obs_lm), "obs_lm"),
+                         std::make_pair(static_cast<const void*>(desc->obs_uv), "obs_uv")}) {
+    if (n == 0 && pw.first != desc->cam_P) continue;
+    const int rc = check_device_ptr(pw.first, pw.second);
+    if (rc != POVAR_OK) return rc;
+  }
+  {
+    const int rc = wait_for(stream_, static_cast<cudaStream_t>(desc->stream));
+    if (rc != POVAR_OK) return rc;
+  }
+  CreateLap lap;
+  C_ = C;
+  L_ = L;
+  // scratch, returned to the pool when this function returns
+  const size_t keep = allocs_.size();
+  struct Scratch {
+    Engine* e;
+    std::vector<void*> mine;
+    ~Scratch() {
+      for (void* p : mine) {
+        cudaFreeAsync(p, e->stream_);
+        e->allocs_.erase(std::find(e->allocs_.begin(), e->allocs_.end(), p));
+      }
+    }
+  } scratch{this, {}};
+  unsigned long long *keys_a = nullptr, *keys_b = nullptr;
+  int *pos_a = nullptr, *pos_b = nullptr, *info = nullptr, *long_tmp = nullptr;
+  unsigned char* is_long = nullptr;
+  char* temp = nullptr;
+  const int end_bit = order_end_bit(C, desc->num_lms);
+  const size_t temp_bytes = device_order_temp_bytes(n, L, end_bit);
+  PV_ALLOC(keys_a, n);
+  PV_ALLOC(keys_b, n);
+  PV_ALLOC(pos_a, n);
+  PV_ALLOC(pos_b, n);
+  PV_ALLOC(info, kOrderInfo);
+  PV_ALLOC(long_tmp, L);
+  PV_ALLOC(is_long, L);
+  PV_ALLOC(temp, temp_bytes);
+  scratch.mine.assign(allocs_.begin() + keep, allocs_.end());
+  int* counts = reinterpret_cast<int*>(host_out_);   // pinned: the read-backs below overlap the device work
+  PV_CUDA(device_order_keys(n, C, desc->num_lms, desc->lm_begin, desc->lm_end, desc->obs_cam, desc->obs_lm, keys_a,
+                            pos_a, info, lc()));
+  PV_CUDA(cudaMemcpyAsync(counts, info, sizeof(int) * kOrderInfo, cudaMemcpyDeviceToHost, stream_));
+  PV_CUDA(cudaEventRecord(join_ev_, stream_));
+  PV_CUDA(device_order_sort(n, end_bit, keys_a, keys_b, pos_a, pos_b, temp, temp_bytes, lc()));
+  PV_CUDA(cudaEventSynchronize(join_ev_));
+  if (counts[kOrderFlags] & 1) return fail(POVAR_ERR_INVALID, "povar_create_device: camera or landmark index out of range");
+  const int nnz = counts[kOrderCount];
+  nnz_ = nnz;
+  lap("order keys + counts (device)");
+  DeviceIndex& ix = d_.ix;
+  PV_ALLOC(ix.lm_ptr, L + 1);
+  PV_ALLOC(ix.obs_cam, nnz);
+  PV_ALLOC(ix.obs_lm, nnz);
+  PV_ALLOC(ix.obs_uv, nnz);
+  ix.L = L;
+  PV_CUDA(device_order_place(n, C, desc->lm_begin, sm_count(), keys_b, pos_b, desc->obs_uv, info, ix, is_long, long_tmp,
+                             temp, temp_bytes, lc()));
+  PV_CUDA(cudaMemcpyAsync(counts, info, sizeof(int) * kOrderInfo, cudaMemcpyDeviceToHost, stream_));
+  PV_CUDA(cudaStreamSynchronize(stream_));
+  if (counts[kOrderFlags] & 2) return fail(POVAR_ERR_INVALID, "povar_create_device: duplicate (camera, landmark) pair");
+  ix.num_long = counts[kOrderLong];
+  d_.ix.sell_max_deg = sell_max_degree(nnz, sm_count());
+  lap("canonical order + landmark table (device)");
+  return build_index(counts[kOrderSell], long_tmp, nullptr, desc->cam_P);
+}
+
+// Back half, shared by both routes: from the landmark-major list in ix (lm_ptr, obs_cam; obs_uv unless host_uv
+// still has to be uploaded) and the landmark table (sell_n, ix.num_long long landmarks at long_lms) to the whole
+// index and the state.  long_lms and cam_P may be host or device memory.
+int Engine::build_index(int sell_n, const int* long_lms, const double* host_uv, const double* cam_P) {
+  const int C = C_, L = L_;
+  const int nnz = static_cast<int>(nnz_);
+  const int sell_max_deg = d_.ix.sell_max_deg;
+  CreateLap lap;
+  std::vector<int> cam_ptr(C + 1, 0);
+  SellLayout sell;    // sliced-ELL order: the slices from the device
+#define PV_UP(dst, src, n) PV_CUDA(cudaMemcpyAsync((dst), (src), (n), cudaMemcpyHostToDevice, stream_))
+  DeviceIndex& ix = d_.ix;
   {
     int* d_count = nullptr;
     const size_t keep = allocs_.size();
@@ -779,8 +915,8 @@ int Engine::upload(const povar_problem_desc* desc) {
     cudaEvent_t counted = nullptr;
     PV_CUDA(cudaEventCreateWithFlags(&counted, cudaEventDisableTiming));
     cudaEventRecord(counted, stream_);
-    if (nnz > 0) {
-      const cudaError_t ce = cudaMemcpyAsync(ix.obs_uv, desc->obs_uv, sizeof(double) * 2 * static_cast<size_t>(nnz),
+    if (host_uv && nnz > 0) {
+      const cudaError_t ce = cudaMemcpyAsync(ix.obs_uv, host_uv, sizeof(double) * 2 * static_cast<size_t>(nnz),
                                              cudaMemcpyHostToDevice, stream_);
       if (ce != cudaSuccess) {
         cudaEventDestroy(counted);
@@ -850,7 +986,6 @@ int Engine::upload(const povar_problem_desc* desc) {
   ix.num_items = static_cast<int>(item_cam.size());
   ix.num_slices = static_cast<int>(sell.slice_ptr.size()) - 1;
   ix.sell_slots = static_cast<long long>(kSellWidth) * sell.rows;
-  ix.num_long = static_cast<int>(sell.long_lms.size());
   const size_t slots = static_cast<size_t>(ix.sell_slots);
   PV_ALLOC(ix.cam_ptr, C + 1);
   PV_ALLOC(ix.csc_lm, nnz);
@@ -865,7 +1000,7 @@ int Engine::upload(const povar_problem_desc* desc) {
   PV_ALLOC(ix.sell_uv_e0, slots);
   PV_ALLOC(ix.sell_row_e0, slots + 32);
   PV_ALLOC(ix.obs_slot, nnz);
-  PV_ALLOC(ix.long_lm, sell.long_lms.size());
+  PV_ALLOC(ix.long_lm, ix.num_long);
   if (nnz > 0) PV_UP(ix.item_cam, item_cam.data(), sizeof(int) * item_cam.size());
   PV_UP(ix.slice_ptr, sell.slice_ptr.data(), sizeof(int) * sell.slice_ptr.size());
   // landmark half: ranges of slices per warp, windows of cameras per block (kernels_series.cu), per model
@@ -884,7 +1019,10 @@ int Engine::upload(const povar_problem_desc* desc) {
     PV_UP(d_.plan[m].range_slice, h.range_slice.data(), sizeof(int) * h.range_slice.size());
     PV_UP(d_.plan[m].blk_lo, h.blk_lo.data(), sizeof(int) * h.blk_lo.size());
   }
-  if (ix.num_long > 0) PV_UP(ix.long_lm, sell.long_lms.data(), sizeof(int) * sell.long_lms.size());
+  if (ix.num_long > 0) {
+    PV_CUDA(cudaMemcpyAsync(ix.long_lm, long_lms, sizeof(int) * static_cast<size_t>(ix.num_long), cudaMemcpyDefault,
+                            stream_));
+  }
   PV_UP(ix.cam_ptr, cam_ptr.data(), sizeof(int) * (C + 1));
   PV_UP(ix.item_ptr, item_ptr.data(), sizeof(int) * item_ptr.size());
   PV_UP(ix.cam_item_ptr, cam_item_ptr.data(), sizeof(int) * (C + 1));
@@ -958,7 +1096,7 @@ int Engine::upload(const povar_problem_desc* desc) {
   PV_ALLOC(d_.flags, 4);
   PV_ALLOC(d_.ctl, 1);
   PV_ALLOC(d_.cg, 1);
-  PV_UP(d_.P, desc->cam_P, sizeof(double) * C12);
+  PV_CUDA(cudaMemcpyAsync(d_.P, cam_P, sizeof(double) * C12, cudaMemcpyDefault, stream_));
 #undef PV_UP
   lap("allocate + enqueue uploads");
   // the host tables above live on this stack frame
@@ -1921,6 +2059,50 @@ int Engine::set_state(int which, const double* cam_P, const double* lms) {
     PV_CUDA(cudaMemcpy(d_.X, h.data(), sizeof(double) * h.size(), cudaMemcpyHostToDevice));
   }
   return POVAR_OK;
+}
+
+// get_state / set_state in device memory, ordered between the caller's stream and the handle's: the copies wait for
+// the caller's work so far, the caller's stream waits for the copies
+int Engine::get_state_device(int which, double* cam_P, double* lms, cudaStream_t caller) {
+  PV_CUDA(cudaSetDevice(device_));
+  if (cam_P && check_device_ptr(cam_P, "cam_P") != POVAR_OK) return POVAR_ERR_INVALID;
+  if (lms && L_ > 0 && check_device_ptr(lms, "lms") != POVAR_OK) return POVAR_ERR_INVALID;
+  int rc = wait_for(stream_, caller);
+  if (rc != POVAR_OK) return rc;
+  if (cam_P) {
+    PV_CUDA(cudaMemcpyAsync(cam_P, d_.P, sizeof(double) * static_cast<size_t>(C_) * 12, cudaMemcpyDeviceToDevice, stream_));
+  }
+  if (lms && L_ > 0) {
+    if (which == POVAR_STATE_JOINT) {
+      PV_CUDA(cudaMemcpyAsync(lms, d_.X, sizeof(double) * 4 * static_cast<size_t>(L_), cudaMemcpyDeviceToDevice, stream_));
+    } else {
+      PV_CUDA(cudaMemcpy2DAsync(lms, 3 * sizeof(double), d_.X, 4 * sizeof(double), 3 * sizeof(double),
+                                static_cast<size_t>(L_), cudaMemcpyDeviceToDevice, stream_));
+    }
+  }
+  return wait_for(caller, stream_);
+}
+
+int Engine::set_state_device(int which, const double* cam_P, const double* lms, cudaStream_t caller) {
+  PV_CUDA(cudaSetDevice(device_));
+  if (cam_P && check_device_ptr(cam_P, "cam_P") != POVAR_OK) return POVAR_ERR_INVALID;
+  if (lms && L_ > 0 && check_device_ptr(lms, "lms") != POVAR_OK) return POVAR_ERR_INVALID;
+  int rc = wait_for(stream_, caller);
+  if (rc != POVAR_OK) return rc;
+  if (cam_P) {
+    PV_CUDA(cudaMemcpyAsync(d_.P, cam_P, sizeof(double) * static_cast<size_t>(C_) * 12, cudaMemcpyDeviceToDevice, stream_));
+  }
+  if (lms && L_ > 0) {
+    if (which == POVAR_STATE_JOINT) {
+      PV_CUDA(cudaMemcpyAsync(d_.X, lms, sizeof(double) * 4 * static_cast<size_t>(L_), cudaMemcpyDeviceToDevice, stream_));
+    } else {
+      PV_CUDA(cudaMemcpy2DAsync(d_.X, 4 * sizeof(double), lms, 3 * sizeof(double), 3 * sizeof(double),
+                                static_cast<size_t>(L_), cudaMemcpyDeviceToDevice, stream_));
+      launch_to_homogeneous(d_, lc());   // w = 1, as set_state writes it
+      PV_CUDA(cudaGetLastError());
+    }
+  }
+  return wait_for(caller, stream_);
 }
 
 int64_t Engine::debug_read(const char* name, double* out, int64_t capacity) {

@@ -1,6 +1,7 @@
 // Engine: owns the device state of one shard and sequences the kernels of the hot path.
 #pragma once
 
+#include <functional>
 #include <string>
 #include <vector>
 
@@ -20,6 +21,8 @@ class Engine {
  public:
   static int create(const povar_problem_desc* desc, const povar_options* opt,
                     const povar_comm_desc* comm, Engine** out, std::string* err);
+  static int create_device(const povar_device_problem_desc* desc, const povar_options* opt,
+                           const povar_comm_desc* comm, Engine** out, std::string* err);
   ~Engine();
 
   int init_varproj(double alpha);
@@ -38,6 +41,8 @@ class Engine {
   int normalize_joint();
   int get_state(int which, double* cam_P, double* lms);
   int set_state(int which, const double* cam_P, const double* lms);
+  int get_state_device(int which, double* cam_P, double* lms, cudaStream_t caller);
+  int set_state_device(int which, const double* cam_P, const double* lms, cudaStream_t caller);
   int64_t debug_read(const char* name, double* out, int64_t capacity);
   int right_mul_e0(bool joint, const double* x, double* out);
   int bench_power_terms(bool joint, int terms, double* seconds_per_term);
@@ -59,7 +64,16 @@ class Engine {
   Engine() = default;
   int fail(int code, const std::string& what);
   int check(cudaError_t e, const char* what);
+  // device, stream, communicator; then `upload` fills the index and the state
+  static int create_with(const povar_options* opt, const povar_comm_desc* comm, Engine** out, std::string* err,
+                         const std::function<int(Engine*)>& upload);
+  // the two front halves of the index build (host list in canonical order / device list in any order) and the
+  // shared back half (build_index)
   int upload(const povar_problem_desc* desc);
+  int upload_device(const povar_device_problem_desc* desc);
+  int build_index(int sell_n, const int* long_lms, const double* host_uv, const double* cam_P);
+  int check_device_ptr(const void* p, const char* what);
+  int wait_for(cudaStream_t waiter, cudaStream_t producer);   // waiter waits for the work enqueued on producer
   int allreduce(double* buf, size_t n, bool skip_when_done = false);
   int setup_peer_exchange();
   TermMode term_mode() const { return peer_ok_ ? kTermPeer : (world_ == 1 ? kTermFused : kTermRaw); }
@@ -88,6 +102,7 @@ class Engine {
   std::vector<void*> allocs_;
   cudaStream_t stream_ = nullptr;
   cudaEvent_t ev_[8] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};   // [6], [7]: linearize
+  cudaEvent_t join_ev_ = nullptr;   // wait_for: ordering against a caller's stream
   long long launches_ = 0;
   std::string err_;
   PhaseTimes times_;
@@ -142,7 +157,6 @@ struct SellLayout {
 void set_host_threads_override(int n);   // 0 = automatic
 void build_sell(const std::vector<int>& lm_ptr, const int* obs_cam, int num_cams, int max_window,
                 SellLayout* out, int max_deg = 32);
-int sell_max_degree(long long nnz, int sms);
 int sell_window(int landmarks, int max_window);
 int sell_key(const int* cams, int deg, int span);
 

@@ -12,6 +12,8 @@
 #include <algorithm>
 
 #include <cub/device/device_radix_sort.cuh>
+#include <cub/device/device_select.cuh>
+#include <cub/iterator/counting_input_iterator.cuh>
 
 #include "povar_internal.h"
 
@@ -378,6 +380,147 @@ cudaError_t build_device_sell(int L, int num_cams, int n, int window, int max_de
   k_sell_slices<<<(num_slices * 32 + kBlock - 1) / kBlock, kBlock, 0, st>>>(num_slices, n, ids_a, lm_ptr, obs_cam,
                                                                           sell_lm, slice_len, slice_lo, slice_hi);
   if (lc.launch_counter) *lc.launch_counter += 5;
+  return cudaGetLastError();
+}
+
+// ---- canonical order of an unordered observation list (povar_create_device) -----------------------------------
+// The order of povar_canonical_order (host/bal_io.cpp): landmark, then camera ascending.  Every observation of the
+// list gets the 64-bit key (landmark << cam_bits) | camera, one radix sort by key brings them into that order, and
+// the shard [lm_begin, lm_end) is then one contiguous run of the sorted list.  The keys are those of the whole
+// problem, not of the shard, so that every rank sees a duplicate pair or an index out of range anywhere in the list
+// and fails its povar_create_device, as povar_canonical_order fails for every rank of the host route.
+namespace {
+
+// key of every entry (all ones for an entry with an index out of range: it sorts last), its position, and the
+// counts: info[kOrderBefore] valid entries of landmarks below lm_begin, info[kOrderCount] of the shard,
+// info[kOrderFlags] |= 1 for an index out of range.  Integer sums: the counts do not depend on the order of the
+// atomics.
+__global__ void __launch_bounds__(kBlock)
+k_obs_keys(int n, int C, int num_lms, int lm_begin, int lm_end, int cam_bits, const int* __restrict__ obs_cam,
+           const int* __restrict__ obs_lm, unsigned long long* __restrict__ keys, int* __restrict__ pos,
+           int* __restrict__ info) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  bool before = false, in = false, bad = false;
+  if (i < n) {
+    const int c = obs_cam[i], l = obs_lm[i];
+    bad = static_cast<unsigned>(c) >= static_cast<unsigned>(C) || static_cast<unsigned>(l) >= static_cast<unsigned>(num_lms);
+    keys[i] = bad ? ~0ULL : (static_cast<unsigned long long>(l) << cam_bits) | static_cast<unsigned>(c);
+    pos[i] = i;
+    before = !bad && l < lm_begin;
+    in = !bad && l >= lm_begin && l < lm_end;
+  }
+  const int nb = __syncthreads_count(before), ni = __syncthreads_count(in), nbad = __syncthreads_or(bad);
+  if (threadIdx.x == 0) {
+    if (nb) atomicAdd(&info[kOrderBefore], nb);
+    if (ni) atomicAdd(&info[kOrderCount], ni);
+    if (nbad) atomicOr(&info[kOrderFlags], 1);
+  }
+}
+
+// One thread per sorted entry: equal neighbours are a duplicate pair (info[kOrderFlags] |= 2); an entry of the shard
+// goes to its place in the landmark-major arrays, and the first entry of every landmark opens the ranges of the
+// landmarks up to its own (those in between have no observations: empty ranges, as povar_canonical_order makes
+// them); the last entry of the shard closes the ranges of the landmarks after it.
+__global__ void __launch_bounds__(kBlock)
+k_obs_place(int n, int cam_bits, int lm_begin, int L, const unsigned long long* __restrict__ keys,
+            const int* __restrict__ pos, const double* __restrict__ uv_in, int* __restrict__ info,
+            int* __restrict__ lm_ptr, int* __restrict__ obs_cam, int* __restrict__ obs_lm, double2* __restrict__ obs_uv) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const unsigned long long key = keys[i];
+  if (key == ~0ULL) return;   // an index out of range, already flagged
+  if (i > 0 && keys[i - 1] == key) atomicOr(&info[kOrderFlags], 2);
+  const int l = static_cast<int>(key >> cam_bits) - lm_begin;
+  if (l < 0 || l >= L) return;
+  const int lo = info[kOrderBefore], cnt = info[kOrderCount];
+  const int p = i - lo;
+  const int src = pos[i];
+  obs_cam[p] = static_cast<int>(key & ((1ULL << cam_bits) - 1));
+  obs_lm[p] = l;
+  obs_uv[p] = make_double2(uv_in[2 * static_cast<size_t>(src)], uv_in[2 * static_cast<size_t>(src) + 1]);
+  const int prev = p == 0 ? -1 : static_cast<int>(keys[i - 1] >> cam_bits) - lm_begin;
+  for (int m = prev + 1; m <= l; ++m) lm_ptr[m] = p;
+  if (p == cnt - 1) {
+    for (int m = l + 1; m <= L; ++m) lm_ptr[m] = cnt;
+  }
+}
+
+// The landmark table of Engine::upload on the device: info[kOrderSell] landmarks with 1..max_deg observations, and
+// is_long[l] for the stable compaction of the long ones (max_deg = sell_max_degree of the shard's observation count).
+__global__ void __launch_bounds__(kBlock)
+k_lm_table(int L, int sms, const int* __restrict__ lm_ptr, int* __restrict__ info, unsigned char* __restrict__ is_long) {
+  const int l = blockIdx.x * blockDim.x + threadIdx.x;
+  const int max_deg = sell_max_degree(info[kOrderCount], sms);
+  bool sell = false;
+  if (l < L) {
+    const int deg = lm_ptr[l + 1] - lm_ptr[l];
+    is_long[l] = deg > max_deg ? 1 : 0;
+    sell = deg > 0 && deg <= max_deg;
+  }
+  const int ns = __syncthreads_count(sell);
+  if (threadIdx.x == 0 && ns) atomicAdd(&info[kOrderSell], ns);
+}
+
+int value_bits(long long n) {   // bits that hold every value below n
+  int b = 1;
+  while ((1LL << b) < n) ++b;
+  return b;
+}
+
+}  // namespace
+
+int order_cam_bits(int num_cams) { return value_bits(num_cams); }
+
+// the key of an entry of landmark num_lms - 1 stays below the all-ones key of the rejected entries
+int order_end_bit(int num_cams, int num_lms) { return order_cam_bits(num_cams) + value_bits(num_lms + 1LL); }
+
+size_t device_order_temp_bytes(int n, int L, int end_bit) {
+  size_t a = 0, b = 0;
+  cub::DeviceRadixSort::SortPairs(nullptr, a, static_cast<const unsigned long long*>(nullptr),
+                                  static_cast<unsigned long long*>(nullptr), static_cast<const int*>(nullptr),
+                                  static_cast<int*>(nullptr), n > 0 ? n : 1, 0, end_bit);
+  cub::DeviceSelect::Flagged(nullptr, b, cub::CountingInputIterator<int>(0), static_cast<const unsigned char*>(nullptr),
+                             static_cast<int*>(nullptr), static_cast<int*>(nullptr), L > 0 ? L : 1);
+  return a > b ? a : b;
+}
+
+cudaError_t device_order_keys(int n, int C, int num_lms, int lm_begin, int lm_end, const int* obs_cam, const int* obs_lm,
+                              unsigned long long* keys, int* pos, int* info, const LaunchCfg& lc) {
+  if (n <= 0) return cudaSuccess;
+  k_obs_keys<<<(n + kBlock - 1) / kBlock, kBlock, 0, lc.stream>>>(n, C, num_lms, lm_begin, lm_end, order_cam_bits(C),
+                                                                  obs_cam, obs_lm, keys, pos, info);
+  if (lc.launch_counter) *lc.launch_counter += 1;
+  return cudaGetLastError();
+}
+
+cudaError_t device_order_sort(int n, int end_bit, const unsigned long long* keys_in, unsigned long long* keys_out,
+                              const int* pos_in, int* pos_out, void* temp, size_t temp_bytes, const LaunchCfg& lc) {
+  if (n <= 0) return cudaSuccess;
+  const cudaError_t e = cub::DeviceRadixSort::SortPairs(temp, temp_bytes, keys_in, keys_out, pos_in, pos_out, n, 0,
+                                                        end_bit, lc.stream);
+  if (lc.launch_counter) *lc.launch_counter += 1;   // counted once, like the other radix sorts
+  return e;
+}
+
+cudaError_t device_order_place(int n, int C, int lm_begin, int sms, const unsigned long long* keys, const int* pos,
+                               const double* obs_uv_in, int* info, const DeviceIndex& ix, unsigned char* is_long,
+                               int* long_lms, void* temp, size_t temp_bytes, const LaunchCfg& lc) {
+  cudaStream_t st = lc.stream;
+  const int L = ix.L;
+  int launches = 0;
+  if (n > 0) {
+    k_obs_place<<<(n + kBlock - 1) / kBlock, kBlock, 0, st>>>(n, order_cam_bits(C), lm_begin, L, keys, pos, obs_uv_in,
+                                                              info, ix.lm_ptr, ix.obs_cam, ix.obs_lm, ix.obs_uv);
+    ++launches;
+  }
+  if (L > 0) {
+    k_lm_table<<<(L + kBlock - 1) / kBlock, kBlock, 0, st>>>(L, sms, ix.lm_ptr, info, is_long);
+    const cudaError_t e = cub::DeviceSelect::Flagged(temp, temp_bytes, cub::CountingInputIterator<int>(0), is_long,
+                                                     long_lms, info + kOrderLong, L, st);
+    if (e != cudaSuccess) return e;
+    launches += 2;
+  }
+  if (lc.launch_counter) *lc.launch_counter += launches;
   return cudaGetLastError();
 }
 

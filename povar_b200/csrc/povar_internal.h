@@ -239,6 +239,22 @@ struct LaunchCfg {
   long long* launch_counter = nullptr;
 };
 
+// Largest degree of a landmark of the sliced-ELL set.  A slice is walked row by row by ONE warp, so a slice of 32
+// rows is a chain of 32 dependent steps (0.76 us each when the SM is not full); on a large shard every warp has
+// dozens of rows anyway, on a small one (a venice-1778 shard on 8 GPUs: one slice of ~5 rows per warp) the few
+// slices of 30 rows set the time of the whole launch (27 us where the median block needs 19).  There the
+// landmarks with more than about twice the rows a warp has anyway go to the warp-per-landmark kernels instead
+// (32 observations per step): 31 -> 22 us per launch with 12, measured on that shard.  (Host and device: the
+// device canonical order makes the landmark table with it, kernels_index.cu.)
+__host__ __device__ inline int sell_max_degree(long long nnz, int sms) {
+  const long long rows_per_warp = nnz / (32LL * 32 * sms);   // rows of one resident wave of warps
+  if (rows_per_warp >= 16) return 32;
+  long long t = (2 * rows_per_warp + 3) / 4 * 4;
+  if (t < 8) t = 8;
+  if (t > 32) t = 32;
+  return static_cast<int>(t);
+}
+
 struct ModelParams {
   double c1, c2;        // sqrt(1-alpha), sqrt(alpha)
   int robust_norm;
@@ -257,6 +273,20 @@ cudaError_t validate_obs(int L, int C, int sms, const int* lm_ptr, const int* ob
 size_t index_sort_temp_bytes(int nnz, int num_cams);
 cudaError_t build_device_index(const DeviceIndex& ix, int* iota, int* keys_out, int* perm, int* lm_slot,
                                void* sort_temp, size_t sort_temp_bytes, const LaunchCfg& lc);
+// canonical order of an unordered device list (povar_create_device): keys + counts, radix sort, then the shard's
+// entries gathered into ix.lm_ptr / obs_cam / obs_lm / obs_uv and the landmark table.  info: kOrderInfo zeroed ints.
+enum { kOrderBefore = 0, kOrderCount = 1, kOrderFlags = 2, kOrderSell = 3, kOrderLong = 4, kOrderInfo = 5 };
+int order_cam_bits(int num_cams);
+int order_end_bit(int num_cams, int num_lms);
+size_t device_order_temp_bytes(int n, int L, int end_bit);
+cudaError_t device_order_keys(int n, int C, int num_lms, int lm_begin, int lm_end, const int* obs_cam, const int* obs_lm,
+                              unsigned long long* keys, int* pos, int* info, const LaunchCfg& lc);
+cudaError_t device_order_sort(int n, int end_bit, const unsigned long long* keys_in, unsigned long long* keys_out,
+                              const int* pos_in, int* pos_out, void* temp, size_t temp_bytes, const LaunchCfg& lc);
+// is_long [ix.L], long_lms [ix.L] scratch: the first info[kOrderLong] of long_lms are the long landmarks, ascending
+cudaError_t device_order_place(int n, int C, int lm_begin, int sms, const unsigned long long* keys, const int* pos,
+                               const double* obs_uv_in, int* info, const DeviceIndex& ix, unsigned char* is_long,
+                               int* long_lms, void* temp, size_t temp_bytes, const LaunchCfg& lc);
 
 // ---- landmark-major kernels (kernels_landmark.cu) ----
 void launch_init_varproj(const DeviceState& d, const ModelParams& mp, const LaunchCfg& lc);
