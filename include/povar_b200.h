@@ -308,6 +308,23 @@ typedef struct povar_solve_summary {
 int povar_bundle_adjust(povar_handle* h, const povar_options* opt, povar_iteration* iterations,
                         int32_t max_iterations, povar_solve_summary* summary);
 
+/* povar_bundle_adjust, enqueued: the same two-step solve on the state held by the handle, ordered after the work
+ * enqueued on `stream` (cudaStream_t, NULL = legacy default stream) so far; `stream` waits for it.  No host
+ * synchronisation, nothing printed.  `iterations` (room for max_iterations entries; may be NULL when max_iterations
+ * is 0), `summary` and `status` are device memory of the handle's device, written when the solve ends: *status =
+ * what povar_bundle_adjust returns for the same handle, state and options.
+ * Both LM loops run on the device, with the host driver's decisions (the same code) and log columns; the times
+ * come from the GPU's global timer, and the function-tolerance message ends after "Function tolerance reached.".
+ * The radius update's cube is correctly rounded on the device, so a trust-region radius may differ from the host
+ * driver's in the last bit.  The first call with given options (and debug settings) builds and instantiates one
+ * CUDA graph for the solve; later calls with byte-identical options only launch it.  Not advanced by it:
+ * povar_get_timings, povar_launch_count.
+ * POVAR_ERR_INVALID: the checks of povar_bundle_adjust, max_iterations < 0, an output pointer that is not device
+ * memory of the handle's device.  POVAR_ERR_UNSUPPORTED: a sharded handle whose reductions go through ncclAllReduce
+ * (povar_peer_exchange_active(h) == 0 with more than one rank). */
+int povar_bundle_adjust_async(povar_handle* h, const povar_options* opt, povar_iteration* iterations,
+                              int32_t max_iterations, povar_solve_summary* summary, int32_t* status, void* stream);
+
 /* ba_log.json with the reference's complete key set (bal/ba_log.hpp:85-245, bal/ba_log_utils.cpp:100-175), so that
  * the reference's python/rootba tooling loads it unchanged; what `bal --log-log-path` writes.  lm_ptr may be NULL
  * (then per_lm_obs is zero).  Host only. */

@@ -30,6 +30,7 @@ LIB_SOURCES = [
     "kernels_chol.cu",
     "kernels_series.cu",
     "kernels_index.cu",
+    "kernels_lm.cu",
     "engine.cu",
     "capi.cpp",
     "host/bal_io.cpp",
@@ -37,7 +38,9 @@ LIB_SOURCES = [
     "host/lm_driver.cpp",
     "host/chol_symbolic.cpp",
 ]
-HEADERS = ["device_math.cuh", "sell_walk.cuh", "povar_internal.h", "engine.h", "../../include/povar_b200.h"]
+HEADERS = ["device_math.cuh", "sell_walk.cuh", "povar_internal.h", "engine.h", "lm_step.h", "../../include/povar_b200.h"]
+# the LM decision kernels compute what the host driver computes: no contracted multiply-adds (lm_step.h)
+EXTRA_FLAGS = {"kernels_lm.cu": ["-fmad=false"]}
 
 
 def _nvcc() -> str:
@@ -82,8 +85,9 @@ def build(force: bool = False, verbose: bool = False, defines=(), suffix: str = 
         obj = os.path.join(OBJ, src.replace("/", "_") + ".o")
         if not force and _newer(obj, [path] + headers):
             return obj
-        cmd = [nvcc] + ARCH + COMMON + ["-x", "cu", "-Xptxas", "-v" if verbose else "-warn-spills",
-                                        "-c", path, "-o", obj]
+        cmd = [nvcc] + ARCH + COMMON + EXTRA_FLAGS.get(src, []) + ["-x", "cu", "-Xptxas",
+                                                                   "-v" if verbose else "-warn-spills",
+                                                                   "-c", path, "-o", obj]
         _run(cmd, verbose)
         return obj
 
@@ -108,7 +112,8 @@ def _build_variant(nvcc, defines, suffix, verbose):
 
     def compile_one(src):
         obj = os.path.join(obj_dir, src.replace("/", "_") + ".o")
-        _run([nvcc] + ARCH + COMMON + ["-D" + d for d in defines] + ["-x", "cu", "-Xptxas", "-warn-spills", "-c",
+        _run([nvcc] + ARCH + COMMON + EXTRA_FLAGS.get(src, []) + ["-D" + d for d in defines] +
+             ["-x", "cu", "-Xptxas", "-warn-spills", "-c",
                                                                     os.path.join(CSRC, src), "-o", obj], verbose)
         return obj
 

@@ -163,6 +163,8 @@ SIGNATURES = {
     "povar_set_state_device": (C.c_int, [_H, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]),
     "povar_bundle_adjust": (C.c_int, [_H, C.POINTER(Options), C.POINTER(Iteration), C.c_int32,
                                       C.POINTER(SolveSummary)]),
+    "povar_bundle_adjust_async": (C.c_int, [_H, C.POINTER(Options), C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p,
+                                            C.c_void_p]),
     "povar_comm_finalize": (C.c_int, []),
     "povar_debug_read": (C.c_int64, [_H, C.c_char_p, _DP, C.c_int64]),
     "povar_right_mul_e0": (C.c_int, [_H, C.c_int32, _DP, _DP]),
@@ -535,6 +537,28 @@ class Solver:
             raise PovarError(rc, summary.message.decode() + " / " + self.lib.povar_last_error(self.h).decode())
         return [its[i] for i in range(summary.num_iterations)], summary
 
+    def bundle_adjust_async(self, options: Options | None = None) -> "AsyncSolve":
+        """bundle_adjust enqueued on the current torch stream of the handle's device, without a host
+        synchronisation; `.result()` of the returned object gives what bundle_adjust returns."""
+        import torch
+        opt = options if options is not None else self.options
+        if not isinstance(opt, Options):
+            raise ValueError("bundle_adjust_async: options must be a capi.Options")
+        if opt.max_num_iterations_step_1 < 0 or opt.max_num_iterations_step_2 < 0:
+            raise ValueError("bundle_adjust_async: negative maximum number of iterations")
+        if not getattr(self, "h", None):
+            raise ValueError("bundle_adjust_async: the solver is closed")
+        cap = opt.max_num_iterations_step_1 + opt.max_num_iterations_step_2 + 2
+        dev = torch.device("cuda", self.device_index)
+        log = torch.empty(cap * C.sizeof(Iteration), dtype=torch.uint8, device=dev)
+        summary = torch.empty(C.sizeof(SolveSummary), dtype=torch.uint8, device=dev)
+        status = torch.empty(1, dtype=torch.int32, device=dev)
+        with torch.cuda.device(dev):
+            stream = torch.cuda.current_stream()
+        self._check(self.lib.povar_bundle_adjust_async(self.h, C.byref(opt), log.data_ptr(), cap, summary.data_ptr(),
+                                                       status.data_ptr(), stream.cuda_stream))
+        return AsyncSolve(self, log, summary, status, stream)
+
     def debug_read(self, name: str) -> np.ndarray:
         n = self.lib.povar_debug_read(self.h, name.encode(), None, 0)
         if n < 0:
@@ -591,6 +615,26 @@ class Solver:
 
     def reset_timings(self) -> None:
         self._check(self.lib.povar_reset_timings(self.h))
+
+
+class AsyncSolve:
+    """An enqueued solve (Solver.bundle_adjust_async): the log, the summary and the status in device tensors, written
+    on `stream` when the solve ends."""
+
+    def __init__(self, solver, log, summary, status, stream):
+        self.solver, self.log, self.summary, self.status, self.stream = solver, log, summary, status, stream
+
+    def result(self):
+        """Synchronises the stream and decodes -> (list[Iteration], SolveSummary); PovarError on a failed solve."""
+        self.stream.synchronize()
+        summary = SolveSummary.from_buffer_copy(self.summary.cpu().numpy().tobytes())
+        raw = self.log.cpu().numpy().tobytes()
+        n = min(summary.num_iterations, len(raw) // C.sizeof(Iteration))
+        its = [Iteration.from_buffer_copy(raw, i * C.sizeof(Iteration)) for i in range(n)]
+        rc = int(self.status.cpu()[0])
+        if rc != OK:
+            raise PovarError(rc, summary.message.decode())
+        return its, summary
 
 
 def write_ba_log(path: str, hp: "HostProblem", options, iterations, summary, input_path: str = "", load_time=0.0,

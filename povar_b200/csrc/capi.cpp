@@ -213,6 +213,17 @@ int povar_set_state_device(povar_handle* h, int32_t which, const double* cam_P, 
   return e.set_state_device(which, cam_P, lms, static_cast<cudaStream_t>(stream));
 }
 
+int povar_bundle_adjust_async(povar_handle* h, const povar_options* opt, povar_iteration* iterations,
+                              int32_t max_iterations, povar_solve_summary* summary, int32_t* status, void* stream) {
+  PV_ENGINE(h);
+  // the checks of povar_bundle_adjust (check_options, bal_bundle_adjustment.cpp:228-250)
+  if (!opt || max_iterations < 0 || !(opt->min_trust_region_radius <= opt->initial_trust_region_radius) ||
+      !(opt->initial_trust_region_radius <= opt->max_trust_region_radius) || opt->jacobi_scaling_epsilon < 0) {
+    return POVAR_ERR_INVALID;
+  }
+  return e.bundle_adjust_async(*opt, iterations, max_iterations, summary, status, static_cast<cudaStream_t>(stream));
+}
+
 int64_t povar_debug_read(povar_handle* h, const char* name, double* out, int64_t capacity) {
   if (!h || !h->engine) return POVAR_ERR_INVALID;
   return h->engine->debug_read(name, out, capacity);

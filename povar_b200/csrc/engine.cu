@@ -20,6 +20,7 @@
 #include <cmath>
 #include <cstdio>
 #include <cstring>
+#include <limits>
 #include <map>
 #include <mutex>
 #include <numeric>
@@ -708,6 +709,8 @@ Engine::~Engine() {
     if (g) cudaGraphExecDestroy(static_cast<cudaGraphExec_t>(g));
     g = nullptr;
   }
+  if (solve_graph_) cudaGraphExecDestroy(static_cast<cudaGraphExec_t>(solve_graph_));
+  solve_graph_ = nullptr;
   lap("graphs");
   if (peer_owned_ && peer_) {
     peer_->release();
@@ -1341,7 +1344,7 @@ int Engine::linearize(bool joint, double alpha, bool defer_check) {
     PV_ALLOC(d_.csc_w, static_cast<size_t>(nnz_));
     PV_ALLOC(d_.sell_w, static_cast<size_t>(d_.ix.sell_slots));
   }
-  PV_CUDA(cudaEventRecord(ev_[6], stream_));
+  PV_CUDA(mark(6));
   PV_CUDA(cudaMemsetAsync(d_.flags, 0, 4 * sizeof(int), stream_));
   // landmark side: Jl^T Jl, Jl^T r, column scales (LinearizorSC step 1 does not scale Jl:
   // solver/linearizor_sc.cpp:174-203)
@@ -1361,8 +1364,9 @@ int Engine::linearize(bool joint, double alpha, bool defer_check) {
     const int rc = allreduce(d_.trial_out + 9, 1);
     if (rc != POVAR_OK) return rc;
   }
-  PV_CUDA(cudaEventRecord(ev_[7], stream_));
+  PV_CUDA(mark(7));
   PV_CUDA(cudaGetLastError());
+  if (capturing_) return POVAR_OK;   // the decision kernel of the trial reads the flag
   if (defer_check) {
     // the caller goes on to a trial(): the flag comes back with that trial's results (one synchronisation)
     lin_check_pending_ = true;
@@ -1391,23 +1395,23 @@ int Engine::e0_product(bool joint, bool skip_when_done, bool fused_reduce) {
 int Engine::solve_power(bool joint, double lambda) {
   const bool poba = !joint && opt_.solver_type_step_1 == POVAR_POWER_SCHUR_COMPLEMENT;
   const double lambda_lm = joint ? lambda : (poba ? lambda : 0.0);
-  PV_CUDA(cudaEventRecord(ev_[0], stream_));
+  PV_CUDA(mark(0));
   // prepare_Hb_*: Hll^-1 and Hll^-1 Jl^T r per landmark; B^-1 per camera; b
-  launch_prep_landmark(d_, joint, lambda_lm, false, lc());
-  launch_cam_binv(d_, joint, lambda, lc());
+  launch_prep_landmark(d_, joint, lambda_lm, false, lc(), (joint || poba) ? lambda_dev_ : nullptr);
+  launch_cam_binv(d_, joint, lambda, lc(), lambda_dev_);
   launch_passB(d_, mp_, joint, lc());
   launch_reduce_items(d_, d_.item_part, 12, d_.cam_raw, false, lc());
   {
     const int rc = allreduce(d_.cam_raw, static_cast<size_t>(C_) * 12);
     if (rc != POVAR_OK) return rc;
   }
-  PV_CUDA(cudaEventRecord(ev_[1], stream_));
+  PV_CUDA(mark(1));
   // solve_*: accum = B^-1(-b); tmp = B^-1 E0 tmp; accum += tmp; early exit on zeta < eta
   {
     const int rc = enqueue_series(joint);
     if (rc != POVAR_OK) return rc;
   }
-  PV_CUDA(cudaEventRecord(ev_[2], stream_));
+  PV_CUDA(mark(2));
   PV_CUDA(cudaGetLastError());
   return POVAR_OK;
 }
@@ -1421,6 +1425,7 @@ int Engine::solve_power(bool joint, double lambda) {
 // 430 skipped launches of 2-4 us per venice-1778 solve.)  The first solve of a model runs eagerly -- it sets
 // function attributes -- and so does a series whose exchange is ncclAllReduce (no peer memory).
 int Engine::enqueue_series(bool joint) {
+  if (capturing_) return capture_series(joint);
   const int m = opt_.power_sc_iterations;
   const int which = joint ? 1 : 0;
   const bool graphable = term_mode() != kTermRaw;
@@ -1434,6 +1439,14 @@ int Engine::enqueue_series(bool joint) {
     }
     series_terms_counted_ = true;   // the launches above are in launches_ (skipped ones included)
     return POVAR_OK;
+  }
+  // the graph holds the model parameters of its capture (alpha, robust norm): other ones need a new graph
+  const ModelParams& was = series_mp_[which];
+  if (series_graph_[which] && (was.c1 != mp_.c1 || was.c2 != mp_.c2 || was.robust_norm != mp_.robust_norm ||
+                               was.huber != mp_.huber || was.jacobi_eps != mp_.jacobi_eps)) {
+    PV_CUDA(cudaStreamSynchronize(stream_));   // its last launch may still run
+    cudaGraphExecDestroy(static_cast<cudaGraphExec_t>(series_graph_[which]));
+    series_graph_[which] = nullptr;
   }
   if (!series_graph_[which]) {
     const long long before = launches_;
@@ -1496,6 +1509,7 @@ int Engine::enqueue_series(bool joint) {
       return check(e, "cudaGraphInstantiate");
     }
     series_graph_[which] = exec;
+    series_mp_[which] = mp_;
     launches_ = before;   // nothing ran during the capture
   }
   PV_CUDA(cudaGraphLaunch(static_cast<cudaGraphExec_t>(series_graph_[which]), stream_));
@@ -1555,8 +1569,8 @@ int Engine::solve(bool joint, double lambda, double* inc, int32_t* iterations) {
 
 // b (and B, B^-1) exactly as the power solvers build them; shared by PCG / RIPCG / CHOLESKY
 int Engine::prepare_reduced_system(bool joint, double lambda, double lambda_lm) {
-  launch_prep_landmark(d_, joint, lambda_lm, true, lc());
-  launch_cam_binv(d_, joint, lambda, lc());
+  launch_prep_landmark(d_, joint, lambda_lm, true, lc(), joint ? lambda_dev_ : nullptr);
+  launch_cam_binv(d_, joint, lambda, lc(), lambda_dev_);
   launch_passB(d_, mp_, joint, lc());
   launch_reduce_items(d_, d_.item_part, 12, d_.cam_raw, false, lc());
   const int rc = allreduce(d_.cam_raw, static_cast<size_t>(C_) * 12);
@@ -1587,7 +1601,7 @@ int Engine::solve_pcg(bool joint, double lambda) {
   const int D = joint ? 11 : 12;
   const int n = C_ * D;
   const size_t bytes = sizeof(double) * static_cast<size_t>(n);
-  PV_CUDA(cudaEventRecord(ev_[0], stream_));
+  PV_CUDA(mark(0));
   // LinearizorSC step 1 has no landmark damping (landmark_block.hpp:360-374); step 2 has (:414-431)
   int rc = prepare_reduced_system(joint, lambda, joint ? lambda : 0.0);
   if (rc != POVAR_OK) return rc;
@@ -1596,7 +1610,7 @@ int Engine::solve_pcg(bool joint, double lambda) {
   rc = allreduce(d_.kron2, static_cast<size_t>(C_) * kKron);
   if (rc != POVAR_OK) return rc;
   launch_cam_precond(d_, joint, d_.kron2, lc());
-  PV_CUDA(cudaEventRecord(ev_[1], stream_));
+  PV_CUDA(mark(1));
 
   const double* b = d_.b;
   double *x = d_.cg_x, *r = d_.cg_r, *p = d_.cg_p, *z = d_.cg_z, *q = d_.cg_q, *tmp = d_.vec_tmp;
@@ -1606,37 +1620,62 @@ int Engine::solve_pcg(bool joint, double lambda) {
   PV_CUDA(cudaMemcpyAsync(r, b, bytes, cudaMemcpyDeviceToDevice, stream_));   // r = b - S*0
   launch_dot_partials(d_, n, b, b, lc());
   launch_cg_scalar(d_, CG_BEGIN, 0, opt_.eta, min_it, max_it, lc());          // |b| = 0: done at once
-  SeriesCtl* hctl = reinterpret_cast<SeriesCtl*>(host_out_);
-  constexpr int kBatch = 4;
-  for (int it = 1; it <= max_it;) {
-    for (int k = 0; k < kBatch && it <= max_it; ++k, ++it) {
-      launch_block_matvec(d_, D, d_.Mprec, r, z, lc());                       // z = M^-1 r
-      launch_dot_partials(d_, n, r, z, lc());
-      launch_cg_scalar(d_, CG_RHO, it, opt_.eta, min_it, max_it, lc());
-      launch_cg_update(d_, CG_UPDATE_P, n, it, z, p, lc());                   // p = z + beta p
-      rc = schur_product(joint, p, q, true);                                  // q = S p
-      if (rc != POVAR_OK) return rc;
-      launch_dot_partials(d_, n, p, q, lc());
-      launch_cg_scalar(d_, CG_PQ, it, opt_.eta, min_it, max_it, lc());
-      launch_cg_update(d_, CG_UPDATE_X, n, it, p, x, lc());                   // x += alpha p
-      if (it % 10 == 0) {                                                     // residual_reset_period
-        rc = schur_product(joint, x, tmp, true);
-        if (rc != POVAR_OK) return rc;
-        launch_axpby(d_, n, 1.0, b, -1.0, tmp, r, lc());                      // r = b - S x
-      } else {
-        launch_cg_update(d_, CG_UPDATE_R, n, it, q, r, lc());                 // r -= alpha q
-      }
-      launch_axpby(d_, n, 1.0, b, 1.0, r, tmp, lc());
-      launch_dot_partials(d_, n, x, tmp, lc());
-      launch_cg_scalar(d_, CG_ZETA, it, opt_.eta, min_it, max_it, lc());      // Q, zeta < eta, max iterations
+  // iteration it (+ *base on the device)
+  auto iteration = [&](int it, const int* base) -> int {
+    launch_block_matvec(d_, D, d_.Mprec, r, z, lc());                         // z = M^-1 r
+    launch_dot_partials(d_, n, r, z, lc());
+    launch_cg_scalar(d_, CG_RHO, it, opt_.eta, min_it, max_it, lc(), base);
+    launch_cg_update(d_, CG_UPDATE_P, n, it, z, p, lc(), base);               // p = z + beta p
+    int rc2 = schur_product(joint, p, q, true);                               // q = S p
+    if (rc2 != POVAR_OK) return rc2;
+    launch_dot_partials(d_, n, p, q, lc());
+    launch_cg_scalar(d_, CG_PQ, it, opt_.eta, min_it, max_it, lc(), base);
+    launch_cg_update(d_, CG_UPDATE_X, n, it, p, x, lc(), base);               // x += alpha p
+    if (it % 10 == 0) {                                                       // residual_reset_period
+      rc2 = schur_product(joint, x, tmp, true);
+      if (rc2 != POVAR_OK) return rc2;
+      launch_axpby(d_, n, 1.0, b, -1.0, tmp, r, lc());                        // r = b - S x
+    } else {
+      launch_cg_update(d_, CG_UPDATE_R, n, it, q, r, lc(), base);             // r -= alpha q
     }
-    PV_CUDA(cudaMemcpyAsync(hctl, d_.ctl, sizeof(SeriesCtl), cudaMemcpyDeviceToHost, stream_));
-    PV_CUDA(cudaStreamSynchronize(stream_));
-    if (hctl->done) break;
+    launch_axpby(d_, n, 1.0, b, 1.0, r, tmp, lc());
+    launch_dot_partials(d_, n, x, tmp, lc());
+    launch_cg_scalar(d_, CG_ZETA, it, opt_.eta, min_it, max_it, lc(), base);  // Q, zeta < eta, max iterations
+    return POVAR_OK;
+  };
+  if (capturing_) {
+    // a WHILE node around ten iterations, numbered from a device counter, so that the residual reset falls on
+    // the same iterations; the node ends when the device's termination tests set ctl->done
+    int* base = &lm_->cg_base;
+    unsigned long long h = 0;
+    rc = new_cond(&h);
+    if (rc != POVAR_OK) return rc;
+    launch_cg_loop(d_.ctl, base, max_it, false, h, lc());
+    rc = capture_cond(cudaGraphCondTypeWhile, h, [&]() -> int {
+      for (int k = 1; k <= 10; ++k) {
+        const int rc2 = iteration(k, base);
+        if (rc2 != POVAR_OK) return rc2;
+      }
+      launch_cg_loop(d_.ctl, base, max_it, true, h, lc());
+      return POVAR_OK;
+    });
+    if (rc != POVAR_OK) return rc;
+  } else {
+    SeriesCtl* hctl = reinterpret_cast<SeriesCtl*>(host_out_);
+    constexpr int kBatch = 4;
+    for (int it = 1; it <= max_it;) {
+      for (int k = 0; k < kBatch && it <= max_it; ++k, ++it) {
+        rc = iteration(it, nullptr);
+        if (rc != POVAR_OK) return rc;
+      }
+      PV_CUDA(cudaMemcpyAsync(hctl, d_.ctl, sizeof(SeriesCtl), cudaMemcpyDeviceToHost, stream_));
+      PV_CUDA(cudaStreamSynchronize(stream_));
+      if (hctl->done) break;
+    }
   }
   launch_axpby(d_, n, -1.0, x, 0.0, nullptr, d_.vec_acc, lc());   // "negate the pose increment"
   launch_finite_check(d_, n, d_.vec_acc, lc());
-  PV_CUDA(cudaEventRecord(ev_[2], stream_));
+  PV_CUDA(mark(2));
   PV_CUDA(cudaGetLastError());
   return POVAR_OK;
 }
@@ -1714,7 +1753,7 @@ int Engine::solve_cholesky(double lambda) {
   const int n_pad = chol_padded(n);
   const bool tiled = chol_storage_ == 1 || static_cast<long long>(n_pad) * n_pad * 8 > kCholDenseCap;
   chol_tiled_active_ = tiled;
-  PV_CUDA(cudaEventRecord(ev_[0], stream_));
+  PV_CUDA(mark(0));
   int rc = prepare_reduced_system(false, lambda, 0.0);
   if (rc != POVAR_OK) return rc;
   if (tiled) {
@@ -1733,7 +1772,7 @@ int Engine::solve_cholesky(double lambda) {
     PV_CUDA(cudaMemsetAsync(d_.dense_S, 0, sizeof(double) * static_cast<size_t>(n_pad) * n_pad, stream_));
     launch_schur_lower(d_, mp_, d_.dense_S, n_pad, lc());
   }
-  PV_CUDA(cudaEventRecord(ev_[1], stream_));
+  PV_CUDA(mark(1));
   PV_CUDA(cudaMemsetAsync(chol_rhs_, 0, sizeof(double) * static_cast<size_t>(n_pad), stream_));
   int* info = d_.flags + 2;
   if (tiled) {
@@ -1746,6 +1785,13 @@ int Engine::solve_cholesky(double lambda) {
     launch_cholesky_factor(d_.dense_S, n_pad, chol_linv_, info, lc());
     launch_cholesky_solve(d_.dense_S, n_pad, chol_linv_, chol_rhs_, info, lc());
     PV_CUDA(cudaMemcpyAsync(d_.vec_acc, chol_rhs_, sizeof(double) * static_cast<size_t>(n), cudaMemcpyDeviceToDevice, stream_));
+  }
+  if (capturing_) {   // the read-back below as a kernel: info != 0 makes the step invalid
+    launch_chol_status(info, d_.ctl, lc());
+    launch_finite_check(d_, n, d_.vec_acc, lc());
+    PV_CUDA(mark(2));
+    PV_CUDA(cudaGetLastError());
+    return POVAR_OK;
   }
   int hinfo = 0;
   PV_CUDA(cudaMemcpyAsync(&hinfo, info, sizeof(int), cudaMemcpyDeviceToHost, stream_));
@@ -1762,7 +1808,7 @@ int Engine::solve_cholesky(double lambda) {
   } else {
     launch_finite_check(d_, n, d_.vec_acc, lc());
   }
-  PV_CUDA(cudaEventRecord(ev_[2], stream_));
+  PV_CUDA(mark(2));
   PV_CUDA(cudaGetLastError());
   return POVAR_OK;
 }
@@ -2273,6 +2319,257 @@ int Engine::bench_power_kernels(bool joint, int reps, double* seconds) {
     seconds[k] = elapsed(ev_[0], ev_[1]) / reps;
   }
   return POVAR_OK;
+}
+
+
+// ---------------------------------------------------------------------------------------------
+// povar_bundle_adjust_async: the two LM loops of host/lm_driver.cpp as ONE CUDA graph on the handle's stream.
+//
+//   step 1:  init_varproj -> cost -> k_lm_begin
+//            WHILE(run): k_lm_top; IF(lin) { linearize }; solve -> backup -> apply -> cost -> k_lm_decide;
+//                        IF(restore) { restore }
+//            k_lm_end_step
+//   IF(step 1 ok): to_homogeneous -> cost -> k_lm_begin -> the same WHILE for step 2 -> k_lm_end_step
+//   k_lm_finish
+//
+// The bodies are stream captures of the host route's own enqueue functions (capturing_ set): the damping comes from
+// the control block (lambda_dev_), the CG iterations from a device counter, the events become %globaltimer stamps
+// (mark), the power series and the CG loop become nested WHILE nodes, CHOLESKY's read-back a kernel.  Nothing in a
+// capture allocates or synchronises: build_solve_graph makes every allocation the host route makes lazily first.
+
+cudaError_t Engine::mark(int k) {
+  if (capturing_) {
+    launch_lm_stamp(&lm_->stamp[k], lc());
+    return cudaGetLastError();
+  }
+  return cudaEventRecord(ev_[k], stream_);
+}
+
+int Engine::new_cond(unsigned long long* h) {
+  cudaGraphConditionalHandle c = 0;
+  PV_CUDA(cudaGraphConditionalHandleCreate(&c, static_cast<cudaGraph_t>(cap_graph_), 0, 0));
+  *h = static_cast<unsigned long long>(c);
+  return POVAR_OK;
+}
+
+// a conditional node at the capture position of stream_ whose body `body` captures; the capture of the enclosing graph
+// continues behind the node
+int Engine::capture_cond(int type, unsigned long long h, const std::function<int()>& body) {
+  cudaGraph_t g = static_cast<cudaGraph_t>(cap_graph_);
+  cudaStreamCaptureStatus st = cudaStreamCaptureStatusNone;
+  const cudaGraphNode_t* deps = nullptr;
+  size_t num_deps = 0;
+  PV_CUDA(cudaStreamGetCaptureInfo(stream_, &st, nullptr, nullptr, &deps, &num_deps));
+  if (st != cudaStreamCaptureStatusActive) return fail(POVAR_ERR_CUDA, "stream capture of the solve is not active");
+  cudaGraphNodeParams params{};
+  params.type = cudaGraphNodeTypeConditional;
+  params.conditional.handle = static_cast<cudaGraphConditionalHandle>(h);
+  params.conditional.type = static_cast<cudaGraphConditionalNodeType>(type);
+  params.conditional.size = 1;
+  cudaGraphNode_t node = nullptr;
+  PV_CUDA(cudaGraphAddNode(&node, g, deps, num_deps, &params));
+  cudaGraph_t same = nullptr;
+  PV_CUDA(cudaStreamEndCapture(stream_, &same));
+  cap_graph_ = params.conditional.phGraph_out[0];
+  PV_CUDA(cudaStreamBeginCaptureToGraph(stream_, params.conditional.phGraph_out[0], nullptr, nullptr, 0,
+                                        cudaStreamCaptureModeRelaxed));
+  const int rc = body();
+  const cudaError_t e = cudaStreamEndCapture(stream_, &same);
+  cap_graph_ = g;
+  if (rc != POVAR_OK) return rc;
+  PV_CUDA(e);
+  PV_CUDA(cudaStreamBeginCaptureToGraph(stream_, g, &node, nullptr, 1, cudaStreamCaptureModeRelaxed));
+  return POVAR_OK;
+}
+
+// the series graph of enqueue_series, built into the graph being captured
+int Engine::capture_series(bool joint) {
+  const int m = opt_.power_sc_iterations;
+  unsigned long long h = 0;
+  const int rc = new_cond(&h);
+  if (rc != POVAR_OK) return rc;
+  SeriesLoop loop;
+  loop.handle = h;
+  loop.active = 1;
+  loop.max_terms = m;
+  launch_finish_b(d_, joint, lc());
+  launch_series_start(d_, opt_.r_tolerance, m, lc(), loop);
+  return capture_cond(cudaGraphCondTypeWhile, h, [&]() -> int {
+    const int rc2 = e0_product(joint, true, true);
+    launch_series_term(d_, joint, 0, opt_.eta, opt_.r_tolerance, term_mode(), exchange(), lc(), loop);
+    return rc2;
+  });
+}
+
+// one LM loop (run_step): iteration 0, then WHILE(run) over the trials; `ok`: the IF node of step 2 (step 1 only)
+int Engine::capture_lm_step(const povar_options& opt, bool joint, unsigned long long ok) {
+  const int step = joint ? 2 : 1;
+  const int max_iter = joint ? opt.max_num_iterations_step_2 : opt.max_num_iterations_step_1;
+  const bool power = joint ? opt.solver_type_step_2 == POVAR_RIPOBA
+                           : (opt.solver_type_step_1 == POVAR_POWER_VARPROJ ||
+                              opt.solver_type_step_1 == POVAR_POWER_SCHUR_COMPLEMENT);
+  PV_CUDA(mark(0));
+  int rc = enqueue_cost(joint, opt.alpha);
+  if (rc != POVAR_OK) return rc;
+  PV_CUDA(mark(1));
+  LmConds h;
+  rc = new_cond(&h.run);
+  if (rc != POVAR_OK) return rc;
+  launch_lm_begin(lm_, d_.trial_out, opt, step, lm_log_, lm_cap_, h, lc());
+  rc = capture_cond(cudaGraphCondTypeWhile, h.run, [&]() -> int {
+    LmConds b = h;
+    int rc2 = new_cond(&b.lin);
+    if (rc2 == POVAR_OK) rc2 = new_cond(&b.restore);
+    if (rc2 != POVAR_OK) return rc2;
+    launch_lm_top(lm_, b, lc());
+    rc2 = capture_cond(cudaGraphCondTypeIf, b.lin, [&]() { return linearize(joint, opt.alpha, true); });
+    if (rc2 != POVAR_OK) return rc2;
+    // Engine::trial: solve, backup, apply, (step 2: normalise,) cost, one exchange of trial_out[0..9)
+    rc2 = enqueue_solve(joint, 0.0);
+    if (rc2 == POVAR_OK) rc2 = backup(0);
+    if (rc2 == POVAR_OK) rc2 = enqueue_apply(joint, opt.alpha, /*reduce=*/false);
+    if (rc2 != POVAR_OK) return rc2;
+    if (joint) {
+      launch_normalize_cams(d_, lc());
+      launch_normalize_joint(d_, lc());
+    }
+    PV_CUDA(mark(3));
+    rc2 = enqueue_cost(joint, opt.alpha, /*reduce=*/false);
+    if (rc2 == POVAR_OK) rc2 = allreduce(d_.trial_out, 9);
+    if (rc2 != POVAR_OK) return rc2;
+    PV_CUDA(mark(4));
+    launch_lm_decide(lm_, d_.trial_out, d_.ctl, opt, step, power, lm_log_, lm_cap_, b, lc());
+    return capture_cond(cudaGraphCondTypeIf, b.restore, [&]() { return restore(0); });
+  });
+  if (rc != POVAR_OK) return rc;
+  launch_lm_end_step(lm_, step, max_iter, ok, lc());
+  PV_CUDA(cudaGetLastError());
+  return POVAR_OK;
+}
+
+int Engine::build_solve_graph(const povar_options& opt) {
+  // every allocation the host route makes on first use (linearize, solve_cholesky), and the control block and log
+  if (!d_.obs_d) {
+    PV_ALLOC(d_.obs_d, static_cast<size_t>(nnz_) * 3);
+    PV_ALLOC(d_.csc_d, static_cast<size_t>(nnz_) * 3);
+    PV_ALLOC(d_.sell_d, static_cast<size_t>(d_.ix.sell_slots) * 3);
+  }
+  if (opt_.robust_norm == POVAR_NORM_HUBER && !d_.obs_w) {
+    PV_ALLOC(d_.obs_w, static_cast<size_t>(nnz_));
+    PV_ALLOC(d_.csc_w, static_cast<size_t>(nnz_));
+    PV_ALLOC(d_.sell_w, static_cast<size_t>(d_.ix.sell_slots));
+  }
+  if (opt_.solver_type_step_1 == POVAR_CHOLESKY) {
+    const int n_pad = chol_padded(12 * C_);
+    const bool tiled = chol_storage_ == 1 || static_cast<long long>(n_pad) * n_pad * 8 > kCholDenseCap;
+    if (tiled && !chol_tiled_ready_) {
+      const int rc = setup_cholesky_tiles();
+      if (rc != POVAR_OK) return rc;
+    }
+    if (!tiled && !d_.dense_S) PV_ALLOC(d_.dense_S, static_cast<size_t>(n_pad) * n_pad);
+    if (!chol_linv_) {
+      PV_ALLOC(chol_linv_, static_cast<size_t>(n_pad) * 64);
+      PV_ALLOC(chol_rhs_, static_cast<size_t>(n_pad));
+    }
+  }
+  if (!lm_) {
+    PV_ALLOC(lm_, 1);
+    PV_ALLOC(lm_sum_, 1);
+    PV_ALLOC(lm_status_, 1);
+  }
+  const long long cap = 2LL + std::max(0, opt.max_num_iterations_step_1) + std::max(0, opt.max_num_iterations_step_2);
+  if (cap > std::numeric_limits<int>::max()) return fail(POVAR_ERR_INVALID, "too many iterations");
+  if (cap > lm_cap_) {
+    PV_ALLOC(lm_log_, static_cast<size_t>(cap));
+    lm_cap_ = static_cast<int>(cap);
+  }
+  cudaGraph_t graph = nullptr;
+  PV_CUDA(cudaGraphCreate(&graph, 0));
+  const long long before = launches_;
+  capturing_ = true;
+  cap_graph_ = graph;
+  lambda_dev_ = &lm_->loop.lambda;
+  auto body = [&]() -> int {
+    cudaError_t e = cudaStreamBeginCaptureToGraph(stream_, graph, nullptr, nullptr, 0, cudaStreamCaptureModeRelaxed);
+    if (e != cudaSuccess) return check(e, "cudaStreamBeginCaptureToGraph");
+    launch_lm_stamp(&lm_->t_start, lc());
+    launch_lm_stamp(&lm_->t_it, lc());
+    int rc = init_varproj(opt.alpha);   // :302-304
+    unsigned long long ok = kNoCond;
+    if (rc == POVAR_OK) rc = new_cond(&ok);
+    if (rc == POVAR_OK) rc = capture_lm_step(opt, false, ok);
+    if (rc == POVAR_OK) {
+      rc = capture_cond(cudaGraphCondTypeIf, ok, [&]() -> int {
+        int rc2 = to_homogeneous();   // create_homogeneous_landmark, :544-553
+        if (rc2 != POVAR_OK) return rc2;
+        launch_lm_stamp(&lm_->t_it, lc());
+        return capture_lm_step(opt, true, kNoCond);
+      });
+    }
+    if (rc != POVAR_OK) return rc;
+    launch_lm_finish(lm_, lm_cap_, lm_sum_, lm_status_, lc());
+    cudaGraph_t same = nullptr;
+    return check(cudaStreamEndCapture(stream_, &same), "cudaStreamEndCapture");
+  };
+  int rc = body();
+  capturing_ = false;
+  cap_graph_ = nullptr;
+  lambda_dev_ = nullptr;
+  launches_ = before;   // nothing ran
+  cudaStreamCaptureStatus st = cudaStreamCaptureStatusNone;
+  if (cudaStreamIsCapturing(stream_, &st) == cudaSuccess && st != cudaStreamCaptureStatusNone) {
+    cudaGraph_t dummy = nullptr;
+    cudaStreamEndCapture(stream_, &dummy);
+    if (dummy && dummy != graph) cudaGraphDestroy(dummy);
+  }
+  cudaGraphExec_t exec = nullptr;
+  if (rc == POVAR_OK) rc = check(cudaGraphInstantiate(&exec, graph, 0), "cudaGraphInstantiate");
+  cudaGraphDestroy(graph);
+  if (rc != POVAR_OK) {
+    cudaGetLastError();
+    return rc;
+  }
+  solve_graph_ = exec;
+  solve_opt_ = opt;
+  solve_window_ = d_.debug_window_cams;
+  solve_storage_ = chol_storage_;
+  return POVAR_OK;
+}
+
+int Engine::bundle_adjust_async(const povar_options& opt, povar_iteration* iterations, int max_iterations,
+                                povar_solve_summary* summary, int* status, cudaStream_t caller) {
+  PV_CUDA(cudaSetDevice(device_));
+  if (max_iterations > 0 && check_device_ptr(iterations, "iterations") != POVAR_OK) return POVAR_ERR_INVALID;
+  if (check_device_ptr(summary, "summary") != POVAR_OK) return POVAR_ERR_INVALID;
+  if (check_device_ptr(status, "status") != POVAR_OK) return POVAR_ERR_INVALID;
+  if (world_ > 1 && !peer_ok_) {
+    return fail(POVAR_ERR_UNSUPPORTED, "povar_bundle_adjust_async: the reductions of this handle go through "
+                                       "ncclAllReduce, which is not captured into graphs");
+  }
+  const bool same = solve_graph_ && std::memcmp(&solve_opt_, &opt, sizeof(opt)) == 0 &&
+                    solve_window_ == d_.debug_window_cams && solve_storage_ == chol_storage_;
+  if (!same) {
+    if (solve_graph_) {
+      PV_CUDA(cudaStreamSynchronize(stream_));   // a launch of the old graph may still be in flight
+      cudaGraphExecDestroy(static_cast<cudaGraphExec_t>(solve_graph_));
+      solve_graph_ = nullptr;
+    }
+    const int rc = build_solve_graph(opt);
+    if (rc != POVAR_OK) return rc;
+  }
+  int rc = wait_for(stream_, caller);
+  if (rc != POVAR_OK) return rc;
+  PV_CUDA(cudaGraphLaunch(static_cast<cudaGraphExec_t>(solve_graph_), stream_));
+  launch_lm_clip(lm_sum_, max_iterations, LaunchCfg{stream_, nullptr});
+  const int n = std::min(max_iterations, lm_cap_);
+  if (n > 0) {
+    PV_CUDA(cudaMemcpyAsync(iterations, lm_log_, sizeof(povar_iteration) * static_cast<size_t>(n),
+                            cudaMemcpyDeviceToDevice, stream_));
+  }
+  PV_CUDA(cudaMemcpyAsync(summary, lm_sum_, sizeof(povar_solve_summary), cudaMemcpyDeviceToDevice, stream_));
+  PV_CUDA(cudaMemcpyAsync(status, lm_status_, sizeof(int), cudaMemcpyDeviceToDevice, stream_));
+  PV_CUDA(cudaGetLastError());
+  return wait_for(caller, stream_);
 }
 
 }  // namespace povar

@@ -43,6 +43,10 @@ class Engine {
   int set_state(int which, const double* cam_P, const double* lms);
   int get_state_device(int which, double* cam_P, double* lms, cudaStream_t caller);
   int set_state_device(int which, const double* cam_P, const double* lms, cudaStream_t caller);
+  // povar_bundle_adjust_async: the solve as one CUDA graph (built on the first call with these options), enqueued
+  // behind the work on `caller`; the results land in device memory
+  int bundle_adjust_async(const povar_options& opt, povar_iteration* iterations, int max_iterations,
+                          povar_solve_summary* summary, int* status, cudaStream_t caller);
   int64_t debug_read(const char* name, double* out, int64_t capacity);
   int right_mul_e0(bool joint, const double* x, double* out);
   int bench_power_terms(bool joint, int terms, double* seconds_per_term);
@@ -93,6 +97,13 @@ class Engine {
   int enqueue_apply(bool joint, double alpha, bool reduce = true);
   int enqueue_series(bool joint);
   static void decode_cost(const double* v, povar_residual_info* out);
+  // the device-side solve (bundle_adjust_async): stream capture into nested conditional nodes
+  cudaError_t mark(int k);   // ev_[k], or a %globaltimer stamp into lm_->stamp[k] while capturing
+  int new_cond(unsigned long long* h);
+  int capture_cond(int type, unsigned long long h, const std::function<int()>& body);
+  int capture_series(bool joint);
+  int capture_lm_step(const povar_options& opt, bool joint, unsigned long long ok);
+  int build_solve_graph(const povar_options& opt);
   LaunchCfg lc() { return LaunchCfg{stream_, &launches_}; }
   double elapsed(cudaEvent_t a, cudaEvent_t b);
 
@@ -117,8 +128,20 @@ class Engine {
   // a power series as one CUDA graph per model (pOSE / joint): prefix + WHILE node around one term
   void* series_graph_[2] = {nullptr, nullptr};   // cudaGraphExec_t
   int series_calls_[2] = {0, 0};
+  ModelParams series_mp_[2] = {};                // the model parameters each series graph was captured with
   bool series_terms_counted_ = true;             // the term launches of the last series are in launches_
   void count_series_terms(int terms);
+  bool capturing_ = false;          // the enqueue functions are being captured into the solve graph
+  void* cap_graph_ = nullptr;       // cudaGraph_t the capture writes to
+  const double* lambda_dev_ = nullptr;   // while capturing: the damping in device memory (lm_->loop.lambda)
+  LmCtl* lm_ = nullptr;
+  povar_iteration* lm_log_ = nullptr;   // [lm_cap_] log of the device-side solve
+  int lm_cap_ = 0;
+  povar_solve_summary* lm_sum_ = nullptr;
+  int* lm_status_ = nullptr;
+  void* solve_graph_ = nullptr;     // cudaGraphExec_t of the solve, for solve_opt_ and the debug settings below
+  povar_options solve_opt_{};
+  int solve_window_ = 0, solve_storage_ = 0;
   double* chol_linv_ = nullptr;   // CHOLESKY: inverses of the factor's diagonal tiles [n_pad / 64][64][64]
   double* chol_rhs_ = nullptr;    // CHOLESKY: padded right-hand side / solution [n_pad]
   // CHOLESKY on tile-sparse storage (when the dense matrix would exceed kCholDenseCap, or forced)

@@ -17,11 +17,11 @@
 #include <cmath>
 #include <cstdio>
 #include <cstring>
-#include <limits>
 #include <string>
 #include <vector>
 
 #include "../engine.h"
+#include "../lm_step.h"
 
 namespace povar {
 const PhaseTimes& handle_times(povar_handle* h);
@@ -43,70 +43,34 @@ double seconds_since(Clock::time_point t0) {
   return std::chrono::duration<double>(Clock::now() - t0).count();
 }
 
+// Log::push: the non-timing columns are lm_log_push's (lm_step.h), the times are the host clock's and the events'
 struct Log {
   povar_iteration* out;
   int32_t capacity;
-  int32_t count = 0;
-  // cost (all / valid) of summary.iterations.back() as the reference's finish_iteration sees it
-  // (bal_bundle_adjustment.cpp:75-78): cost_change of a trial is measured against the previous LIST entry
-  double back_cost = 0.0, back_cost_valid = 0.0;
-  // last logged values (for failed trials the log repeats them, ba_log_utils.cpp:128-147)
-  double logged_cost = 0.0, logged_cost_valid = 0.0;
-  double logged_res_mean = 0.0, logged_res_valid_mean = 0.0;
-  int64_t logged_valid = 0;
-  // finish_solve (:97-159), kept here so that they do not depend on the caller's optional buffer
-  int32_t num_successful = 0, num_unsuccessful = 0;
-  double initial_cost = 0.0, final_cost = 0.0;
+  povar::LmLog st;
 
   void push(povar_handle* h, int step, int it, bool valid, bool successful, double trial_cost,
             const povar_residual_info* ri, double rel, double radius, int lin_it, double it_time,
             double cum_time) {
-    if (successful || count == 0 || (it == 0)) {
-      if (ri) {
-        logged_cost = ri->error_all;
-        logged_cost_valid = ri->error_valid;
-        logged_valid = ri->num_obs_valid;
-        logged_res_mean = ri->num_obs_all > 0 ? ri->residual_sum_all / static_cast<double>(ri->num_obs_all) : 0.0;
-        logged_res_valid_mean =
-            ri->num_obs_valid > 0 ? ri->residual_sum_valid / static_cast<double>(ri->num_obs_valid) : 0.0;
-      }
-    }
-    back_cost = ri ? ri->error_all : 0.0;   // an "Invalid" trial leaves a default-constructed cost
-    back_cost_valid = ri ? ri->error_valid : 0.0;
-    if (count == 0) initial_cost = logged_cost;
-    if (successful) {
-      ++num_successful;
-      final_cost = logged_cost;
-    } else {
-      ++num_unsuccessful;
-    }
+    povar_iteration* e = (st.count < capacity && out) ? out + st.count : nullptr;
+    povar::lm_log_push(st, e, step, it, valid, successful, trial_cost, ri, rel, radius, lin_it);
+    stamp(h, e, it_time, cum_time);
+  }
+  void stamp(povar_handle* h, povar_iteration* e, double it_time, double cum_time) {
     const povar::PhaseTimes& t = povar::handle_times(h);
-    if (count < capacity && out) {
-      povar_iteration& e = out[count];
-      e.step = step;
-      e.iteration = it;
-      e.step_is_valid = valid ? 1 : 0;
-      e.step_is_successful = successful ? 1 : 0;
-      e.cost = logged_cost;
-      e.cost_valid = logged_cost_valid;
-      e.trial_cost = trial_cost;
-      e.num_obs_valid = logged_valid;
-      e.relative_decrease = successful ? rel : 0.0;
-      e.trust_region_radius = radius;
-      e.linear_solver_iterations = lin_it;
-      e.iteration_time = it_time;
-      e.cumulative_time = cum_time;
-      e.residual_evaluation_time = t.residual;
-      e.jacobian_evaluation_time = t.linearize;
-      e.prepare_time = t.prepare;
-      e.solve_reduced_system_time = t.reduced_solve;
-      e.back_substitution_time = t.back_substitution;
-      e.residual_mean = logged_res_mean;
-      e.residual_valid_mean = logged_res_valid_mean;
+    if (e) {
+      e->iteration_time = it_time;
+      e->cumulative_time = cum_time;
+      e->residual_evaluation_time = t.residual;
+      e->jacobian_evaluation_time = t.linearize;
+      e->prepare_time = t.prepare;
+      e->solve_reduced_system_time = t.reduced_solve;
+      e->back_substitution_time = t.back_substitution;
     }
-    ++count;
     povar::handle_reset_times(h);
   }
+  // the entry the next push writes (nullptr: no room)
+  povar_iteration* next() { return (st.count < capacity && out) ? out + st.count : nullptr; }
 };
 
 struct StepResult {
@@ -115,21 +79,17 @@ struct StepResult {
   int rc = POVAR_OK;
 };
 
-// one LM loop; `joint` selects step 2
+// one LM loop; `joint` selects step 2.  The decisions are lm_step.h's (shared with the device-side solve).
 StepResult run_step(povar_handle* h, const povar_options& opt, bool joint, Log& log,
                     Clock::time_point t_total, bool verbose, long long* power_terms,
                     double* power_time) {
   StepResult res;
-  const double min_lambda = 1.0 / opt.max_trust_region_radius;
-  const double max_lambda = 1.0 / opt.min_trust_region_radius;
   const int max_iter = joint ? opt.max_num_iterations_step_2 : opt.max_num_iterations_step_1;
-  double lambda = 1.0 / opt.initial_trust_region_radius;
-  double vee = opt.initial_vee;
-  const int step = joint ? 2 : 1;
   const bool power = joint ? opt.solver_type_step_2 == POVAR_RIPOBA
                            : (opt.solver_type_step_1 == POVAR_POWER_VARPROJ ||
                               opt.solver_type_step_1 == POVAR_POWER_SCHUR_COMPLEMENT);
-  bool terminated = false;
+  povar::LmLoop s;
+  s.lambda = 1.0 / opt.initial_trust_region_radius;
   bool first = true;
 
   auto cost = [&](povar_residual_info* ri) {
@@ -138,7 +98,7 @@ StepResult run_step(povar_handle* h, const povar_options& opt, bool joint, Log& 
 
   povar_residual_info ri_accepted;   // cost of the state an accepted trial left behind
   bool have_accepted = false;
-  for (int it = 0; it <= max_iter && !terminated;) {
+  for (int it = 0; it <= max_iter && s.stop == povar::LM_RUNNING;) {
     Clock::time_point t_it = Clock::now();
     povar_residual_info ri;
     if (!joint && first) {
@@ -164,9 +124,10 @@ StepResult run_step(povar_handle* h, const povar_options& opt, bool joint, Log& 
       return res;
     }
     if (it == 0) {   // iteration 0 is just error evaluation and logging, :316-328
-      log.push(h, step, 0, true, true, ri.error_all, &ri, 0.0, 1.0 / lambda, 0, seconds_since(t_it),
-               seconds_since(t_total));
-      ++it;
+      povar_iteration* e = log.next();
+      povar::lm_begin(opt, joint, s, log.st, e, ri);
+      log.stamp(h, e, seconds_since(t_it), seconds_since(t_total));
+      it = s.it;
       continue;
     }
     res.rc = povar::handle_linearize_deferred(h, joint, opt.alpha);
@@ -175,7 +136,7 @@ StepResult run_step(povar_handle* h, const povar_options& opt, bool joint, Log& 
       return res;
     }
 
-    for (int j = 0; it <= max_iter && !terminated; ++j) {
+    for (int j = 0; it <= max_iter && s.stop == povar::LM_RUNNING; ++j) {
       if (j > 0) {
         if (verbose) std::printf("Iteration %d, backtracking\n", it);
         t_it = Clock::now();
@@ -184,7 +145,7 @@ StepResult run_step(povar_handle* h, const povar_options& opt, bool joint, Log& 
       double l_diff = 0.0;
       povar_residual_info ri2;
       // solve, backup, apply, (step 2) normalise, cost: :346-420 / :655-720, one synchronisation
-      const int src = povar::handle_trial(h, joint, opt.alpha, lambda, &lin_it, &l_diff, &ri2);
+      const int src = povar::handle_trial(h, joint, opt.alpha, s.lambda, &lin_it, &l_diff, &ri2);
       if (src < 0 || src == POVAR_NUM_LINEARIZATION) {
         res.rc = src;
         res.message = povar_last_error(h);
@@ -194,111 +155,48 @@ StepResult run_step(povar_handle* h, const povar_options& opt, bool joint, Log& 
         *power_terms += lin_it;
         *power_time += povar::handle_times(h).reduced_solve;
       }
-      if (src == POVAR_NUM_NONFINITE_INC) {   // :362-401
-        // the reference does not apply such an increment; here it was applied to the copy the backup protects
-        res.rc = povar_restore(h, joint ? POVAR_STATE_JOINT : POVAR_STATE_POSE);
-        if (res.rc != POVAR_OK) return res;
-        if (verbose) {
+      const double lambda = s.lambda;   // of this trial (printed)
+      const bool nonfinite = src == POVAR_NUM_NONFINITE_INC;
+      povar::LmEval ev;
+      povar_iteration* e = log.next();
+      const bool accepted = povar::lm_trial_step(opt, joint, s, log.st, e, ri, ri2, nonfinite, l_diff, lin_it, &ev);
+      log.stamp(h, e, seconds_since(t_it), seconds_since(t_total));
+      it = s.it;
+      if (verbose) {
+        if (nonfinite) {
           std::printf("\t[Invalid] Numeric issues when computing increment (contains NaNs), lambda: %.1e, cg_iter: %d\n",
                       lambda, lin_it);
-        }
-        lambda = vee * lambda;
-        vee *= opt.vee_factor;
-        log.push(h, step, it, false, false, std::numeric_limits<double>::quiet_NaN(), nullptr, 0.0,
-                 1.0 / lambda, lin_it, seconds_since(t_it), seconds_since(t_total));
-        ++it;
-        if (lambda > max_lambda) {
-          terminated = true;
-          res.termination = 1;
-          res.message = "Solver did not converge and reached maximum damping lambda";
-        }
-        continue;
-      }
-
-      bool valid = false, successful = false;
-      double rho = 0.0;
-      if (ri2.is_numerically_valid) {
-        double f_diff;
-        switch (opt.optimized_cost) {   // compute_cost_decrease, :163-176
-          case POVAR_COST_ERROR_VALID:
-            f_diff = ri.error_valid - ri2.error_valid;
-            break;
-          case POVAR_COST_ERROR_VALID_AVG:
-            f_diff = (ri.num_obs_valid > 0 ? ri.error_valid / ri.num_obs_valid : 0.0) -
-                     (ri2.num_obs_valid > 0 ? ri2.error_valid / ri2.num_obs_valid : 0.0);
-            l_diff /= static_cast<double>(ri.num_obs_valid);
-            break;
-          default:
-            f_diff = ri.error_all - ri2.error_all;
-        }
-        rho = f_diff / l_diff;
-        if (verbose) {
-          std::printf("\t[EVAL] f_diff %.4e l_diff %.4e ri1 %.4e ri2 %.4e\n", f_diff, l_diff,
-                      ri.error_valid, ri2.error_valid);
-        }
-        if (joint) {   // :742-745
-          valid = l_diff > 0;
-          successful = valid && rho > opt.min_relative_decrease;
-        } else {       // :442-445
-          valid = true;
-          successful = f_diff > 0;
+        } else {
+          if (ri2.is_numerically_valid) {
+            std::printf("\t[EVAL] f_diff %.4e l_diff %.4e ri1 %.4e ri2 %.4e\n", ev.f_diff, ev.l_diff,
+                        ri.error_valid, ri2.error_valid);
+          }
+          std::printf("\t[%s] error: %.4e (num valid: %lld), lambda: %.1e, cg_iter: %d, it_time: %.3fs, total_time: %.3fs\n",
+                      accepted ? "Success" : (ev.valid ? "Reject" : "Invalid"), ri2.error_all,
+                      static_cast<long long>(ri2.num_obs_valid), lambda, lin_it, seconds_since(t_it),
+                      seconds_since(t_total));
         }
       }
-
-      if (successful) {
-        if (verbose) {
-          std::printf("\t[Success] error: %.4e (num valid: %lld), lambda: %.1e, cg_iter: %d, it_time: %.3fs, total_time: %.3fs\n",
-                      ri2.error_all, static_cast<long long>(ri2.num_obs_valid), lambda, lin_it,
-                      seconds_since(t_it), seconds_since(t_total));
-        }
-        lambda *= std::max(1.0 / 3, 1 - std::pow(2 * rho - 1, 3));   // :461-463
-        lambda = std::max(min_lambda, lambda);
-        vee = opt.initial_vee;
-        const double prev_cost = log.back_cost, prev_cost_valid = log.back_cost_valid;
-        log.push(h, step, it, true, true, ri2.error_all, &ri2, rho, 1.0 / lambda, lin_it,
-                 seconds_since(t_it), seconds_since(t_total));
-        ++it;
+      if (accepted) {
         ri_accepted = ri2;
         have_accepted = true;
-        // function_tolerance_reached (:179-205): cost_change against the previous list entry
-        double cost_now, change;
-        if (opt.optimized_cost == POVAR_COST_ERROR) {
-          cost_now = ri2.error_all;
-          change = std::fabs(prev_cost - ri2.error_all);
-        } else {
-          cost_now = ri2.error_valid;
-          change = std::fabs(prev_cost_valid - ri2.error_valid);   // |cost_change.valid.error|, :190-194
-        }
-        if (change <= opt.function_tolerance * cost_now) {
-          terminated = true;
-          res.termination = 0;
-          char buf[160];
-          std::snprintf(buf, sizeof(buf), "Function tolerance reached. |cost_change|/cost: %g <= %g",
-                        change / cost_now, opt.function_tolerance);
-          res.message = buf;
-        }
         break;   // stop inner lm loop
       }
-      if (verbose) {
-        std::printf("\t[%s] error: %.4e (num valid: %lld), lambda: %.1e, cg_iter: %d, it_time: %.3fs, total_time: %.3fs\n",
-                    valid ? "Reject" : "Invalid", ri2.error_all, static_cast<long long>(ri2.num_obs_valid),
-                    lambda, lin_it, seconds_since(t_it), seconds_since(t_total));
-      }
-      lambda = vee * lambda;   // :498-499
-      vee *= opt.vee_factor;
-      log.push(h, step, it, valid, false, ri2.error_all, &ri2, 0.0, 1.0 / lambda, lin_it,
-               seconds_since(t_it), seconds_since(t_total));
+      // the reference does not apply a non-finite increment; here it was applied to the copy the backup protects
       res.rc = povar_restore(h, joint ? POVAR_STATE_JOINT : POVAR_STATE_POSE);
       if (res.rc != POVAR_OK) return res;
-      ++it;
-      if (lambda > max_lambda) {
-        terminated = true;
-        res.termination = 1;
-        res.message = "Solver did not converge and reached maximum damping lambda";
-      }
     }
   }
-  if (!terminated) {
+  if (s.stop == povar::LM_STOP_FUNCTION_TOLERANCE) {
+    res.termination = 0;
+    char buf[160];
+    std::snprintf(buf, sizeof(buf), "Function tolerance reached. |cost_change|/cost: %g <= %g", s.ftol_ratio,
+                  opt.function_tolerance);
+    res.message = buf;
+  } else if (s.stop == povar::LM_STOP_MAX_DAMPING) {
+    res.termination = 1;
+    res.message = "Solver did not converge and reached maximum damping lambda";
+  } else {
     res.termination = 1;
     char buf[128];
     std::snprintf(buf, sizeof(buf), "Solver did not converge after maximum number of %d iterations", max_iter);
@@ -340,7 +238,7 @@ extern "C" int povar_bundle_adjust(povar_handle* h, const povar_options* opt_in,
 
   if (summary) {
     std::memset(summary, 0, sizeof(*summary));
-    summary->num_iterations = std::min(log.count, log.capacity);
+    summary->num_iterations = std::min(log.st.count, log.capacity);
     summary->termination_type_step_1 = s1.termination;
     summary->termination_type_step_2 = s2.termination;
     summary->total_time = t_all;
@@ -349,10 +247,10 @@ extern "C" int povar_bundle_adjust(povar_handle* h, const povar_options* opt_in,
     summary->power_terms = power_terms;
     summary->power_series_time = power_time;
     // finish_solve (:97-159): iteration 0 entries count as successful; the reference subtracts one
-    summary->num_successful_steps = log.num_successful - 1;
-    summary->num_unsuccessful_steps = log.num_unsuccessful;
-    summary->initial_cost = log.initial_cost;
-    summary->final_cost = log.final_cost;
+    summary->num_successful_steps = log.st.num_successful - 1;
+    summary->num_unsuccessful_steps = log.st.num_unsuccessful;
+    summary->initial_cost = log.st.initial_cost;
+    summary->final_cost = log.st.final_cost;
     const std::string& msg = (s1.rc != POVAR_OK) ? s1.message : s2.message;
     std::snprintf(summary->message, sizeof(summary->message), "%s", msg.c_str());
   }

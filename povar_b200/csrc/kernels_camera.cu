@@ -374,9 +374,10 @@ __device__ __forceinline__ bool chol_inverse(double (&A)[D][D], double (&Inv)[D]
 template <bool JOINT, int MODE>
 __global__ void __launch_bounds__(kBlock)
 k_cam_binv16(int C, const double* __restrict__ P, const double* __restrict__ kron,
-             const double* __restrict__ pose_scale, double lambda, double* __restrict__ Bmat,
-             double* __restrict__ Binv) {
+             const double* __restrict__ pose_scale, double lambda, const double* __restrict__ lambda_dev,
+             double* __restrict__ Bmat, double* __restrict__ Binv) {
   constexpr int D = JOINT ? 11 : 12;
+  if (MODE == 0 && lambda_dev != nullptr) lambda = *lambda_dev;
   constexpr int kCams = kBlock / 16;
   __shared__ double As[kCams][12][13];
   __shared__ double Us[kCams][12];
@@ -1083,12 +1084,12 @@ void launch_cam_scale(const DeviceState& d, const ModelParams& mp, const LaunchC
   count(lc);
 }
 
-void launch_cam_binv(const DeviceState& d, bool joint, double lambda, const LaunchCfg& lc) {
+void launch_cam_binv(const DeviceState& d, bool joint, double lambda, const LaunchCfg& lc, const double* lambda_dev) {
   const int blocks16 = (d.ix.C + kBlock / 16 - 1) / (kBlock / 16);
   if (joint) {
-    k_cam_binv16<true, 0><<<blocks16, kBlock, 0, lc.stream>>>(d.ix.C, d.P, d.kron, d.pose_scale, lambda, d.Bmat, d.Binv);
+    k_cam_binv16<true, 0><<<blocks16, kBlock, 0, lc.stream>>>(d.ix.C, d.P, d.kron, d.pose_scale, lambda, lambda_dev, d.Bmat, d.Binv);
   } else {
-    k_cam_binv16<false, 0><<<blocks16, kBlock, 0, lc.stream>>>(d.ix.C, d.P, d.kron, d.pose_scale, lambda, d.Bmat, d.Binv);
+    k_cam_binv16<false, 0><<<blocks16, kBlock, 0, lc.stream>>>(d.ix.C, d.P, d.kron, d.pose_scale, lambda, lambda_dev, d.Bmat, d.Binv);
   }
   count(lc);
 }
@@ -1096,9 +1097,9 @@ void launch_cam_binv(const DeviceState& d, bool joint, double lambda, const Laun
 void launch_cam_precond(const DeviceState& d, bool joint, const double* kron_sdiag, const LaunchCfg& lc) {
   const int blocks16 = (d.ix.C + kBlock / 16 - 1) / (kBlock / 16);
   if (joint) {
-    k_cam_binv16<true, 1><<<blocks16, kBlock, 0, lc.stream>>>(d.ix.C, d.P, kron_sdiag, d.pose_scale, 0.0, d.Bmat, d.Mprec);
+    k_cam_binv16<true, 1><<<blocks16, kBlock, 0, lc.stream>>>(d.ix.C, d.P, kron_sdiag, d.pose_scale, 0.0, nullptr, d.Bmat, d.Mprec);
   } else {
-    k_cam_binv16<false, 1><<<blocks16, kBlock, 0, lc.stream>>>(d.ix.C, d.P, kron_sdiag, d.pose_scale, 0.0, d.Bmat, d.Mprec);
+    k_cam_binv16<false, 1><<<blocks16, kBlock, 0, lc.stream>>>(d.ix.C, d.P, kron_sdiag, d.pose_scale, 0.0, nullptr, d.Bmat, d.Mprec);
   }
   count(lc);
 }

@@ -455,10 +455,11 @@ template <bool JOINT>
 __global__ void __launch_bounds__(kBlock)
 k_prep_long(int num_long, const int* __restrict__ long_lm, const double* __restrict__ X,
             const double* __restrict__ lm_hraw, const double* __restrict__ lm_graw,
-            const double* __restrict__ lm_scale, double lambda_lm, double* __restrict__ hll_inv,
-            double* __restrict__ lm_rec, double* __restrict__ lm_fold) {
+            const double* __restrict__ lm_scale, double lambda_lm, const double* __restrict__ lambda_dev,
+            double* __restrict__ hll_inv, double* __restrict__ lm_rec, double* __restrict__ lm_fold) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= num_long) return;
+  if (lambda_dev != nullptr) lambda_lm = *lambda_dev;
   const int l = long_lm[i];
   double x[4], s[4], inv[6], H[4], fold[10];
   load_lm4(X, l, x);
@@ -484,10 +485,12 @@ template <bool JOINT>
 __global__ void __launch_bounds__(kBlock)
 k_prep_sell(int slots, const int* __restrict__ sell_lm, const double* __restrict__ sell_x,
             const double* __restrict__ sell_hraw, const double* __restrict__ sell_graw,
-            const double* __restrict__ sell_scale, double lambda_lm, double* __restrict__ sell_hinv,
-            double* __restrict__ sell_fold, double* __restrict__ hll_inv, double* __restrict__ lm_rec) {
+            const double* __restrict__ sell_scale, double lambda_lm, const double* __restrict__ lambda_dev,
+            double* __restrict__ sell_hinv, double* __restrict__ sell_fold, double* __restrict__ hll_inv,
+            double* __restrict__ lm_rec) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= slots) return;
+  if (lambda_dev != nullptr) lambda_lm = *lambda_dev;
   const int sl = i / kSellWidth, lane = i % kSellWidth;
   const int lm = sell_lm[i];
   double* ip = sell_hinv + 6 * kSellWidth * static_cast<size_t>(sl) + lane;
@@ -1518,18 +1521,18 @@ void launch_lin_landmark(const DeviceState& d, const ModelParams& mp, bool joint
 }
 
 void launch_prep_landmark(const DeviceState& d, bool joint, double lambda_lm, bool hinv_by_landmark,
-                          const LaunchCfg& lc) {
+                          const LaunchCfg& lc, const double* lambda_dev) {
   const int slots = kSellWidth * d.ix.num_slices;
   double* hinv_out = hinv_by_landmark ? d.hll_inv : nullptr;
   if (slots > 0) {
     const int blocks = (slots + kBlock - 1) / kBlock;
     if (joint) {
       k_prep_sell<true><<<blocks, kBlock, 0, lc.stream>>>(slots, d.ix.sell_lm, d.sell_x, d.sell_hraw, d.sell_graw,
-                                                          d.sell_scale, lambda_lm, d.sell_hinv, d.sell_fold, hinv_out,
+                                                          d.sell_scale, lambda_lm, lambda_dev, d.sell_hinv, d.sell_fold, hinv_out,
                                                           d.lm_rec);
     } else {
       k_prep_sell<false><<<blocks, kBlock, 0, lc.stream>>>(slots, d.ix.sell_lm, d.sell_x, d.sell_hraw, d.sell_graw,
-                                                           d.sell_scale, lambda_lm, d.sell_hinv, d.sell_fold, hinv_out,
+                                                           d.sell_scale, lambda_lm, lambda_dev, d.sell_hinv, d.sell_fold, hinv_out,
                                                            d.lm_rec);
     }
     count(lc);
@@ -1538,10 +1541,10 @@ void launch_prep_landmark(const DeviceState& d, bool joint, double lambda_lm, bo
     const int blocks = (d.ix.num_long + kBlock - 1) / kBlock;
     if (joint) {
       k_prep_long<true><<<blocks, kBlock, 0, lc.stream>>>(d.ix.num_long, d.ix.long_lm, d.X, d.lm_hraw, d.lm_graw,
-                                                          d.lm_scale, lambda_lm, d.hll_inv, d.lm_rec, d.lm_fold);
+                                                          d.lm_scale, lambda_lm, lambda_dev, d.hll_inv, d.lm_rec, d.lm_fold);
     } else {
       k_prep_long<false><<<blocks, kBlock, 0, lc.stream>>>(d.ix.num_long, d.ix.long_lm, d.X, d.lm_hraw, d.lm_graw,
-                                                           d.lm_scale, lambda_lm, d.hll_inv, d.lm_rec, d.lm_fold);
+                                                           d.lm_scale, lambda_lm, lambda_dev, d.hll_inv, d.lm_rec, d.lm_fold);
     }
     count(lc);
   }

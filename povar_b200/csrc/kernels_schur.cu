@@ -50,9 +50,10 @@ k_dot_final(int nblocks, const double* __restrict__ part, double* out) {
 // ---- conjugate gradients on the device (cg/conjugate_gradient.hpp:114-489): the scalar recurrences and every
 // termination test of the reference's loop, one thread, after the ordered sum of the dot-product partials
 __global__ void __launch_bounds__(kBlock)
-k_cg_scalar(int nblocks, const double* __restrict__ part, int stage, int it, double eta, int min_it, int max_it,
-            CgState* cg, SeriesCtl* ctl) {
+k_cg_scalar(int nblocks, const double* __restrict__ part, int stage, int it, const int* __restrict__ it_base, double eta,
+            int min_it, int max_it, CgState* cg, SeriesCtl* ctl) {
   if (stage != CG_BEGIN && ctl->done) return;
+  if (it_base != nullptr) it += *it_base;
   __shared__ double smem[kBlock / 32];
   double acc[1] = {0.0};
   for (int b = threadIdx.x; b < nblocks; b += blockDim.x) acc[0] += part[b];
@@ -111,9 +112,10 @@ k_cg_scalar(int nblocks, const double* __restrict__ part, int stage, int it, dou
 
 // p = z (+ beta p);  x += alpha p;  r -= alpha q  -- with the device's scalars, nothing after termination
 __global__ void __launch_bounds__(kBlock)
-k_cg_update(int n, int what, int it, const double* __restrict__ src, double* __restrict__ dst,
-            const CgState* __restrict__ cg, const SeriesCtl* __restrict__ ctl) {
+k_cg_update(int n, int what, int it, const int* __restrict__ it_base, const double* __restrict__ src,
+            double* __restrict__ dst, const CgState* __restrict__ cg, const SeriesCtl* __restrict__ ctl) {
   if (ctl->done) return;
+  if (it_base != nullptr) it += *it_base;
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
   if (what == CG_UPDATE_P) {
@@ -163,18 +165,19 @@ void launch_dot_partials(const DeviceState& d, int n, const double* x, const dou
 }
 
 void launch_cg_scalar(const DeviceState& d, CgStage stage, int it, double eta, int min_it, int max_it,
-                      const LaunchCfg& lc) {
+                      const LaunchCfg& lc, const int* it_base) {
   int blocks = (d.ix.C * 12 + kBlock - 1) / kBlock;   // as launch_dot_partials for a camera-sized vector
   const int cap = scalar_blocks(d);
   if (blocks > cap) blocks = cap;
-  k_cg_scalar<<<1, kBlock, 0, lc.stream>>>(blocks, d.scalar_part, static_cast<int>(stage), it, eta, min_it, max_it, d.cg,
+  k_cg_scalar<<<1, kBlock, 0, lc.stream>>>(blocks, d.scalar_part, static_cast<int>(stage), it, it_base, eta, min_it, max_it, d.cg,
                                            d.ctl);
   count(lc);
 }
 
 void launch_cg_update(const DeviceState& d, CgUpdate what, int n, int it, const double* src, double* dst,
-                      const LaunchCfg& lc) {
-  k_cg_update<<<(n + kBlock - 1) / kBlock, kBlock, 0, lc.stream>>>(n, static_cast<int>(what), it, src, dst, d.cg, d.ctl);
+                      const LaunchCfg& lc, const int* it_base) {
+  k_cg_update<<<(n + kBlock - 1) / kBlock, kBlock, 0, lc.stream>>>(n, static_cast<int>(what), it, it_base, src, dst, d.cg,
+                                                                   d.ctl);
   count(lc);
 }
 

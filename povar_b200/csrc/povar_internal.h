@@ -9,6 +9,7 @@
 #include <vector>
 
 #include "../../include/povar_b200.h"
+#include "lm_step.h"
 
 namespace povar {
 
@@ -296,8 +297,9 @@ void launch_flag_to_double(const DeviceState& d, const LaunchCfg& lc);
 void launch_lin_landmark(const DeviceState& d, const ModelParams& mp, bool joint, bool scale_jl,
                          const LaunchCfg& lc);
 // hinv_by_landmark: also store Hll^-1 of the sliced-ELL landmarks by landmark (PCG / CHOLESKY read it camera-major)
+// lambda_dev (not null): the damping is read from device memory instead (the device-side solve)
 void launch_prep_landmark(const DeviceState& d, bool joint, double lambda_lm, bool hinv_by_landmark,
-                          const LaunchCfg& lc);
+                          const LaunchCfg& lc, const double* lambda_dev = nullptr);
 void launch_backsub_varpro(const DeviceState& d, const ModelParams& mp, const double* inc,
                            const LaunchCfg& lc);
 void launch_backsub_poba(const DeviceState& d, const ModelParams& mp, const double* y,
@@ -316,7 +318,8 @@ void launch_kron(const DeviceState& d, const ModelParams& mp, bool joint, KronKi
 void launch_reduce_items(const DeviceState& d, const double* item_vals, int width, double* out,
                          bool in_series, const LaunchCfg& lc);
 void launch_cam_scale(const DeviceState& d, const ModelParams& mp, const LaunchCfg& lc);
-void launch_cam_binv(const DeviceState& d, bool joint, double lambda, const LaunchCfg& lc);
+void launch_cam_binv(const DeviceState& d, bool joint, double lambda, const LaunchCfg& lc,
+                     const double* lambda_dev = nullptr);
 void launch_cam_precond(const DeviceState& d, bool joint, const double* kron_sdiag, const LaunchCfg& lc);
 enum PassBMode { PASSB_E0 = 0, PASSB_B = 1 };
 void launch_passB(const DeviceState& d, const ModelParams& mp, bool joint, const LaunchCfg& lc);
@@ -410,9 +413,55 @@ void launch_perm_scatter(int C, const int* perm, const double* r, double* x, con
 // at once when ctl->done is set
 enum CgStage { CG_BEGIN = 0, CG_RHO = 1, CG_PQ = 2, CG_ZETA = 3 };
 // reduces the partials of the preceding launch_dot_partials and applies stage `stage` of iteration `it`
-void launch_cg_scalar(const DeviceState& d, CgStage stage, int it, double eta, int min_it, int max_it, const LaunchCfg& lc);
+// it_base (not null): the iteration is it + *it_base (the loop of the device-side solve counts on the device)
+void launch_cg_scalar(const DeviceState& d, CgStage stage, int it, double eta, int min_it, int max_it, const LaunchCfg& lc,
+                      const int* it_base = nullptr);
 void launch_dot_partials(const DeviceState& d, int n, const double* x, const double* y, const LaunchCfg& lc);
 enum CgUpdate { CG_UPDATE_P = 0, CG_UPDATE_X = 1, CG_UPDATE_R = 2 };
-void launch_cg_update(const DeviceState& d, CgUpdate what, int n, int it, const double* src, double* dst, const LaunchCfg& lc);
+void launch_cg_update(const DeviceState& d, CgUpdate what, int n, int it, const double* src, double* dst, const LaunchCfg& lc,
+                      const int* it_base = nullptr);
+
+// ---- the LM loops on the device (kernels_lm.cu, Engine::bundle_adjust_async) ----
+// control block of the device-side solve: the state run_step / povar_bundle_adjust keep on the host
+enum LmMessage { LM_MSG_NONE = 0, LM_MSG_LINEARIZATION, LM_MSG_PEER_TIMEOUT, LM_MSG_FUNCTION_TOLERANCE,
+                 LM_MSG_MAX_DAMPING, LM_MSG_MAX_ITERATIONS };
+struct LmCtl {
+  LmLoop loop;
+  LmLog log;
+  povar_residual_info ri;           // cost of the current state
+  int32_t status;                   // what povar_bundle_adjust returns
+  int32_t termination[2];
+  int32_t message, message_iterations;
+  int32_t lin_next;                 // the next trial starts with a linearisation (its failure flag is read with the trial)
+  int32_t cg_base;                  // PCG / RIPCG: iterations of the running solve before the current loop body
+  long long power_terms;
+  double power_time;
+  double times[5];                  // residual, linearize, prepare, reduced solve, back-substitution (s, since the last entry)
+  unsigned long long t_start, t_it, t_step1;
+  unsigned long long stamp[8];      // %globaltimer where the host route records its events ev_[0..7]
+};
+// condition handles of the graph (cudaGraphConditionalHandle values; kNoCond: none)
+constexpr unsigned long long kNoCond = ~0ULL;
+struct LmConds {
+  unsigned long long run = kNoCond, lin = kNoCond, restore = kNoCond;
+};
+void launch_lm_stamp(unsigned long long* at, const LaunchCfg& lc);
+// t_it = now; the IF(linearise) node of the trial body runs when ctl->lin_next
+void launch_lm_top(LmCtl* ctl, const LmConds& h, const LaunchCfg& lc);
+// iteration 0 of step `step` from the cost in trial_out[0..8) (stamps 0 / 1 around it); step 1 also resets ctl
+void launch_lm_begin(LmCtl* ctl, const double* trial_out, const povar_options& opt, int step, povar_iteration* log,
+                     int capacity, const LmConds& h, const LaunchCfg& lc);
+// the decision of one trial (lm_trial_step) and its log entry
+void launch_lm_decide(LmCtl* ctl, const double* trial_out, const SeriesCtl* sctl, const povar_options& opt, int step,
+                      bool power, povar_iteration* log, int capacity, const LmConds& h, const LaunchCfg& lc);
+// termination type and message of a step; step 1: `ok` (IF node of step 2) = no failure
+void launch_lm_end_step(LmCtl* ctl, int step, int max_iter, unsigned long long ok, const LaunchCfg& lc);
+void launch_lm_finish(LmCtl* ctl, int capacity, povar_solve_summary* summary, int* status, const LaunchCfg& lc);
+// summary->num_iterations = min(it, max_iterations): the caller's capacity, applied after the graph
+void launch_lm_clip(povar_solve_summary* summary, int max_iterations, const LaunchCfg& lc);
+// CHOLESKY inside a graph: info != 0 -> an invalid step (what solve_cholesky's host read-back does)
+void launch_chol_status(const int* info, SeriesCtl* ctl, const LaunchCfg& lc);
+// PCG / RIPCG inside a graph: the WHILE node around 10 iterations; advance = 0 before the node (base = 0)
+void launch_cg_loop(SeriesCtl* ctl, int* base, int max_it, bool advance, unsigned long long handle, const LaunchCfg& lc);
 
 }  // namespace povar
