@@ -1094,7 +1094,6 @@ int Engine::build_index(int sell_n, const int* long_lms, const double* host_uv, 
   PV_ALLOC(d_.cost_part, static_cast<size_t>(cost_blocks(d_)) * 8);
   PV_ALLOC(d_.cost_out, 1);
   PV_ALLOC(d_.scalar_part, static_cast<size_t>(scalar_blocks(d_)) + 8);
-  PV_ALLOC(d_.scalar_out, 8);
   PV_ALLOC(d_.trial_out, 16);
   PV_ALLOC(d_.flags, 4);
   PV_ALLOC(d_.ctl, 1);
@@ -1272,19 +1271,18 @@ int Engine::allreduce(double* buf, size_t n, bool skip_when_done) {
   return POVAR_OK;
 }
 
-void Engine::set_model(bool joint, double alpha) {
+void Engine::set_model(double alpha) {
   mp_.c1 = std::sqrt(1.0 - alpha);
   mp_.c2 = std::sqrt(alpha);
   mp_.robust_norm = opt_.robust_norm;
   mp_.huber = opt_.huber_parameter;
   mp_.jacobi_eps = opt_.jacobi_scaling_epsilon > 0 ? opt_.jacobi_scaling_epsilon : kEpsSqrtHost;
-  (void)joint;
 }
 
 // ---------------------------------------------------------------------------------------------
 int Engine::init_varproj(double alpha) {
   PV_CUDA(cudaSetDevice(device_));
-  set_model(false, alpha);
+  set_model(alpha);
   launch_init_varproj(d_, mp_, lc());
   PV_CUDA(cudaGetLastError());
   return POVAR_OK;
@@ -1292,7 +1290,7 @@ int Engine::init_varproj(double alpha) {
 
 // cost kernels + (sharded) the in-place sum over the ranks: the result is trial_out[0..7] on the device
 int Engine::enqueue_cost(bool joint, double alpha, bool reduce) {
-  set_model(joint, joint ? opt_.alpha : alpha);
+  set_model(joint ? opt_.alpha : alpha);
   launch_cost(d_, mp_, joint, lc());
   return reduce ? allreduce(d_.trial_out, 8) : POVAR_OK;
 }
@@ -1324,16 +1322,9 @@ int Engine::cost(bool joint, double alpha, povar_residual_info* out) {
   return POVAR_OK;
 }
 
-int Engine::linearize(bool joint, double alpha, bool defer_check) {
-  PV_CUDA(cudaSetDevice(device_));
-  set_model(joint, joint ? opt_.alpha : alpha);
-  joint_lin_ = joint ? 1 : 0;
-  have_solve_ = false;
-  dim_ = joint ? 11 : 12;
-  const bool power = joint ? true
-                           : (opt_.solver_type_step_1 == POVAR_POWER_VARPROJ ||
-                              opt_.solver_type_step_1 == POVAR_POWER_SCHUR_COMPLEMENT);
-  // per-observation coefficients the term kernels stream (kernels_series.cu): first use allocates
+// per-observation coefficients the term kernels stream (kernels_series.cu): step 2's coefficients, step 1's HUBER
+// weights
+int Engine::alloc_lin_buffers(bool joint) {
   if (joint && !d_.obs_d) {
     PV_ALLOC(d_.obs_d, static_cast<size_t>(nnz_) * 3);
     PV_ALLOC(d_.csc_d, static_cast<size_t>(nnz_) * 3);
@@ -1344,11 +1335,24 @@ int Engine::linearize(bool joint, double alpha, bool defer_check) {
     PV_ALLOC(d_.csc_w, static_cast<size_t>(nnz_));
     PV_ALLOC(d_.sell_w, static_cast<size_t>(d_.ix.sell_slots));
   }
+  return POVAR_OK;
+}
+
+int Engine::linearize(bool joint, double alpha, bool defer_check) {
+  PV_CUDA(cudaSetDevice(device_));
+  set_model(joint ? opt_.alpha : alpha);
+  joint_lin_ = joint ? 1 : 0;
+  have_solve_ = false;
+  dim_ = joint ? 11 : 12;
+  {
+    const int rc = alloc_lin_buffers(joint);
+    if (rc != POVAR_OK) return rc;
+  }
   PV_CUDA(mark(6));
   PV_CUDA(cudaMemsetAsync(d_.flags, 0, 4 * sizeof(int), stream_));
   // landmark side: Jl^T Jl, Jl^T r, column scales (LinearizorSC step 1 does not scale Jl:
-  // solver/linearizor_sc.cpp:174-203)
-  launch_lin_landmark(d_, mp_, joint, power, lc());
+  // solver/linearizor_sc.cpp:174-203; step 2 scales it for every solver)
+  launch_lin_landmark(d_, mp_, joint, joint || lm_power_step(opt_, false), lc());
   // camera side: Jp^T Jp as Kronecker sums, then the pose scales
   launch_kron(d_, mp_, joint, KRON_HPP, lc());
   launch_reduce_items(d_, d_.item_kron, kKron, d_.kron, false, lc());
@@ -1418,12 +1422,13 @@ int Engine::solve_power(bool joint, double lambda) {
 
 // One power series is b -> x0, series start, then per term landmark half, camera half, term kernel -- the same
 // arguments in every solve of a model (the damping enters before, the stopping rule is applied on the device, the
-// number of a peer exchange and of a term are device-side counters).  It is built once per model as a CUDA graph
-// with a conditional WHILE node whose body is one term: k_series_start and the last block of k_term16 set the
-// condition (cudaGraphSetConditional), so a solve is ONE launch that runs exactly the terms the reference's
+// number of a peer exchange and of a term are device-side counters).  capture_series builds it once per model as a
+// CUDA graph with a conditional WHILE node whose body is one term: k_series_start and the last block of k_term16 set
+// the condition (cudaGraphSetConditional), so a solve is ONE launch that runs exactly the terms the reference's
 // stopping rule asks for.  (Until this round the graph held all m terms and the converged ones returned at once:
 // 430 skipped launches of 2-4 us per venice-1778 solve.)  The first solve of a model runs eagerly -- it sets
-// function attributes -- and so does a series whose exchange is ncclAllReduce (no peer memory).
+// function attributes -- and so does a series whose exchange is ncclAllReduce (no peer memory).  Inside the solve
+// graph the same prefix and WHILE node go into the graph being captured.
 int Engine::enqueue_series(bool joint) {
   if (capturing_) return capture_series(joint);
   const int m = opt_.power_sc_iterations;
@@ -1449,68 +1454,9 @@ int Engine::enqueue_series(bool joint) {
     series_graph_[which] = nullptr;
   }
   if (!series_graph_[which]) {
-    const long long before = launches_;
-    cudaGraph_t graph = nullptr;
-    cudaGraphConditionalHandle handle = 0;
-    PV_CUDA(cudaGraphCreate(&graph, 0));
-    auto bail = [&](cudaError_t e, const char* what) {
-      cudaStreamCaptureStatus st = cudaStreamCaptureStatusNone;
-      if (cudaStreamIsCapturing(stream_, &st) == cudaSuccess && st != cudaStreamCaptureStatusNone) {
-        cudaGraph_t dummy = nullptr;
-        cudaStreamEndCapture(stream_, &dummy);
-      }
-      cudaGraphDestroy(graph);
-      cudaGetLastError();
-      launches_ = before;
-      return e != cudaSuccess ? check(e, what) : fail(POVAR_ERR_CUDA, what);
-    };
-    cudaError_t e = cudaGraphConditionalHandleCreate(&handle, graph, 0, 0);   // set by k_series_start in every run
-    if (e != cudaSuccess) return bail(e, "cudaGraphConditionalHandleCreate");
-    SeriesLoop loop;
-    loop.handle = static_cast<unsigned long long>(handle);
-    loop.active = 1;
-    loop.max_terms = m;
-    // prefix: b -> x0, norms, loop condition
-    e = cudaStreamBeginCaptureToGraph(stream_, graph, nullptr, nullptr, 0, cudaStreamCaptureModeThreadLocal);
-    if (e != cudaSuccess) return bail(e, "cudaStreamBeginCaptureToGraph");
-    launch_finish_b(d_, joint, lc());
-    launch_series_start(d_, opt_.r_tolerance, m, lc(), loop);
-    cudaStreamCaptureStatus status = cudaStreamCaptureStatusNone;
-    const cudaGraphNode_t* deps = nullptr;
-    size_t num_deps = 0;
-    e = cudaStreamGetCaptureInfo(stream_, &status, nullptr, nullptr, &deps, &num_deps);
-    if (e != cudaSuccess || status != cudaStreamCaptureStatusActive) return bail(e, "cudaStreamGetCaptureInfo");
-    cudaGraphNodeParams params{};
-    params.type = cudaGraphNodeTypeConditional;
-    params.conditional.handle = handle;
-    params.conditional.type = cudaGraphCondTypeWhile;
-    params.conditional.size = 1;
-    cudaGraphNode_t loop_node = nullptr;
-    e = cudaGraphAddNode(&loop_node, graph, deps, num_deps, &params);
-    if (e != cudaSuccess) return bail(e, "cudaGraphAddNode(conditional)");
-    e = cudaStreamUpdateCaptureDependencies(stream_, &loop_node, 1, cudaStreamSetCaptureDependencies);
-    if (e != cudaSuccess) return bail(e, "cudaStreamUpdateCaptureDependencies");
-    cudaGraph_t same = nullptr;
-    e = cudaStreamEndCapture(stream_, &same);
-    if (e != cudaSuccess) return bail(e, "cudaStreamEndCapture");
-    // body: one term
-    cudaGraph_t body = params.conditional.phGraph_out[0];
-    e = cudaStreamBeginCaptureToGraph(stream_, body, nullptr, nullptr, 0, cudaStreamCaptureModeThreadLocal);
-    if (e != cudaSuccess) return bail(e, "cudaStreamBeginCaptureToGraph(body)");
-    const int rc = e0_product(joint, true, true);
-    launch_series_term(d_, joint, 0, opt_.eta, opt_.r_tolerance, term_mode(), exchange(), lc(), loop);
-    e = cudaStreamEndCapture(stream_, &same);
-    if (rc != POVAR_OK || e != cudaSuccess) return bail(e, "stream capture of a power-series term failed");
-    cudaGraphExec_t exec = nullptr;
-    e = cudaGraphInstantiate(&exec, graph, 0);
-    cudaGraphDestroy(graph);
-    if (e != cudaSuccess) {
-      launches_ = before;
-      return check(e, "cudaGraphInstantiate");
-    }
-    series_graph_[which] = exec;
+    const int rc = capture_graph(&series_graph_[which], [&]() { return capture_series(joint); });
+    if (rc != POVAR_OK) return rc;
     series_mp_[which] = mp_;
-    launches_ = before;   // nothing ran during the capture
   }
   PV_CUDA(cudaGraphLaunch(static_cast<cudaGraphExec_t>(series_graph_[which]), stream_));
   launches_ += 2;                  // b -> x0 and the series start; the terms are counted when the solve reports them
@@ -1545,7 +1491,6 @@ void Engine::count_series_terms(int terms) {
 int Engine::enqueue_solve(bool joint, double lambda) {
   if (static_cast<int>(joint) != joint_lin_) return fail(POVAR_ERR_INVALID, "solve called without a matching linearize");
   have_solve_ = true;
-  lambda_ = lambda;
   if (joint) return opt_.solver_type_step_2 == POVAR_RIPOBA ? solve_power(true, lambda) : solve_pcg(true, lambda);
   switch (opt_.solver_type_step_1) {
     case POVAR_POWER_VARPROJ:
@@ -1717,10 +1662,6 @@ int Engine::setup_cholesky_tiles() {
   }
   int *slot = nullptr, *col_ptr = nullptr, *col_row = nullptr, *row_ptr = nullptr, *row_col = nullptr, *perm = nullptr;
   PV_ALLOC(chol_dev_.tiles, tiles * 4096);
-  if (!chol_linv_) {   // the same sizes as on the dense path: a handle switched between the two shares them
-    PV_ALLOC(chol_linv_, T * 4096);
-    PV_ALLOC(chol_rhs_, p.n_pad);
-  }
   PV_ALLOC(slot, T * T);
   PV_ALLOC(col_ptr, T + 1);
   PV_ALLOC(row_ptr, T + 1);
@@ -1748,27 +1689,38 @@ int Engine::setup_cholesky_tiles() {
   return POVAR_OK;
 }
 
+// S dense or tile-sparse; the first solve with either builds the tile pattern or allocates the dense matrix, then the
+// factor's diagonal inverses and the right-hand side (the same sizes on both paths: a handle switched between the two
+// shares them)
+int Engine::alloc_cholesky(bool* tiled) {
+  const int n_pad = chol_padded(12 * C_);
+  *tiled = chol_storage_ == 1 || static_cast<long long>(n_pad) * n_pad * 8 > kCholDenseCap;
+  if (*tiled && !chol_tiled_ready_) {
+    const int rc = setup_cholesky_tiles();
+    if (rc != POVAR_OK) return rc;
+  }
+  if (!*tiled && !d_.dense_S) PV_ALLOC(d_.dense_S, static_cast<size_t>(n_pad) * n_pad);
+  if (!chol_linv_) {
+    PV_ALLOC(chol_linv_, static_cast<size_t>(n_pad) * 64);
+    PV_ALLOC(chol_rhs_, static_cast<size_t>(n_pad));
+  }
+  return POVAR_OK;
+}
+
 int Engine::solve_cholesky(double lambda) {
   const int n = 12 * C_;
   const int n_pad = chol_padded(n);
-  const bool tiled = chol_storage_ == 1 || static_cast<long long>(n_pad) * n_pad * 8 > kCholDenseCap;
-  chol_tiled_active_ = tiled;
   PV_CUDA(mark(0));
   int rc = prepare_reduced_system(false, lambda, 0.0);
   if (rc != POVAR_OK) return rc;
+  bool tiled = false;
+  rc = alloc_cholesky(&tiled);   // on first use inside this trial's prepare time
+  chol_tiled_active_ = tiled;
+  if (rc != POVAR_OK) return rc;
   if (tiled) {
-    if (!chol_tiled_ready_) {   // once per handle, inside this trial's prepare time
-      rc = setup_cholesky_tiles();
-      if (rc != POVAR_OK) return rc;
-    }
     PV_CUDA(cudaMemsetAsync(chol_dev_.tiles, 0, sizeof(double) * 4096 * static_cast<size_t>(chol_pat_.tiles()), stream_));
     launch_schur_tiles(d_, mp_, chol_dev_, n_pad, lc());
   } else {
-    if (!d_.dense_S) PV_ALLOC(d_.dense_S, static_cast<size_t>(n_pad) * n_pad);
-    if (!chol_linv_) {
-      PV_ALLOC(chol_linv_, static_cast<size_t>(n_pad) * 64);
-      PV_ALLOC(chol_rhs_, static_cast<size_t>(n_pad));
-    }
     PV_CUDA(cudaMemsetAsync(d_.dense_S, 0, sizeof(double) * static_cast<size_t>(n_pad) * n_pad, stream_));
     launch_schur_lower(d_, mp_, d_.dense_S, n_pad, lc());
   }
@@ -1953,7 +1905,7 @@ int Engine::enqueue_apply(bool joint, double alpha, bool reduce) {
   if (static_cast<int>(joint) != joint_lin_ || !have_solve_) {
     return fail(POVAR_ERR_INVALID, "apply called without a matching linearize + solve");
   }
-  set_model(joint, joint ? opt_.alpha : alpha);
+  set_model(joint ? opt_.alpha : alpha);
   const size_t C12 = static_cast<size_t>(C_) * 12;
   if (joint) {
     // apply_joint (linearizor_power_varproj.cpp:276-308): landmarks first, then P += s o (Pi inc)
@@ -1994,10 +1946,9 @@ int Engine::apply(bool joint, double alpha, double* l_diff) {
   return POVAR_OK;
 }
 
-int Engine::trial(bool joint, double alpha, double lambda, int32_t* iterations, double* l_diff,
-                  povar_residual_info* ri) {
-  PV_CUDA(cudaSetDevice(device_));
-  int rc = enqueue_solve(joint, lambda);   // records ev_[0] (start), ev_[1] (prepared), ev_[2] (solved)
+// marks 0 (start), 1 (prepared), 2 (solved), 3 (applied)
+int Engine::enqueue_trial(bool joint, double alpha, double lambda) {
+  int rc = enqueue_solve(joint, lambda);
   if (rc != POVAR_OK) return rc;
   rc = backup(joint ? POVAR_STATE_JOINT : POVAR_STATE_POSE);
   if (rc != POVAR_OK) return rc;
@@ -2008,10 +1959,16 @@ int Engine::trial(bool joint, double alpha, double lambda, int32_t* iterations, 
     launch_normalize_cams(d_, lc());
     launch_normalize_joint(d_, lc());
   }
-  PV_CUDA(cudaEventRecord(ev_[3], stream_));
+  PV_CUDA(mark(3));
   rc = enqueue_cost(joint, alpha, /*reduce=*/false);
   if (rc != POVAR_OK) return rc;
-  rc = allreduce(d_.trial_out, 9);
+  return allreduce(d_.trial_out, 9);
+}
+
+int Engine::trial(bool joint, double alpha, double lambda, int32_t* iterations, double* l_diff,
+                  povar_residual_info* ri) {
+  PV_CUDA(cudaSetDevice(device_));
+  const int rc = enqueue_trial(joint, alpha, lambda);
   if (rc != POVAR_OK) return rc;
   PV_CUDA(cudaGetLastError());
   static_assert(sizeof(SeriesCtl) <= 64, "SeriesCtl shares the pinned read-back buffer");
@@ -2345,6 +2302,35 @@ cudaError_t Engine::mark(int k) {
   return cudaEventRecord(ev_[k], stream_);
 }
 
+// what `body` enqueues on stream_, captured into a new graph (cap_graph_ while it runs) and instantiated into *exec.
+// Nothing runs: launches_ is left as it was.
+int Engine::capture_graph(void** exec, const std::function<int()>& body) {
+  const long long before = launches_;
+  cudaGraph_t graph = nullptr;
+  PV_CUDA(cudaGraphCreate(&graph, 0));
+  cap_graph_ = graph;
+  int rc = check(cudaStreamBeginCaptureToGraph(stream_, graph, nullptr, nullptr, 0, cudaStreamCaptureModeRelaxed),
+                 "cudaStreamBeginCaptureToGraph");
+  if (rc == POVAR_OK) rc = body();
+  cudaGraph_t same = nullptr;
+  if (rc == POVAR_OK) rc = check(cudaStreamEndCapture(stream_, &same), "cudaStreamEndCapture");
+  cudaGraphExec_t e = nullptr;
+  if (rc == POVAR_OK) rc = check(cudaGraphInstantiate(&e, graph, 0), "cudaGraphInstantiate");
+  cudaStreamCaptureStatus st = cudaStreamCaptureStatusNone;
+  if (rc != POVAR_OK && cudaStreamIsCapturing(stream_, &st) == cudaSuccess && st != cudaStreamCaptureStatusNone) {
+    cudaStreamEndCapture(stream_, &same);
+  }
+  cudaGraphDestroy(graph);
+  cap_graph_ = nullptr;
+  launches_ = before;
+  if (rc != POVAR_OK) {
+    cudaGetLastError();
+    return rc;
+  }
+  *exec = e;
+  return POVAR_OK;
+}
+
 int Engine::new_cond(unsigned long long* h) {
   cudaGraphConditionalHandle c = 0;
   PV_CUDA(cudaGraphConditionalHandleCreate(&c, static_cast<cudaGraph_t>(cap_graph_), 0, 0));
@@ -2360,7 +2346,7 @@ int Engine::capture_cond(int type, unsigned long long h, const std::function<int
   const cudaGraphNode_t* deps = nullptr;
   size_t num_deps = 0;
   PV_CUDA(cudaStreamGetCaptureInfo(stream_, &st, nullptr, nullptr, &deps, &num_deps));
-  if (st != cudaStreamCaptureStatusActive) return fail(POVAR_ERR_CUDA, "stream capture of the solve is not active");
+  if (st != cudaStreamCaptureStatusActive) return fail(POVAR_ERR_CUDA, "stream capture is not active");
   cudaGraphNodeParams params{};
   params.type = cudaGraphNodeTypeConditional;
   params.conditional.handle = static_cast<cudaGraphConditionalHandle>(h);
@@ -2382,7 +2368,8 @@ int Engine::capture_cond(int type, unsigned long long h, const std::function<int
   return POVAR_OK;
 }
 
-// the series graph of enqueue_series, built into the graph being captured
+// the power series as prefix + WHILE(term), into the graph being captured: the series graph of enqueue_series, or a
+// node of the solve graph
 int Engine::capture_series(bool joint) {
   const int m = opt_.power_sc_iterations;
   unsigned long long h = 0;
@@ -2405,9 +2392,6 @@ int Engine::capture_series(bool joint) {
 int Engine::capture_lm_step(const povar_options& opt, bool joint, unsigned long long ok) {
   const int step = joint ? 2 : 1;
   const int max_iter = joint ? opt.max_num_iterations_step_2 : opt.max_num_iterations_step_1;
-  const bool power = joint ? opt.solver_type_step_2 == POVAR_RIPOBA
-                           : (opt.solver_type_step_1 == POVAR_POWER_VARPROJ ||
-                              opt.solver_type_step_1 == POVAR_POWER_SCHUR_COMPLEMENT);
   PV_CUDA(mark(0));
   int rc = enqueue_cost(joint, opt.alpha);
   if (rc != POVAR_OK) return rc;
@@ -2424,21 +2408,10 @@ int Engine::capture_lm_step(const povar_options& opt, bool joint, unsigned long 
     launch_lm_top(lm_, b, lc());
     rc2 = capture_cond(cudaGraphCondTypeIf, b.lin, [&]() { return linearize(joint, opt.alpha, true); });
     if (rc2 != POVAR_OK) return rc2;
-    // Engine::trial: solve, backup, apply, (step 2: normalise,) cost, one exchange of trial_out[0..9)
-    rc2 = enqueue_solve(joint, 0.0);
-    if (rc2 == POVAR_OK) rc2 = backup(0);
-    if (rc2 == POVAR_OK) rc2 = enqueue_apply(joint, opt.alpha, /*reduce=*/false);
-    if (rc2 != POVAR_OK) return rc2;
-    if (joint) {
-      launch_normalize_cams(d_, lc());
-      launch_normalize_joint(d_, lc());
-    }
-    PV_CUDA(mark(3));
-    rc2 = enqueue_cost(joint, opt.alpha, /*reduce=*/false);
-    if (rc2 == POVAR_OK) rc2 = allreduce(d_.trial_out, 9);
+    rc2 = enqueue_trial(joint, opt.alpha, 0.0);   // the damping comes from lm_->loop.lambda
     if (rc2 != POVAR_OK) return rc2;
     PV_CUDA(mark(4));
-    launch_lm_decide(lm_, d_.trial_out, d_.ctl, opt, step, power, lm_log_, lm_cap_, b, lc());
+    launch_lm_decide(lm_, d_.trial_out, d_.ctl, opt, step, lm_power_step(opt, joint), lm_log_, lm_cap_, b, lc());
     return capture_cond(cudaGraphCondTypeIf, b.restore, [&]() { return restore(0); });
   });
   if (rc != POVAR_OK) return rc;
@@ -2449,28 +2422,14 @@ int Engine::capture_lm_step(const povar_options& opt, bool joint, unsigned long 
 
 int Engine::build_solve_graph(const povar_options& opt) {
   // every allocation the host route makes on first use (linearize, solve_cholesky), and the control block and log
-  if (!d_.obs_d) {
-    PV_ALLOC(d_.obs_d, static_cast<size_t>(nnz_) * 3);
-    PV_ALLOC(d_.csc_d, static_cast<size_t>(nnz_) * 3);
-    PV_ALLOC(d_.sell_d, static_cast<size_t>(d_.ix.sell_slots) * 3);
-  }
-  if (opt_.robust_norm == POVAR_NORM_HUBER && !d_.obs_w) {
-    PV_ALLOC(d_.obs_w, static_cast<size_t>(nnz_));
-    PV_ALLOC(d_.csc_w, static_cast<size_t>(nnz_));
-    PV_ALLOC(d_.sell_w, static_cast<size_t>(d_.ix.sell_slots));
+  for (const bool joint : {true, false}) {
+    const int rc = alloc_lin_buffers(joint);
+    if (rc != POVAR_OK) return rc;
   }
   if (opt_.solver_type_step_1 == POVAR_CHOLESKY) {
-    const int n_pad = chol_padded(12 * C_);
-    const bool tiled = chol_storage_ == 1 || static_cast<long long>(n_pad) * n_pad * 8 > kCholDenseCap;
-    if (tiled && !chol_tiled_ready_) {
-      const int rc = setup_cholesky_tiles();
-      if (rc != POVAR_OK) return rc;
-    }
-    if (!tiled && !d_.dense_S) PV_ALLOC(d_.dense_S, static_cast<size_t>(n_pad) * n_pad);
-    if (!chol_linv_) {
-      PV_ALLOC(chol_linv_, static_cast<size_t>(n_pad) * 64);
-      PV_ALLOC(chol_rhs_, static_cast<size_t>(n_pad));
-    }
+    bool tiled = false;
+    const int rc = alloc_cholesky(&tiled);
+    if (rc != POVAR_OK) return rc;
   }
   if (!lm_) {
     PV_ALLOC(lm_, 1);
@@ -2483,53 +2442,30 @@ int Engine::build_solve_graph(const povar_options& opt) {
     PV_ALLOC(lm_log_, static_cast<size_t>(cap));
     lm_cap_ = static_cast<int>(cap);
   }
-  cudaGraph_t graph = nullptr;
-  PV_CUDA(cudaGraphCreate(&graph, 0));
-  const long long before = launches_;
   capturing_ = true;
-  cap_graph_ = graph;
   lambda_dev_ = &lm_->loop.lambda;
-  auto body = [&]() -> int {
-    cudaError_t e = cudaStreamBeginCaptureToGraph(stream_, graph, nullptr, nullptr, 0, cudaStreamCaptureModeRelaxed);
-    if (e != cudaSuccess) return check(e, "cudaStreamBeginCaptureToGraph");
+  const int rc = capture_graph(&solve_graph_, [&]() -> int {
     launch_lm_stamp(&lm_->t_start, lc());
     launch_lm_stamp(&lm_->t_it, lc());
-    int rc = init_varproj(opt.alpha);   // :302-304
+    int rc2 = init_varproj(opt.alpha);   // :302-304
     unsigned long long ok = kNoCond;
-    if (rc == POVAR_OK) rc = new_cond(&ok);
-    if (rc == POVAR_OK) rc = capture_lm_step(opt, false, ok);
-    if (rc == POVAR_OK) {
-      rc = capture_cond(cudaGraphCondTypeIf, ok, [&]() -> int {
-        int rc2 = to_homogeneous();   // create_homogeneous_landmark, :544-553
-        if (rc2 != POVAR_OK) return rc2;
+    if (rc2 == POVAR_OK) rc2 = new_cond(&ok);
+    if (rc2 == POVAR_OK) rc2 = capture_lm_step(opt, false, ok);
+    if (rc2 == POVAR_OK) {
+      rc2 = capture_cond(cudaGraphCondTypeIf, ok, [&]() -> int {
+        const int rc3 = to_homogeneous();   // create_homogeneous_landmark, :544-553
+        if (rc3 != POVAR_OK) return rc3;
         launch_lm_stamp(&lm_->t_it, lc());
         return capture_lm_step(opt, true, kNoCond);
       });
     }
-    if (rc != POVAR_OK) return rc;
+    if (rc2 != POVAR_OK) return rc2;
     launch_lm_finish(lm_, lm_cap_, lm_sum_, lm_status_, lc());
-    cudaGraph_t same = nullptr;
-    return check(cudaStreamEndCapture(stream_, &same), "cudaStreamEndCapture");
-  };
-  int rc = body();
+    return POVAR_OK;
+  });
   capturing_ = false;
-  cap_graph_ = nullptr;
   lambda_dev_ = nullptr;
-  launches_ = before;   // nothing ran
-  cudaStreamCaptureStatus st = cudaStreamCaptureStatusNone;
-  if (cudaStreamIsCapturing(stream_, &st) == cudaSuccess && st != cudaStreamCaptureStatusNone) {
-    cudaGraph_t dummy = nullptr;
-    cudaStreamEndCapture(stream_, &dummy);
-    if (dummy && dummy != graph) cudaGraphDestroy(dummy);
-  }
-  cudaGraphExec_t exec = nullptr;
-  if (rc == POVAR_OK) rc = check(cudaGraphInstantiate(&exec, graph, 0), "cudaGraphInstantiate");
-  cudaGraphDestroy(graph);
-  if (rc != POVAR_OK) {
-    cudaGetLastError();
-    return rc;
-  }
-  solve_graph_ = exec;
+  if (rc != POVAR_OK) return rc;
   solve_opt_ = opt;
   solve_window_ = d_.debug_window_cams;
   solve_storage_ = chol_storage_;

@@ -83,7 +83,10 @@ class Engine {
   TermMode term_mode() const { return peer_ok_ ? kTermPeer : (world_ == 1 ? kTermFused : kTermRaw); }
   const PeerExchange* exchange() const;
   int sum_setup_words(unsigned int* host, int words, int phase, int round);
-  void set_model(bool joint, double alpha);
+  void set_model(double alpha);
+  // work buffers allocated on first use (linearize, solve_cholesky) and before a capture (build_solve_graph)
+  int alloc_lin_buffers(bool joint);
+  int alloc_cholesky(bool* tiled);
   int solve_power(bool joint, double lambda);
   int solve_pcg(bool joint, double lambda);
   int solve_cholesky(double lambda);
@@ -96,9 +99,12 @@ class Engine {
   int enqueue_cost(bool joint, double alpha, bool reduce = true);
   int enqueue_apply(bool joint, double alpha, bool reduce = true);
   int enqueue_series(bool joint);
+  // solve, backup, apply, (step 2: normalise,) cost, one exchange of trial_out[0..9): one LM trial, no read-back
+  int enqueue_trial(bool joint, double alpha, double lambda);
   static void decode_cost(const double* v, povar_residual_info* out);
-  // the device-side solve (bundle_adjust_async): stream capture into nested conditional nodes
+  // the series graph and the device-side solve (bundle_adjust_async): stream capture into nested conditional nodes
   cudaError_t mark(int k);   // ev_[k], or a %globaltimer stamp into lm_->stamp[k] while capturing
+  int capture_graph(void** exec, const std::function<int()>& body);
   int new_cond(unsigned long long* h);
   int capture_cond(int type, unsigned long long h, const std::function<int()>& body);
   int capture_series(bool joint);
@@ -120,7 +126,6 @@ class Engine {
   // solver state
   int joint_lin_ = -1;            // model of the current linearisation: -1 none, 0 pOSE, 1 joint
   bool have_solve_ = false;       // a solve ran on the current linearisation (apply needs its increment)
-  double lambda_ = 0.0;           // damping of the last solve (landmark damping of apply)
   int dim_ = 12;
   double* P_prev_ = nullptr;      // cameras of the linearisation point during a VarPro apply
   bool lin_check_pending_ = false;  // linearize(defer_check): the flag is read with the next trial

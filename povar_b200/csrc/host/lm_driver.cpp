@@ -43,19 +43,13 @@ double seconds_since(Clock::time_point t0) {
   return std::chrono::duration<double>(Clock::now() - t0).count();
 }
 
-// Log::push: the non-timing columns are lm_log_push's (lm_step.h), the times are the host clock's and the events'
+// the log of a solve: the non-timing columns are lm_log_push's (lm_step.h), the times are the host clock's and the
+// events'
 struct Log {
   povar_iteration* out;
   int32_t capacity;
   povar::LmLog st;
 
-  void push(povar_handle* h, int step, int it, bool valid, bool successful, double trial_cost,
-            const povar_residual_info* ri, double rel, double radius, int lin_it, double it_time,
-            double cum_time) {
-    povar_iteration* e = (st.count < capacity && out) ? out + st.count : nullptr;
-    povar::lm_log_push(st, e, step, it, valid, successful, trial_cost, ri, rel, radius, lin_it);
-    stamp(h, e, it_time, cum_time);
-  }
   void stamp(povar_handle* h, povar_iteration* e, double it_time, double cum_time) {
     const povar::PhaseTimes& t = povar::handle_times(h);
     if (e) {
@@ -85,9 +79,7 @@ StepResult run_step(povar_handle* h, const povar_options& opt, bool joint, Log& 
                     double* power_time) {
   StepResult res;
   const int max_iter = joint ? opt.max_num_iterations_step_2 : opt.max_num_iterations_step_1;
-  const bool power = joint ? opt.solver_type_step_2 == POVAR_RIPOBA
-                           : (opt.solver_type_step_1 == POVAR_POWER_VARPROJ ||
-                              opt.solver_type_step_1 == POVAR_POWER_SCHUR_COMPLEMENT);
+  const bool power = povar::lm_power_step(opt, joint);
   povar::LmLoop s;
   s.lambda = 1.0 / opt.initial_trust_region_radius;
   bool first = true;

@@ -507,14 +507,13 @@ k_cam_binv16(int C, const double* __restrict__ P, const double* __restrict__ kro
 }
 
 // ------------------------------------------------------------------------------------------
-// camera half of a product:  raw_c = sum_i (Jp_raw^T W t_i), t_i = Jl_i H_l  (E0)  or
-// t_i = r_i - Jl_i H_l (b).  Output per item; k_reduce_items adds the items of a camera.
+// camera half of b:  raw_c = sum_i (Jp_raw^T W t_i), t_i = r_i - Jl_i H_l.  Output per item; k_reduce_items adds
+// the items of a camera.  (The camera half of the E0 products is k_passB_e0_v2, kernels_series.cu.)
 // ------------------------------------------------------------------------------------------
-template <bool JOINT, int MODE>
+template <bool JOINT>
 __global__ void __launch_bounds__(kBlock, 2)
 k_passB(DeviceIndex ix, const double* __restrict__ P, const double* __restrict__ lm_rec, double c1,
-        double c2, Robust rb, double* __restrict__ item_part, const SeriesCtl* __restrict__ ctl) {
-  if (ctl != nullptr && ctl->done) return;
+        double c2, Robust rb, double* __restrict__ item_part) {
   const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int lane = threadIdx.x & 31;
   if (warp >= ix.num_items) return;
@@ -545,13 +544,8 @@ k_passB(DeviceIndex ix, const double* __restrict__ P, const double* __restrict__
       ob.jl_rows(cam, j0, j1);
       const double l0 = dot4(j0, H), l1 = dot4(j1, H);
       const double w = ob.sw * ob.sw;
-      if (MODE == PASSB_E0) {
-        t[0] = w * l0;
-        t[1] = w * l1;
-      } else {
-        t[0] = w * (ob.r[0] - l0);
-        t[1] = w * (ob.r[1] - l1);
-      }
+      t[0] = w * (ob.r[0] - l0);
+      t[1] = w * (ob.r[1] - l1);
       ob.jpT_coef(t, m);
     } else {
       PoseObs ob;
@@ -561,7 +555,7 @@ k_passB(DeviceIndex ix, const double* __restrict__ P, const double* __restrict__
 #pragma unroll
       for (int q = 0; q < 4; ++q) {
         const double l = ob.T[q][0] * H[0] + ob.T[q][1] * H[1] + ob.T[q][2] * H[2];
-        t[q] = (MODE == PASSB_E0) ? w * l : w * (ob.r[q] - l);
+        t[q] = w * (ob.r[q] - l);
       }
       pose_jpT_coef(t, uv_now.x, uv_now.y, c1, c2, m);
     }
@@ -1110,9 +1104,9 @@ void launch_passB(const DeviceState& d, const ModelParams& mp, bool joint, const
   const Robust rb = {mp.robust_norm, mp.huber};
   const int blocks = item_grid(d);
   if (joint) {
-    k_passB<true, PASSB_B><<<blocks, kBlock, 0, lc.stream>>>(d.ix, d.P, d.lm_rec, mp.c1, mp.c2, rb, d.item_part, nullptr);
+    k_passB<true><<<blocks, kBlock, 0, lc.stream>>>(d.ix, d.P, d.lm_rec, mp.c1, mp.c2, rb, d.item_part);
   } else {
-    k_passB<false, PASSB_B><<<blocks, kBlock, 0, lc.stream>>>(d.ix, d.P, d.lm_rec, mp.c1, mp.c2, rb, d.item_part, nullptr);
+    k_passB<false><<<blocks, kBlock, 0, lc.stream>>>(d.ix, d.P, d.lm_rec, mp.c1, mp.c2, rb, d.item_part);
   }
   count(lc);
 }

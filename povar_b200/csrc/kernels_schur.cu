@@ -28,7 +28,7 @@ k_axpby(int n, double a, const double* __restrict__ x, double b, const double* _
   out[i] = (y != nullptr) ? a * x[i] + b * y[i] : a * x[i];
 }
 
-// two-stage deterministic dot product: per-block partials, then one block adds them in order
+// two-stage deterministic dot product: per-block partials, then one block of k_cg_scalar adds them in order
 __global__ void __launch_bounds__(kBlock)
 k_dot_part(int n, const double* __restrict__ x, const double* __restrict__ y, double* __restrict__ part) {
   __shared__ double smem[kBlock / 32];
@@ -36,15 +36,6 @@ k_dot_part(int n, const double* __restrict__ x, const double* __restrict__ y, do
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) acc[0] += x[i] * y[i];
   block_reduce<1>(acc, smem);
   if (threadIdx.x == 0) part[blockIdx.x] = acc[0];
-}
-
-__global__ void __launch_bounds__(kBlock)
-k_dot_final(int nblocks, const double* __restrict__ part, double* out) {
-  __shared__ double smem[kBlock / 32];
-  double acc[1] = {0.0};
-  for (int b = threadIdx.x; b < nblocks; b += blockDim.x) acc[0] += part[b];
-  block_reduce<1>(acc, smem);
-  if (threadIdx.x == 0) out[0] = acc[0];
 }
 
 // ---- conjugate gradients on the device (cg/conjugate_gradient.hpp:114-489): the scalar recurrences and every
@@ -143,16 +134,6 @@ void launch_axpby(const DeviceState& d, int n, double a, const double* x, double
   (void)d;
   k_axpby<<<(n + kBlock - 1) / kBlock, kBlock, 0, lc.stream>>>(n, a, x, b, y, out);
   count(lc);
-}
-
-void launch_dot(const DeviceState& d, int n, const double* x, const double* y, int slot, const LaunchCfg& lc) {
-  int blocks = (n + kBlock - 1) / kBlock;
-  const int cap = scalar_blocks(d);
-  if (blocks > cap) blocks = cap;
-  if (blocks < 1) blocks = 1;
-  k_dot_part<<<blocks, kBlock, 0, lc.stream>>>(n, x, y, d.scalar_part);
-  k_dot_final<<<1, kBlock, 0, lc.stream>>>(blocks, d.scalar_part, d.scalar_out + slot);
-  count(lc, 2);
 }
 
 void launch_dot_partials(const DeviceState& d, int n, const double* x, const double* y, const LaunchCfg& lc) {

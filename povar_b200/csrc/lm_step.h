@@ -75,7 +75,14 @@ POVAR_HD inline double lm_cube(double t) {
 #endif
 }
 
-// Log::push of the host driver without the times: entry `e` (nullptr: no room) gets the non-timing columns
+// whether the solver of a step is a power series (its iterations count as power_terms)
+inline bool lm_power_step(const povar_options& opt, bool joint) {
+  return joint ? opt.solver_type_step_2 == POVAR_RIPOBA
+               : (opt.solver_type_step_1 == POVAR_POWER_VARPROJ ||
+                  opt.solver_type_step_1 == POVAR_POWER_SCHUR_COMPLEMENT);
+}
+
+// one log entry without the times: entry `e` (nullptr: no room) gets the non-timing columns
 POVAR_HD inline void lm_log_push(LmLog& L, povar_iteration* e, int step, int it, bool valid, bool successful,
                                  double trial_cost, const povar_residual_info* ri, double rel, double radius,
                                  int lin_it) {

@@ -93,9 +93,10 @@ struct SeriesCtl {
   unsigned int long_left;   // blocks of the launch that have left the queue (the last one resets both)
 };
 
-// The series as a loop of the CUDA graph (Engine::enqueue_series): `handle` is the conditional handle of the WHILE
-// node whose body is one term; k_series_start and the last block of k_term16 set it (cudaGraphSetConditional), so
-// a series runs exactly the terms the reference's stopping rule asks for and nothing is enqueued to be skipped.
+// The series as a loop of a CUDA graph (Engine::capture_series: the series graph of enqueue_series, or a node of the
+// solve graph): `handle` is the conditional handle of the WHILE node whose body is one term; k_series_start and the
+// last block of k_term16 set it (cudaGraphSetConditional), so a series runs exactly the terms the reference's stopping
+// rule asks for and nothing is enqueued to be skipped.
 struct SeriesLoop {
   unsigned long long handle = 0;   // cudaGraphConditionalHandle
   int active = 0;                  // 0: terms are enqueued one by one with their number (eager launches, benchmarks)
@@ -204,7 +205,6 @@ struct DeviceState {
   double* cost_part = nullptr;   // [blocks * 8]
   CostAccum* cost_out = nullptr;
   double* scalar_part = nullptr; // [blocks] l_diff partials
-  double* scalar_out = nullptr;  // [8]  PCG dot products
   // what one LM trial reports, as doubles so that shards can be summed in place (Engine::allreduce):
   // [0..7] cost {err_all, rsum_all, err_valid, rsum_valid, n_all, n_valid, nonfinite, -}, [8] l_diff,
   // [9] numerical-failure flag of the linearisation
@@ -321,7 +321,6 @@ void launch_cam_scale(const DeviceState& d, const ModelParams& mp, const LaunchC
 void launch_cam_binv(const DeviceState& d, bool joint, double lambda, const LaunchCfg& lc,
                      const double* lambda_dev = nullptr);
 void launch_cam_precond(const DeviceState& d, bool joint, const double* kron_sdiag, const LaunchCfg& lc);
-enum PassBMode { PASSB_E0 = 0, PASSB_B = 1 };
 void launch_passB(const DeviceState& d, const ModelParams& mp, bool joint, const LaunchCfg& lc);
 // series bookkeeping
 void launch_series_start(const DeviceState& d, double r_tolerance, int max_terms, const LaunchCfg& lc,
@@ -359,8 +358,6 @@ void launch_block_matvec(const DeviceState& d, int dim, const double* blocks, co
 // out = a * x + b * y (y may be nullptr)
 void launch_axpby(const DeviceState& d, int n, double a, const double* x, double b, const double* y,
                   double* out, const LaunchCfg& lc);
-// scalar_out[slot] = x . y (deterministic two-stage reduction); slot in [0, 8)
-void launch_dot(const DeviceState& d, int n, const double* x, const double* y, int slot, const LaunchCfg& lc);
 // CHOLESKY (kernels_chol.cu): dense reduced camera system of step 1, S = blockdiag(Bmat) - sum_l Hpl Hll^-1 Hlp,
 // lower block triangle, fixed summation order; blocked LL^T on 64x64 tiles; substitution
 int chol_padded(int n);
